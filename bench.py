@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # engine arm
     python bench.py --impl reference [--gpus N] [--steps K] ...    # CPU reference arm
+    python bench.py ... --dump-outputs DIR     # engine arm, plus the last step's output in DIR
 
 A "step" is one operator apply y = Ahat u over the whole mesh:
   N = 1 : BASELINE.json configs[1], 1024 x 1024 elements, p = 8 (67 125 249 DOF);
@@ -30,6 +31,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "Poisson operator-apply GDOF/s (FP64, p=8)"
 ORDER = 8
+DUMP_ENTRIES = 4000000          # float64 entries written by --dump-outputs (32 MB) over all ranks
 
 
 def parse():
@@ -77,7 +79,15 @@ def parse():
     ap.add_argument("--ho-mode", default="", help="apply-kernel variant passed to poisson_operator")
     ap.add_argument("--ablate", type=int, default=0,
                     help="internal profiling knob: extra apply flag bits (results are wrong)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the apply output of the last step to "
+                         "DIR/apply_output.npy (float64; a fixed seeded sample of its entries "
+                         "when the whole vector exceeds %d entries)" % DUMP_ENTRIES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "engine" or args.sweep):
+        ap.error("--dump-outputs applies to the engine arm's apply only")
     global ORDER, METRIC
     if args.order != ORDER:
         ORDER = args.order
@@ -636,6 +646,19 @@ def run_sweep(args):
     print(json.dumps(res), flush=True)
 
 
+def dump_output(out_dir, name, y, n_keep):
+    """Writes the device vector y to out_dir/name.npy as float64: whole when it has at most
+    n_keep entries, else the entries at sorted indices drawn with a fixed seed from its length
+    alone, so that two builds run with the same arguments can be compared entry for entry."""
+    import numpy as np
+    import torch
+    if y.numel() > n_keep:
+        idx = np.unique(np.random.default_rng(0).integers(0, y.numel(), size=n_keep))
+        y = y[torch.from_numpy(idx).to(y.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), y.to(torch.float64).cpu().numpy())
+
+
 def run_engine(args):
     import numpy as np
     import torch
@@ -720,6 +743,10 @@ def run_engine(args):
         ev1.record()
         barrier()
         elapsed = ev0.elapsed_time(ev1) / 1e3
+    if args.dump_outputs:
+        # the caller of the timed apply receives `out`; under torchrun each rank its own part
+        dump_output(args.dump_outputs, "apply_output" + ("_rank%d" % rank if multi else ""), out,
+                    DUMP_ENTRIES // world)
     if multi:
         t = torch.tensor([elapsed], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
