@@ -28,7 +28,7 @@ import torch
 
 from . import _lib, device
 from ._lib import DIRICHLET_IDENTITY, MASK_IN, MASK_OUT
-from .operators import PCGInfo
+from .operators import PCGInfo, _PoissonBase
 
 __all__ = ["CondensedPoissonOperator", "CondensedLocalSystems", "condensed_tables", "coarse_tables",
            "condensed_tables_device", "coarse_tables_device",
@@ -160,7 +160,7 @@ def _load_key(f):
     return None
 
 
-class CondensedPoissonOperator(object):
+class CondensedPoissonOperator(_PoissonBase):
     def __init__(self, dof_mngr, dirichlet=None, geometric_factors=None, weight=None,
                  store_interior="auto", reaction=None, store_interior_inverse=False):
         """store_interior : keep W_e = A_ii^-1 A_ie of every element (12.5 KB per element at
@@ -197,7 +197,7 @@ class CondensedPoissonOperator(object):
             raise NotImplementedError("condensed_poisson_operator supports one DOF per node")
         self.dof_mngr = dof_mngr
         self.n_nodes = int(mesh.n_nodes)
-        self.n_ext = int(mesh.n_nodes_cell_exterior)
+        self.n_ext = self._n_vec = int(mesh.n_nodes_cell_exterior)
         full_mask = None
         if dirichlet is not None:
             dirichlet = np.asarray(dirichlet)
@@ -250,49 +250,14 @@ class CondensedPoissonOperator(object):
     def _init_geometry(self, geometric_factors, weight):
         """Geometric factors, one plain [3][NN] block per element in reference element
         order (the engine layout of semk_op.G with one-element patches)."""
-        mesh = self.dof_mngr.mesh
-        n1 = self.n1
-        NN = n1 * n1
+        NN = self.n1 * self.n1
         f64 = dict(dtype=torch.float64, device=self.dev)
         self.g_stride = (3 * NN + 1) & ~1
         self.G = torch.zeros((self.n_elem, self.g_stride), **f64)
         self.JxW = torch.empty((self.n_elem, NN), **f64)
-        x_phys = None
-        if geometric_factors is None:
-            nodes_dev = torch.from_numpy(np.ascontiguousarray(mesh.nodes, dtype=np.float64)).to(self.dev)
-            if nodes_dev.shape[0] != 2:
-                raise NotImplementedError("Only supporting 2D elements right now")
-            if callable(weight):
-                x_phys = torch.empty((self.n_elem, 2, NN), **f64)
-            device.geom_factors(self.tab, nodes_dev, self.l2g_dev, self.n_elem, G=self.G,
-                                g_patch_stride=self.g_stride, elems_per_patch=1, JxW=self.JxW,
-                                x_phys=x_phys)
-            del nodes_dev
-        else:
-            invJ, jxw = geometric_factors
-            invJ = device._f64(np.asarray(invJ).reshape(self.n_elem, 4, NN), self.dev)
-            self.JxW.copy_(device._f64(np.asarray(jxw).reshape(self.n_elem, NN), self.dev))
-            _lib.check(self._lib.semk_gfactors_from_invj_f64(
-                n1, self.n_elem, device.ptr(invJ), device.ptr(self.JxW), None,
-                device.ptr(self.G), self.g_stride, 1, device.stream_ptr()))
-            torch.cuda.current_stream().synchronize()
-            del invJ
-        if weight is not None:      # stiffness of -div(w grad u), as PoissonOperator(weight=...)
-            if callable(weight):
-                if x_phys is None:
-                    raise ValueError("a callable weight needs the device geometry")
-                w = weight(x_phys[:, 0, :], x_phys[:, 1, :])
-                w = torch.as_tensor(w, dtype=torch.float64, device=self.dev).expand(self.n_elem, NN)
-            else:
-                w = device._f64(np.asarray(weight, dtype=np.float64).reshape(self.n_elem, NN),
-                                self.dev)
-            w = w.contiguous()
-            _lib.check(self._lib.semk_scale_gfactors_f64(
-                n1, self.n_elem, device.ptr(w), None, device.ptr(self.G), self.g_stride, 1,
-                device.stream_ptr()))
-            torch.cuda.current_stream().synchronize()
-            del w
-        del x_phys
+        device.stiffness_factors(self.tab, self.dof_mngr.mesh, self.l2g_dev, self.n_elem, self.G,
+                                 self.g_stride, 1, self.JxW, geometric_factors=geometric_factors,
+                                 weight=weight)
 
     def _finish_common(self, full_mask):
         f64 = dict(dtype=torch.float64, device=self.dev)
@@ -345,22 +310,16 @@ class CondensedPoissonOperator(object):
         self._dinv = None
 
     # -- element kernel ----------------------------------------------------------------
-    def _full_vec(self, v, name):
-        if not (isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == torch.float64
-                and v.is_contiguous() and v.numel() == self.n_nodes):
-            raise ValueError("%s must be a contiguous float64 CUDA tensor of length n_nodes" % name)
-        return v
-
     def _element_pass(self, mode, S=None, sdiag_loc=None, g_loc=None, u=None, f=1.0, W=None,
                       c=None, Ainv=None):
         """One launch of sc_element_kernel (csrc/semk_sc.cu)."""
         f_nodal, f_scale = None, 1.0
         if isinstance(f, torch.Tensor):
-            f_nodal = self._full_vec(f, "f")
+            f_nodal = self._vec(f, "f", self.n_nodes)
         elif np.ndim(f) == 0:
             f_scale = float(f)
         else:
-            f_nodal = self._full_vec(self.from_host(f), "f")
+            f_nodal = self._vec(self.from_host(f), "f", self.n_nodes)
         self._bad.zero_()
         _lib.check(self._lib.semk_sc_element_react_f64(
             self.n1, self.n_elem, None, device.ptr(self.G), self.g_stride, 1,
@@ -373,21 +332,6 @@ class CondensedPoissonOperator(object):
             raise AssertionError("an element-interior stiffness block is not positive definite")
 
     # -- helpers -----------------------------------------------------------------------
-    def _vec(self, v, name="vector"):
-        if not (isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == torch.float64
-                and v.is_contiguous() and v.numel() == self.n_ext):
-            raise ValueError("%s must be a contiguous float64 CUDA tensor of length "
-                             "ndof_exterior" % name)
-        return v
-
-    def new_vector(self, fill=None):
-        if fill is None:
-            return torch.empty(self.n_ext, dtype=torch.float64, device=self.dev)
-        return torch.full((self.n_ext,), float(fill), dtype=torch.float64, device=self.dev)
-
-    def from_host(self, a):
-        return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(self.dev)
-
     @property
     def algorithmic_bytes_per_apply(self):
         """Packed S_e + one uint32 L2G entry per element-exterior node, read u,
@@ -417,9 +361,6 @@ class CondensedPoissonOperator(object):
             device.stream_ptr()))
         return y
 
-    def apply_unmasked(self, u, out=None):
-        return self.apply(u, out=out, flags=0)
-
     def assemble(self, loc, out=None, mask=False, fill_dirichlet=0.0):
         """Sum an element-local exterior field ``loc[E, 4p]`` into a condensed
         vector (``grhs[inds_ext] += ...``, sem/discrete.py:499)."""
@@ -443,8 +384,8 @@ class CondensedPoissonOperator(object):
         if (getattr(self, "_Ainv", None) is not None and self._W is not None and key is not None
                 and type(self) is CondensedPoissonOperator):
             # stored interior operators: the load is a stream over W and A_ii^-1
-            f_nodal, f_scale = (self._full_vec(f, "f"), 1.0) if isinstance(f, torch.Tensor) \
-                else (None, float(f))
+            f_nodal, f_scale = ((self._vec(f, "f", self.n_nodes), 1.0)
+                                if isinstance(f, torch.Tensor) else (None, float(f)))
             c = torch.empty((self.n_elem, self.n_int_loc), dtype=torch.float64, device=self.dev)
             _lib.check(self._lib.semk_sc_load_stored_f64(
                 self.n1, self.n_elem, device.ptr(self._W), device.ptr(self._Ainv),
@@ -461,29 +402,6 @@ class CondensedPoissonOperator(object):
         if c is not None:
             self._c, self._c_key = c, key
         return self.assemble(g_loc)
-
-    def lift(self, b, dirichlet_values=None):
-        """RHS of the SPD system: free rows b_f - S_fe g_e, Dirichlet rows g_e
-        (sem/discrete.py:505-509)."""
-        self._vec(b, "b")
-        if not self.has_dirichlet:
-            return b.clone()
-        mask = self.dirichlet_dev.bool()
-        g = torch.zeros_like(b)
-        if dirichlet_values is not None:
-            gv = dirichlet_values if isinstance(dirichlet_values, torch.Tensor) \
-                else self.from_host(dirichlet_values)
-            gv = gv[:self.n_ext]
-            g[mask] = gv[mask]
-        t = self.apply(g, flags=MASK_OUT)
-        out = b - t
-        out[mask] = g[mask]
-        return out
-
-    def jacobi_inverse(self):
-        if self._dinv is None:
-            self._dinv = 1.0 / self.diagonal(masked=True)
-        return self._dinv
 
     def _build_coarse(self):
         """Vertex coarse space of the two-level preconditioner (lazy): host tables
@@ -679,13 +597,7 @@ class CondensedPoissonOperator(object):
         self._vec(b, "b")
         if preconditioner not in ("jacobi", "two-level", "three-level"):
             raise ValueError("preconditioner must be 'jacobi', 'two-level' or 'three-level'")
-        if x0 is None:
-            x = torch.zeros_like(b)
-            if self.has_dirichlet:
-                m = self.dirichlet_dev.bool()
-                x[m] = b[m]
-        else:
-            x = self._vec(x0, "x0").clone()
+        x = self._start_iterate(b, x0)
         if preconditioner != "jacobi":
             cs, t, n_v = self._build_coarse()
             levels = 3 if preconditioner == "three-level" else 2
@@ -739,7 +651,7 @@ class CondensedPoissonOperator(object):
         (_solve_interior_dofs, sem/discrete.py:513-524)."""
         self._vec(x_ext, "x_ext")
         u = (torch.empty(self.n_nodes, dtype=torch.float64, device=self.dev) if out is None
-             else self._full_vec(out, "out"))
+             else self._vec(out, "out", self.n_nodes))
         u[:self.n_ext].copy_(x_ext)
         if (getattr(self, "_W", None) is not None and self._c is not None
                 and self._c_key == _load_key(f)):

@@ -90,6 +90,56 @@ def geom_factors(tab, nodes_dev, l2g_dev, n_elem, elem_of_slot=None, G=None, g_p
         raise AssertionError("non-positive Jacobian determinant in the mesh")
 
 
+def stiffness_factors(tab, mesh, l2g_dev, n_slots, G, g_stride, elems_per_patch, JxW,
+                      elem_of_slot=None, geometric_factors=None, weight=None):
+    """Geometric factors of the stiffness into ``G`` (engine layout: ``n_slots`` slots,
+    ``elems_per_patch`` per row of stride ``g_stride``; ``elem_of_slot`` maps slot -> element,
+    None = the identity) and the quadrature weights into ``JxW[E, NN]``: from the mesh nodes
+    by K1, or from the caller's ``geometric_factors = (invJ[E,2,2,N,N], JxW[E,N,N])``.
+    ``weight`` makes it the stiffness of -div(w grad u): nodal values [E, N, N], or a callable
+    w(x, y) of the physical coordinates (needs the device geometry)."""
+    if callable(weight) and geometric_factors is not None:
+        raise ValueError("a callable weight needs the device geometry (geometric_factors=None)")
+    lib = _lib.load()
+    n1 = tab.n1
+    n_elem, NN = JxW.shape
+    dev = G.device
+    x_phys = None
+    if geometric_factors is None:
+        nodes_dev = torch.from_numpy(np.ascontiguousarray(mesh.nodes, dtype=np.float64)).to(dev)
+        if nodes_dev.shape[0] != 2:
+            raise NotImplementedError("Only supporting 2D elements right now")
+        if callable(weight):
+            x_phys = torch.empty((n_elem, 2, NN), dtype=torch.float64, device=dev)
+        geom_factors(tab, nodes_dev, l2g_dev, n_slots, elem_of_slot=elem_of_slot, G=G,
+                     g_patch_stride=g_stride, elems_per_patch=elems_per_patch, JxW=JxW,
+                     x_phys=x_phys)
+        del nodes_dev
+    else:
+        invJ, jxw = geometric_factors
+        invJ = _f64(np.asarray(invJ).reshape(n_elem, 4, NN), dev)
+        JxW.copy_(_f64(np.asarray(jxw).reshape(n_elem, NN), dev))
+        _lib.check(lib.semk_gfactors_from_invj_f64(
+            n1, n_slots, ptr(invJ), ptr(JxW), ptr(elem_of_slot), ptr(G), g_stride,
+            elems_per_patch, stream_ptr()))
+        torch.cuda.current_stream().synchronize()
+        del invJ
+    if weight is None:
+        return
+    # scale the geometric factors node by node (the rho_JxW einsums of
+    # examples/squirmer-axisymmetric.py:194-213 with w = x_phys[0])
+    if callable(weight):
+        w = weight(x_phys[:, 0, :], x_phys[:, 1, :])
+        w = torch.as_tensor(w, dtype=torch.float64, device=dev).expand(n_elem, NN)
+    else:
+        w = _f64(np.asarray(weight, dtype=np.float64).reshape(n_elem, NN), dev)
+    w = w.contiguous()
+    _lib.check(lib.semk_scale_gfactors_f64(
+        n1, n_slots, ptr(w), ptr(elem_of_slot), ptr(G), g_stride, elems_per_patch,
+        stream_ptr()))
+    torch.cuda.current_stream().synchronize()
+
+
 def element_geometry(basis, nodes, l2g, jacobian=True):
     """Geometry of a batch of elements, returned as host arrays in the
     reference's layouts: x_phys [E,2,N,N]; J, invJ [E,2,2,N,N]; detJ [E,N,N]."""

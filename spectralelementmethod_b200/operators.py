@@ -164,7 +164,69 @@ class PCGInfo(object):
                 % (self.iterations, self.status, self.rel_residual, self.bnorm))
 
 
-class PoissonOperator(object):
+class _PoissonBase(object):
+    """Vector plumbing, Dirichlet lifting and the Jacobi-PCG start of the plain and the
+    condensed Poisson operators (condensed.CondensedPoissonOperator).  Their vectors are
+    contiguous float64 CUDA tensors of length ``_n_vec`` (n_nodes, or the n_ext exterior DOFs
+    that lead the exterior-first numbering); a subclass provides ``apply`` and ``diagonal``,
+    ``has_dirichlet`` and the uint8 mask ``dirichlet_dev`` over its vector."""
+
+    def _vec(self, v, name="vector", n=None):
+        n = self._n_vec if n is None else n
+        if not (isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == torch.float64
+                and v.is_contiguous() and v.numel() == n):
+            raise ValueError("%s must be a contiguous float64 CUDA tensor of length %d" % (name, n))
+        return v
+
+    def new_vector(self, fill=None):
+        if fill is None:
+            return torch.empty(self._n_vec, dtype=torch.float64, device=self.dev)
+        return torch.full((self._n_vec,), float(fill), dtype=torch.float64, device=self.dev)
+
+    def from_host(self, a):
+        return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(self.dev)
+
+    def apply_unmasked(self, u, out=None):
+        """y = A u: the operator without Dirichlet rows."""
+        return self.apply(u, out=out, flags=0)
+
+    def lift(self, b, dirichlet_values=None):
+        """RHS of the SPD system Ahat x = bhat: free rows b_f - A_fe g_e,
+        Dirichlet rows g_e (sem/discrete.py:505-509).  ``dirichlet_values``: CUDA tensor or
+        host array of the operator's vector length, or a whole nodal vector (n_nodes), of
+        which the condensed operator reads the leading n_ext entries."""
+        self._vec(b, "b")
+        if not self.has_dirichlet:
+            return b.clone()
+        mask = self.dirichlet_dev.bool()
+        g = torch.zeros_like(b)
+        if dirichlet_values is not None:
+            gv = dirichlet_values if isinstance(dirichlet_values, torch.Tensor) \
+                else self.from_host(dirichlet_values)
+            if gv.numel() == self.n_nodes:
+                gv = gv[:self._n_vec]
+            g[mask] = gv[mask]
+        out = b - self.apply(g, flags=MASK_OUT)      # A (I-M) g on the free rows
+        out[mask] = g[mask]
+        return out
+
+    def jacobi_inverse(self):
+        if self._dinv is None:
+            self._dinv = 1.0 / self.diagonal(masked=True)
+        return self._dinv
+
+    def _start_iterate(self, b, x0):
+        """PCG start: a copy of ``x0``, else zeros with b on the Dirichlet rows."""
+        if x0 is not None:
+            return self._vec(x0, "x0").clone()
+        x = torch.zeros_like(b)
+        if self.has_dirichlet:
+            mask = self.dirichlet_dev.bool()
+            x[mask] = b[mask]
+        return x
+
+
+class PoissonOperator(_PoissonBase):
     def __init__(self, dof_mngr, dirichlet=None, geometric_factors=None, elems_per_patch=None,
                  elem_order=None, keep_l2g=True, tile=None, weight=None, mode="auto",
                  boundary_columns_first=False):
@@ -177,7 +239,7 @@ class PoissonOperator(object):
         NN = n1 * n1
         l2g = mesh.node_map_array().reshape(-1, NN)
         self.n_elem = int(l2g.shape[0])          # elements; engine slots: self.n_order
-        self.n_nodes = int(mesh.n_nodes)
+        self.n_nodes = self._n_vec = int(mesh.n_nodes)
         self.dev = torch.device("cuda", torch.cuda.current_device())
 
         if dirichlet is not None:
@@ -270,48 +332,11 @@ class PoissonOperator(object):
         self.G = torch.zeros((self.n_patch, self.g_patch_stride), **f64)
         self.JxW = torch.empty((self.n_elem, NN), **f64)
         self.l2g_dev = device.as_i32_bits(l2g, self.dev)
-        x_phys = None
-        if geometric_factors is None:
-            nodes_dev = torch.from_numpy(np.ascontiguousarray(mesh.nodes, dtype=np.float64)).to(self.dev)
-            if nodes_dev.shape[0] != 2:
-                raise NotImplementedError("Only supporting 2D elements right now")
-            if callable(weight):
-                x_phys = torch.empty((self.n_elem, 2, NN), **f64)
-            device.geom_factors(self.tab, nodes_dev, self.l2g_dev, self.n_order,
-                                elem_of_slot=t[_lib.PA_ELEM_OF_SLOT], G=self.G,
-                                g_patch_stride=self.g_patch_stride, elems_per_patch=pe,
-                                JxW=self.JxW, x_phys=x_phys)
-            del nodes_dev
-        else:
-            invJ, jxw = geometric_factors
-            invJ = device._f64(np.asarray(invJ).reshape(self.n_elem, 4, NN), self.dev)
-            self.JxW.copy_(device._f64(np.asarray(jxw).reshape(self.n_elem, NN), self.dev))
-            _lib.check(self._lib.semk_gfactors_from_invj_f64(
-                n1, self.n_order, device.ptr(invJ), device.ptr(self.JxW),
-                device.ptr(t[_lib.PA_ELEM_OF_SLOT]), device.ptr(self.G), self.g_patch_stride, pe,
-                device.stream_ptr()))
-            torch.cuda.current_stream().synchronize()
-            del invJ
-        # weighted stiffness -div(w grad u): scale the geometric factors node by node (the
-        # rho_JxW einsums of examples/squirmer-axisymmetric.py:194-213 with w = x_phys[0])
+        device.stiffness_factors(self.tab, mesh, self.l2g_dev, self.n_order, self.G,
+                                 self.g_patch_stride, pe, self.JxW,
+                                 elem_of_slot=t[_lib.PA_ELEM_OF_SLOT],
+                                 geometric_factors=geometric_factors, weight=weight)
         self.weighted = weight is not None
-        if weight is not None:
-            if callable(weight):
-                if x_phys is None:
-                    raise ValueError("a callable weight needs the device geometry "
-                                     "(geometric_factors=None)")
-                w = weight(x_phys[:, 0, :], x_phys[:, 1, :])
-                w = torch.as_tensor(w, dtype=torch.float64, device=self.dev).expand(self.n_elem, NN)
-            else:
-                w = device._f64(np.asarray(weight, dtype=np.float64).reshape(self.n_elem, NN),
-                                self.dev)
-            w = w.contiguous()
-            _lib.check(self._lib.semk_scale_gfactors_f64(
-                n1, self.n_order, device.ptr(w), device.ptr(t[_lib.PA_ELEM_OF_SLOT]),
-                device.ptr(self.G), self.g_patch_stride, pe, device.stream_ptr()))
-            torch.cuda.current_stream().synchronize()
-            del w
-        del x_phys
         self.box_ld = 0
         if self.kernel_variant == 2:
             self.box_ld = self._mark_box_patches(l2g, t)
@@ -404,20 +429,6 @@ class PoissonOperator(object):
         self.n_box_patches = int(ok_patch.sum().item())
         return ld if self.n_box_patches > 0 else 0
 
-    def _vec(self, v, name="vector"):
-        if not (isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == torch.float64
-                and v.is_contiguous() and v.numel() == self.n_nodes):
-            raise ValueError("%s must be a contiguous float64 CUDA tensor of length n_nodes" % name)
-        return v
-
-    def new_vector(self, fill=None):
-        if fill is None:
-            return torch.empty(self.n_nodes, dtype=torch.float64, device=self.dev)
-        return torch.full((self.n_nodes,), float(fill), dtype=torch.float64, device=self.dev)
-
-    def from_host(self, a):
-        return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(self.dev)
-
     @property
     def algorithmic_bytes_per_apply(self):
         """SURVEY.md 8(d): read u, write y, 3 geometric factors + one uint32
@@ -438,10 +449,6 @@ class PoissonOperator(object):
             C.byref(self._op), device.ptr(u), device.ptr(y), int(flags), device.ptr(dot_out),
             device.stream_ptr()))
         return y
-
-    def apply_unmasked(self, u, out=None):
-        """y = A u: the reference's assembled stiffness matrix, no BCs."""
-        return self.apply(u, out=out, flags=0)
 
     def apply_atomic(self, u, out=None, flags=None):
         """Same operator through the independent atomic-scatter kernel."""
@@ -599,42 +606,14 @@ class PoissonOperator(object):
         """Diagonal (lumped = exact for GLL collocation) mass matrix."""
         return self.rhs(1.0)
 
-    def lift(self, b, dirichlet_values=None):
-        """RHS of the SPD system Ahat x = bhat: free rows b_f - A_fe g_e,
-        Dirichlet rows g_e (sem/discrete.py:505-509)."""
-        self._vec(b, "b")
-        if not self.has_dirichlet:
-            return b.clone()
-        mask = self.dirichlet_dev.bool()
-        g = torch.zeros_like(b)
-        if dirichlet_values is not None:
-            gv = dirichlet_values if isinstance(dirichlet_values, torch.Tensor) \
-                else self.from_host(dirichlet_values)
-            g[mask] = gv[mask]
-        t = self.apply(g, flags=MASK_OUT)      # A (I-M) g on the free rows
-        out = b - t
-        out[mask] = g[mask]
-        return out
-
     # -- solver ----------------------------------------------------------------------
-    def jacobi_inverse(self):
-        if self._dinv is None:
-            self._dinv = 1.0 / self.diagonal(masked=True)
-        return self._dinv
-
     def solve_pcg(self, b, x0=None, rtol=1e-12, maxiter=200000, check_every=25):
         """Jacobi-preconditioned CG on Ahat x = b (b already lifted).  Returns
         (x, PCGInfo).  The loop runs on the device (native driver,
         csrc/semk_vec.cu); the host polls 64 bytes every ``check_every``
         iterations."""
         self._vec(b, "b")
-        if x0 is None:
-            x = torch.zeros_like(b)
-            if self.has_dirichlet:
-                m = self.dirichlet_dev.bool()
-                x[m] = b[m]
-        else:
-            x = self._vec(x0, "x0").clone()
+        x = self._start_iterate(b, x0)
         dinv = self.jacobi_inverse()
         work = torch.empty(3 * (self.n_nodes + 32), dtype=torch.float64, device=self.dev)
         sc = torch.zeros(8, dtype=torch.float64, device=self.dev)
