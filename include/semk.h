@@ -427,6 +427,34 @@ int semk_pcg_solve_f64(const semk_op *op, const double *b, double *x, const doub
                        int maxiter, int check_every, semk_pcg_info *info, void *stream);
 
 /* ------------------------------------------------------------------------
+ * Robin boundary term of the plain operator.  The weak form of
+ *     w du/dn + alpha u = g   on a boundary
+ * adds sum_faces sum_k alpha(x_k) dSxW_k u_k v_k to the bilinear form; with the face
+ * quadrature collocated at the GLL nodes that is a DIAGONAL term on the boundary nodes
+ * (the reference user adds alpha * bfe.dSxW to the diagonal of the local matrix).  It is
+ * kept apart from semk_op so that operators without it keep their launch arguments.
+ * ------------------------------------------------------------------------ */
+typedef struct semk_bdiag {
+  int64_t n;                /* distinct boundary nodes */
+  const uint32_t *node;     /* [n] their ids, ascending */
+  const double *val;        /* [n] assembled sum of alpha dSxW over the faces through the node */
+  double *partials;         /* [semk_vec_partials_len()] dot-product scratch, zeroed once */
+} semk_bdiag;
+
+/* semk_poisson_apply_f64, then y[node[k]] += val[k] u[node[k]] on every node that the flags
+ * do not mask (a Dirichlet node under SEMK_MASK_IN or SEMK_MASK_OUT gets nothing; flags == 0:
+ * every node, the unmasked operator).  dot_out includes the term (deterministic, fixed-order
+ * reduction).  bdiag == NULL or bdiag->n == 0: exactly the launches of
+ * semk_poisson_apply_f64. */
+int semk_poisson_apply_bdiag_f64(const semk_op *op, const semk_bdiag *bdiag, const double *u,
+                                 double *y, int flags, double *dot_out, void *stream);
+/* semk_pcg_solve_f64 on M (A + diag) M + (I - M) (graph-captured like it). */
+int semk_pcg_solve_bdiag_f64(const semk_op *op, const semk_bdiag *bdiag, const double *b,
+                             double *x, const double *dinv, double *work, double *sc,
+                             double *vec_partials, double rtol, int maxiter, int check_every,
+                             semk_pcg_info *info, void *stream);
+
+/* ------------------------------------------------------------------------
  * Static condensation on the device (SURVEY.md 8(f) row 1): the reference's
  * actual solver formulation, DOFManagerSC (sem/discrete.py:283-528).  Element
  * interiors are eliminated element by element,
@@ -551,6 +579,12 @@ int semk_sc_apply_f64(const semk_sc_op *op, const double *u, double *y, int flag
  * fill_dirichlet on Dirichlet rows. */
 int semk_sc_assemble_f64(const semk_sc_op *op, const double *loc, double *out, int flags,
                          double fill_dirichlet, void *stream);
+
+/* out[i] = sum of vals[pos[q]], q in [ptr[i], ptr[i+1]), summed in that order: the
+ * deterministic gather-sum of face-node entries (face, k) onto distinct nodes (boundary
+ * loads and Robin terms).  ptr: device uint32 [n + 1]; pos: device uint32 [ptr[n]]. */
+int semk_face_sum_f64(int64_t n, const uint32_t *ptr, const uint32_t *pos, const double *vals,
+                      double *out, void *stream);
 
 /* Jacobi-PCG on Shat = M S M + (I - M); arguments as semk_pcg_solve_f64 with vectors
  * of length n_ext. */

@@ -144,6 +144,11 @@ class semk_pcg_info(C.Structure):
                 ("rel_residual", C.c_double), ("bnorm", C.c_double)]
 
 
+class semk_bdiag(C.Structure):
+    _fields_ = [("n", C.c_int64), ("node", C.c_void_p), ("val", C.c_void_p),
+                ("partials", C.c_void_p)]
+
+
 _P, _I, _L, _D = C.c_void_p, C.c_int, C.c_int64, C.c_double
 
 # name -> (restype, argtypes); every symbol include/semk.h declares
@@ -178,7 +183,12 @@ SIGNATURES = {
     "semk_dot_f64": (_I, [_L, _P, _P, _P, _P, _P]),
     "semk_pcg_solve_f64": (_I, [C.POINTER(semk_op), _P, _P, _P, _P, _P, _P, _D, _I, _I,
                                 C.POINTER(semk_pcg_info), _P]),
-    "semk_poisson_apply_host_staged_f64": (_I, [C.POINTER(semk_op), C.POINTER(semk_stage), _I, _P, _P,
+    "semk_poisson_apply_bdiag_f64": (_I, [C.POINTER(semk_op), C.POINTER(semk_bdiag), _P, _P, _I,
+                                          _P, _P]),
+    "semk_pcg_solve_bdiag_f64": (_I, [C.POINTER(semk_op), C.POINTER(semk_bdiag), _P, _P, _P, _P,
+                                      _P, _P, _D, _I, _I, C.POINTER(semk_pcg_info), _P]),
+    "semk_face_sum_f64": (_I, [_L, _P, _P, _P, _P, _P]),
+    "semk_poisson_apply_host_staged_f64":(_I, [C.POINTER(semk_op), C.POINTER(semk_stage), _I, _P, _P,
                                                 _P, _P, _I, _P]),
     "semk_poisson_apply_host_batch_f64": (_I, [C.POINTER(semk_op), C.POINTER(semk_stage), _I, _I,
                                                C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),

@@ -162,11 +162,17 @@ def _load_key(f):
 
 class CondensedPoissonOperator(_PoissonBase):
     def __init__(self, dof_mngr, dirichlet=None, geometric_factors=None, weight=None,
-                 store_interior="auto", reaction=None, store_interior_inverse=False):
+                 store_interior="auto", reaction=None, store_interior_inverse=False, robin=None):
         """store_interior : keep W_e = A_ii^-1 A_ie of every element (12.5 KB per element at
         p = 8) so that the interior back-substitution is one streaming pass instead of a
         refactorisation per element; "auto" = when it takes less than a third of the free
-        device memory."""
+        device memory.
+
+        robin : {boundary name: alpha}, optional -- Robin condition w du/dn + alpha u = g (see
+        operators.py): ``alpha dSxW`` is added to ``reaction`` on the element-local face nodes
+        before the local Schur complements are formed, so the term reaches S_e, the vertex
+        coarse space and the aggregation level unchanged.  alpha >= 0: a scalar, nodal values
+        (n_nodes) or a callable alpha(x, y) on CUDA tensors."""
         self._store_interior = store_interior
         # store_interior_inverse: also keep A_ii^-1 of every element (19 KB at p = 8): the
         # condensed load of ANY right-hand side then is a streaming pass (semk_sc_load_stored_f64)
@@ -182,7 +188,23 @@ class CondensedPoissonOperator(_PoissonBase):
             self._react = device._f64(reaction, self.dev).reshape(self.n_elem, -1).contiguous()
             if self._react.shape[1] != self.n1 * self.n1:
                 raise ValueError("reaction must have one value per element-local node")
+        if robin:
+            self._add_robin(robin)
         self._schur_pass()
+
+    def _add_robin(self, robin):
+        """reaction += alpha dSxW on the element-local face nodes, [E, NN] in reference element
+        order.  A corner cell has one local node on two faces: the face values are summed per
+        element-local slot in a fixed order (BoundaryFaces.face_sum onto "local")."""
+        terms = self._robin_terms(robin)
+        react = (torch.zeros((self.n_elem, self.n1 * self.n1), dtype=torch.float64, device=self.dev)
+                 if self._react is None else self._react.clone())
+        flat = react.view(-1)
+        for bf, a_dsxw in terms:
+            if bf.n and int(bf.nodes[-1]) >= self.n_ext:
+                raise AssertionError("boundary nodes must be element-exterior nodes")
+            flat[bf.keys_dev] += bf.face_sum(a_dsxw, onto="local")
+        self._react = react
 
     def _init_common(self, dof_mngr, dirichlet):
         """Masks, local orders, the exterior L2G / node -> entries tables, S and the
@@ -663,11 +685,12 @@ class CondensedPoissonOperator(_PoissonBase):
         self._element_pass(_lib.SC_BACKSOLVE, u=u, f=f)
         return u
 
-    def solve(self, f=1.0, dirichlet_values=None, **pcg_kwargs):
+    def solve(self, f=1.0, dirichlet_values=None, flux=None, **pcg_kwargs):
         """The whole DOFManagerSC.solve path (sem/discrete.py:526-528): condensed
-        load, Dirichlet lifting, PCG on the exterior DOFs, interior
+        load (plus the boundary loads of ``flux = {name: g}``, which have no interior
+        entries), Dirichlet lifting, PCG on the exterior DOFs, interior
         back-substitution.  Returns (u[n_nodes], PCGInfo)."""
-        b = self.lift(self.rhs(f), dirichlet_values)
+        b = self.lift(self._load(f, flux), dirichlet_values)
         x, info = self.solve_pcg(b, **pcg_kwargs)
         return self.backsolve(x, f), info
 

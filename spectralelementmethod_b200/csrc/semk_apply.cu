@@ -470,6 +470,57 @@ extern "C" int semk_poisson_apply_f64(const semk_op *op, const double *u, double
   return SEMK_OK;
 }
 
+namespace {
+
+constexpr int kBdiagThreads = 256;
+
+// Robin diagonal on the distinct boundary nodes, after the apply has made y final:
+// y[g] += val u[g], and (dot_out) u[g] * val u[g] summed in a fixed order and added to the
+// apply's own u.y.  One thread per boundary node; a few ten thousand nodes at most per
+// operator, so this is a short gather, not a stream.
+__global__ void __launch_bounds__(kBdiagThreads)
+    bdiag_kernel(int64_t n, const uint32_t *__restrict__ node, const double *__restrict__ val,
+                 const uint8_t *__restrict__ masked, const double *__restrict__ u,
+                 double *__restrict__ y, double *__restrict__ partials,
+                 double *__restrict__ dot_out) {
+  double acc[1] = {0.0};
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t g = node[i];
+    if (masked && masked[g]) continue;
+    const double ug = u[g];
+    const double t = val[i] * ug;
+    y[g] += t;
+    acc[0] = fma(ug, t, acc[0]);
+  }
+  if (dot_out) {
+    double tot[1];
+    if (semk_finish_reduction<1>(acc, partials, tot) && threadIdx.x == 0) dot_out[0] += tot[0];
+  }
+}
+
+}  // namespace
+
+extern "C" int semk_poisson_apply_bdiag_f64(const semk_op *op, const semk_bdiag *bdiag,
+                                            const double *u, double *y, int flags,
+                                            double *dot_out, void *stream) {
+  if (!bdiag || bdiag->n == 0) return semk_poisson_apply_f64(op, u, y, flags, dot_out, stream);
+  SEMK_REQUIRE(op && bdiag->n > 0 && bdiag->n <= op->n_nodes && bdiag->node && bdiag->val,
+               "semk_poisson_apply_bdiag_f64: inconsistent semk_bdiag");
+  SEMK_REQUIRE(!dot_out || bdiag->partials,
+               "semk_poisson_apply_bdiag_f64: dot_out needs bdiag->partials");
+  int rc = semk_poisson_apply_f64(op, u, y, flags, dot_out, stream);
+  if (rc != SEMK_OK) return rc;
+  const uint8_t *masked =
+      (op->dirichlet && (flags & (SEMK_MASK_IN | SEMK_MASK_OUT))) ? op->dirichlet : nullptr;
+  const int64_t want = (bdiag->n + kBdiagThreads - 1) / kBdiagThreads;
+  const unsigned grid = (unsigned)(want < kSemkRedMaxBlocks ? want : kSemkRedMaxBlocks);
+  bdiag_kernel<<<grid, kBdiagThreads, 0, semk_stream(stream)>>>(
+      bdiag->n, bdiag->node, bdiag->val, masked, u, y, bdiag->partials, dot_out);
+  SEMK_LAUNCH_CHECK("bdiag_kernel");
+  return SEMK_OK;
+}
+
 // A sub-range of the apply: patches [patch_begin, patch_end) and the interface entries
 // [chunk_begin, chunk_end) / [rec_begin, rec_end) (both tables are sorted by the highest
 // patch involved, so "everything patches [0, P) complete" is a prefix of each).

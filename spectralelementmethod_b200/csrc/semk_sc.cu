@@ -893,6 +893,15 @@ extern "C" int semk_sc_assemble_f64(const semk_sc_op *op, const double *loc, dou
   return SEMK_OK;
 }
 
+extern "C" int semk_face_sum_f64(int64_t n, const uint32_t *ptr, const uint32_t *pos,
+                                 const double *vals, double *out, void *stream) {
+  SEMK_REQUIRE(n > 0 && ptr && pos && vals && out, "semk_face_sum_f64: bad argument");
+  sc_node_kernel<<<node_blocks(n), kNodeThreads, 0, semk_stream(stream)>>>(
+      n, ptr, pos, vals, nullptr, nullptr, out, 0, 0.0, nullptr, nullptr);
+  SEMK_LAUNCH_CHECK("sc_node_kernel");
+  return SEMK_OK;
+}
+
 extern "C" int semk_sc_coarse_elem_f64(const semk_sc_op *op, const double *phi, double *Ace_out,
                                        void *stream) {
   int rc = check_sc_op(op, "semk_sc_coarse_elem_f64");

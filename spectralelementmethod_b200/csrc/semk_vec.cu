@@ -457,6 +457,25 @@ extern "C" int semk_pcg_solve_f64(const semk_op *op, const double *b, double *x,
                         rtol, maxiter, check_every, info, st);
 }
 
+// The same loop with the Robin boundary diagonal in every apply (and in pAp).
+extern "C" int semk_pcg_solve_bdiag_f64(const semk_op *op, const semk_bdiag *bdiag,
+                                        const double *b, double *x, const double *dinv,
+                                        double *work, double *sc, double *vec_partials,
+                                        double rtol, int maxiter, int check_every,
+                                        semk_pcg_info *info, void *stream) {
+  SEMK_REQUIRE(op && b && x && dinv && work && sc && vec_partials && info,
+               "semk_pcg_solve_bdiag_f64: null pointer");
+  SEMK_REQUIRE(maxiter >= 0 && check_every >= 1 && rtol >= 0.0,
+               "semk_pcg_solve_bdiag_f64: bad control");
+  cudaStream_t st = semk_stream(stream);
+  const int flags = SEMK_MASK_IN | SEMK_MASK_OUT | SEMK_DIRICHLET_IDENTITY;
+  auto apply = [&](const double *in, double *out, double *dot) -> int {
+    return semk_poisson_apply_bdiag_f64(op, bdiag, in, out, flags, dot, st);
+  };
+  return pcg_solve_impl(apply, op->n_nodes, op->dirichlet, b, x, dinv, work, sc, vec_partials,
+                        rtol, maxiter, check_every, info, st);
+}
+
 // The same loop on the statically condensed operator Shat = M S M + (I - M) over the
 // element-exterior DOFs (sem/discrete.py:502-511 solves that system with SuperLU).
 extern "C" int semk_sc_pcg_solve_f64(const semk_sc_op *op, const double *b, double *x,

@@ -11,7 +11,8 @@ import torch
 
 from . import _lib
 
-__all__ = ["stream_ptr", "as_i32_bits", "basis_tables", "element_geometry", "ptr"]
+__all__ = ["stream_ptr", "as_i32_bits", "basis_tables", "element_geometry", "ptr",
+           "boundary_face_tables", "csr_by_key", "BoundaryFaces"]
 
 
 def stream_ptr():
@@ -138,6 +139,110 @@ def stiffness_factors(tab, mesh, l2g_dev, n_slots, G, g_stride, elems_per_patch,
         n1, n_slots, ptr(w), ptr(elem_of_slot), ptr(G), g_stride, elems_per_patch,
         stream_ptr()))
     torch.cuda.current_stream().synchronize()
+
+
+def boundary_face_tables(mesh, name):
+    """Faces of the named boundary, in the order ``DOFManager.boundary_elements(name)`` visits
+    them (cells ascending, the faces of a cell in registration order).  Pure NumPy.
+
+    Returns ``cells[F]``, ``faces[F]`` (0:W 1:E 2:S 3:N), and per face ``nodes[F, n1]`` (uint32
+    node ids) and ``local[F, n1]`` (element-local lexicographic indices) of its GLL nodes in the
+    reference orientation of ``mapping._subface_slice`` (faces 0 and 3 reversed).  An unknown
+    name raises the ``KeyError`` of ``boundary_elements``."""
+    from .mapping import _subface_slice
+    bnd_id = mesh._boundary_id_lookup[name]
+    maps = mesh.node_map_array()
+    if maps.ndim != 3 or maps.shape[1] != maps.shape[2]:
+        raise NotImplementedError("boundary tables need 2-D cells with the same order in both "
+                                  "directions")
+    n1 = int(maps.shape[1])
+    pairs = sorted(mesh._boundary_faces[bnd_id], key=lambda cf: cf[0])      # stable
+    cells = np.array([c for c, _ in pairs], dtype=np.int64)
+    faces = np.array([f for _, f in pairs], dtype=np.int64)
+    lin = np.arange(n1 * n1, dtype=np.int64).reshape(n1, n1)
+    local = np.empty((cells.size, n1), dtype=np.int64)
+    for f in range(4):
+        local[faces == f] = _subface_slice(f, lin, 2)
+    nodes = maps.reshape(-1, n1 * n1)[cells[:, None], local]
+    return cells, faces, np.ascontiguousarray(nodes, dtype=np.uint32), local
+
+
+def csr_by_key(keys):
+    """Group the entries of ``keys`` (any shape; entry i is ``keys.ravel()[i]``) by value:
+    ``uniq`` ascending, and ``pos[ptr[j]:ptr[j+1]]`` the flat positions of the entries equal to
+    ``uniq[j]``, ascending.  Pure NumPy.  That is the fixed summation order in which
+    ``semk_face_sum_f64`` adds face-node entries onto nodes."""
+    flat = np.asarray(keys).ravel()
+    if flat.size >= 2 ** 32:
+        raise NotImplementedError("more than 2^32 face-node entries")
+    pos = np.argsort(flat, kind="stable").astype(np.uint32)
+    uniq, counts = np.unique(flat, return_counts=True)
+    ptr = np.zeros(uniq.size + 1, dtype=np.uint32)
+    np.cumsum(counts, out=ptr[1:])
+    return uniq, ptr, pos
+
+
+class BoundaryFaces(object):
+    """Face tables of one named boundary on the device (``boundary_face_tables``), with:
+
+    * ``x [F, 2, n1]``: physical coordinates of the face nodes, and ``dSxW [F, n1]``: the face's
+      GLL weight times ``|dx/dxi_t|`` -- the host mirror's ``SubFiniteElement.x_phys`` /
+      ``dSxW``.  K1 runs on the boundary cells only (as ``DOFManager.boundary_elements`` does)
+      and the face slice and the tangent length follow ``SubMapping._tangents``.
+    * ``nodes``: the distinct boundary nodes, ascending, and ``keys``: the distinct
+      element-local slots ``cell * NN + local`` of the face nodes; ``face_sum`` adds
+      face-node values ``[F, n1]`` onto either in a fixed order (``csr_by_key``)."""
+
+    def __init__(self, tab, mesh, name, dev):
+        n1, NN = tab.n1, tab.n1 * tab.n1
+        self.name = name
+        self.cells, self.faces, self.node_ids, self.local = boundary_face_tables(mesh, name)
+        if self.node_ids.shape[1] != n1:
+            raise ValueError("the mesh and the basis have different orders")
+        F = self.n_faces = int(self.cells.size)
+        self.dev = dev
+        self.nodes, ptr, pos = csr_by_key(self.node_ids)
+        self.n = int(self.nodes.size)
+        self._csr = {"nodes": (self.n, as_i32_bits(ptr, dev), as_i32_bits(pos, dev))}
+        keys, kptr, kpos = csr_by_key(self.cells[:, None] * NN + self.local)
+        self.keys = keys
+        self._csr["local"] = (int(keys.size), as_i32_bits(kptr, dev), as_i32_bits(kpos, dev))
+        self.nodes_dev = torch.from_numpy(self.nodes.astype(np.int64)).to(dev)
+        self.keys_dev = torch.from_numpy(keys.astype(np.int64)).to(dev)
+        self.node_ids_dev = torch.from_numpy(self.node_ids.astype(np.int64)).to(dev)
+        f64 = dict(dtype=torch.float64, device=dev)
+        self.x = torch.empty((F, 2, n1), **f64)
+        self.dSxW = torch.empty((F, n1), **f64)
+        if F == 0:
+            return
+        l2g = as_i32_bits(mesh.node_map_array().reshape(-1, NN)[self.cells], dev)
+        nodes_dev = torch.from_numpy(np.ascontiguousarray(mesh.nodes, dtype=np.float64)).to(dev)
+        x_phys = torch.empty((F, 2, NN), **f64)
+        J = torch.empty((F, 2, 2, NN), **f64)
+        geom_factors(tab, nodes_dev, l2g, F, x_phys=x_phys, J=J)
+        loc = torch.from_numpy(self.local).to(dev)[:, None, :].expand(F, 2, n1)
+        self.x.copy_(torch.gather(x_phys, 2, loc))
+        # the face runs along parametric direction 1 - face // 2: that column of J is the
+        # (unnormalised) tangent
+        along = torch.from_numpy(1 - self.faces // 2).to(dev)
+        tan = torch.gather(J[torch.arange(F, device=dev), :, along, :], 2, loc)
+        dS = torch.sqrt(tan[:, 0] * tan[:, 0] + tan[:, 1] * tan[:, 1])
+        self.dSxW.copy_(dS * _f64(tab.w_host, dev)[None, :])
+
+    def face_sum(self, vals, onto="nodes"):
+        """Sum face-node values ``vals [F, n1]`` onto the distinct boundary nodes (``onto =
+        "nodes"``, order of ``nodes``) or element-local slots (``"local"``, order of ``keys``);
+        a fixed-order sum on the device (semk_face_sum_f64): bitwise reproducible."""
+        n, row_ptr, pos = self._csr[onto]
+        out = torch.empty(n, dtype=torch.float64, device=self.dev)
+        if n == 0:
+            return out
+        vals = vals.to(dtype=torch.float64).contiguous()
+        if vals.numel() != self.n_faces * self.node_ids.shape[1]:
+            raise ValueError("face values must be [n_faces, n1]")
+        _lib.check(_lib.load().semk_face_sum_f64(n, ptr(row_ptr), ptr(pos), ptr(vals), ptr(out),
+                                                 stream_ptr()))
+        return out
 
 
 def element_geometry(basis, nodes, l2g, jacobian=True):

@@ -394,6 +394,11 @@ class DOFManager(object):
             callable ``w(x, y)`` on device tensors -- the operator becomes the
             stiffness of -div(w grad u) (the rho-weighted twin of the recipe,
             examples/squirmer-axisymmetric.py:194-213).
+        robin (keyword) : {boundary name: alpha} -- Robin condition
+            w du/dn + alpha u = g on those boundaries (alpha >= 0; scalar, nodal values or a
+            callable alpha(x, y)).  Flux data g of flux or Robin boundaries goes to
+            ``op.solve(flux={name: g})`` or ``op.boundary_load(name, g)``; see
+            operators.py for the weak form.
         """
         if self._dpn != 1:
             raise NotImplementedError("poisson_operator supports one DOF per node")
@@ -532,6 +537,9 @@ class DOFManagerSC(DOFManager):
 
         dirichlet : bool[n_nodes] or bool[ndof_exterior], optional -- True on
             essential-BC nodes (the ``on_ebc`` polarity of ``solve``).
+        robin (keyword) : {boundary name: alpha} -- Robin condition
+            w du/dn + alpha u = g, as for ``poisson_operator``; the term enters the local
+            Schur complements through the element reaction diagonal.
         """
         from .condensed import CondensedPoissonOperator
         return CondensedPoissonOperator(self, dirichlet=dirichlet, **kwargs)

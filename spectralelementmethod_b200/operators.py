@@ -11,6 +11,23 @@ whole path on one GPU:
     b  = op.rhs(f=1.0)                    # assembled load vector  Q^T (JxW f)
     x, info = op.solve_pcg(op.lift(b, g)) # Jacobi-PCG, Dirichlet data g lifted
 
+Boundary conditions.  With the operator's weight ``w`` (1 unless ``weight=`` was given) both
+operators here and in condensed.py solve
+
+    -div(w grad u) = f                      in the domain
+    u = u_D                                 on Dirichlet nodes
+    w du/dn = g                             on boundaries given only flux data
+    w du/dn + alpha u = g                   on Robin boundaries (alpha >= 0)
+
+and homogeneous Neumann everywhere else.  The weak form adds
+``sum_faces sum_k g(x_k) dSxW_k v(x_k)`` to the load (``boundary_load``; ``solve(flux={name:
+g})``) and ``alpha(x_k) dSxW_k`` to the diagonal at face node k (``robin={name: alpha}`` of the
+constructor).  ``dSxW`` is the face's GLL weight times ``|dx/dxi_t|``, the host mirror's
+``SubFiniteElement.dSxW`` (same face numbering 0:W 1:E 2:S 3:N, same orientation); the face
+quadrature is collocated at the GLL nodes like the volume mass, so the Robin term is
+diagonal.  Dirichlet wins on a node that is also on a flux or Robin face: ``lift`` discards
+the load there and the Robin diagonal enters no masked row or column.
+
 Vectors are ``torch.float64`` CUDA tensors of length ``n_nodes`` in the
 reference's global node order (whatever numbering the DOF manager produced:
 lexicographic, exterior-first, RCM).  Every number is computed by the CUDA
@@ -225,11 +242,76 @@ class _PoissonBase(object):
             x[mask] = b[mask]
         return x
 
+    # -- flux and Robin boundaries -----------------------------------------------------
+    def boundary_faces(self, name):
+        """Device face tables of the named boundary (device.BoundaryFaces), built on first
+        use and kept.  An unknown name raises the ``KeyError`` of ``boundary_elements``."""
+        cache = self.__dict__.setdefault("_bfaces", {})
+        if name not in cache:
+            cache[name] = device.BoundaryFaces(self.tab, self.dof_mngr.mesh, name, self.dev)
+        return cache[name]
+
+    def _face_values(self, bf, g, what):
+        """``g`` on the face nodes of ``bf`` as a [F, n1] CUDA tensor: a scalar, nodal values
+        (CUDA tensor or host array of n_nodes entries), or a callable ``g(x, y)`` on CUDA tensors
+        of the face-node coordinates (the convention of a callable ``weight``)."""
+        shape = (bf.n_faces, self.n1)
+        if callable(g):
+            v = g(bf.x[:, 0, :], bf.x[:, 1, :])
+            return torch.as_tensor(v, dtype=torch.float64, device=self.dev).expand(shape)
+        if isinstance(g, torch.Tensor) or np.ndim(g) != 0:
+            gv = g if isinstance(g, torch.Tensor) else self.from_host(g)
+            return self._vec(gv, what, self.n_nodes)[bf.node_ids_dev]
+        return torch.full(shape, float(g), dtype=torch.float64, device=self.dev)
+
+    def boundary_load(self, name, g):
+        """Load of the flux condition ``w du/dn = g`` on the named boundary: the vector of the
+        operator's length with ``sum_faces sum_k g(x_k) dSxW_k`` on every face node (the
+        reference recipe ``b[bfe.node_ind] += g * bfe.dSxW`` over
+        ``boundary_elements(name)``), summed over the faces in a fixed order.  ``g``: a scalar,
+        nodal values (n_nodes) or a callable ``g(x, y)`` on CUDA tensors."""
+        bf = self.boundary_faces(name)
+        out = self.new_vector(0.0)
+        if bf.n == 0:
+            return out
+        if int(bf.nodes[-1]) >= self._n_vec:
+            raise AssertionError("boundary nodes must be element-exterior nodes")
+        out[bf.nodes_dev] = bf.face_sum(self._face_values(bf, g, "g") * bf.dSxW)
+        return out
+
+    def _robin_terms(self, robin):
+        """[(BoundaryFaces, alpha dSxW [F, n1])] of ``robin = {name: alpha}``; alpha in the
+        forms of ``boundary_load``, >= 0 on every face node."""
+        terms = []
+        for name, alpha in dict(robin).items():
+            if not callable(alpha) and np.ndim(alpha) == 0 and not float(alpha) >= 0.0:
+                raise ValueError("the Robin coefficient of %r must be >= 0" % (name,))
+            bf = self.boundary_faces(name)
+            if bf.n_faces == 0:
+                continue
+            a = self._face_values(bf, alpha, "alpha")
+            if not bool((a >= 0.0).all()):
+                raise ValueError("the Robin coefficient of %r must be >= 0" % (name,))
+            terms.append((bf, (a * bf.dSxW).contiguous()))
+        return terms
+
+    def _load(self, f, flux):
+        """rhs(f) plus the boundary load of every ``flux = {name: g}`` entry, in dict order."""
+        b = self.rhs(f)
+        for name, g in (flux or {}).items():
+            b += self.boundary_load(name, g)
+        return b
+
 
 class PoissonOperator(_PoissonBase):
     def __init__(self, dof_mngr, dirichlet=None, geometric_factors=None, elems_per_patch=None,
                  elem_order=None, keep_l2g=True, tile=None, weight=None, mode="auto",
-                 boundary_columns_first=False):
+                 boundary_columns_first=False, robin=None):
+        """robin : {boundary name: alpha}, optional -- Robin condition w du/dn + alpha u = g
+            on those boundaries: ``alpha dSxW`` joins the diagonal of every face node
+            (semk_bdiag).  alpha >= 0: a scalar, nodal values (n_nodes) or a callable
+            alpha(x, y) on CUDA tensors.  The load g goes to ``solve(flux=...)`` /
+            ``boundary_load``."""
         _lib.require_device()
         self._lib = _lib.load()
         mesh = dof_mngr.mesh
@@ -386,8 +468,37 @@ class PoissonOperator(_PoissonBase):
         self._op = op
         self._masked_flags = (MASK_IN | MASK_OUT | DIRICHLET_IDENTITY) if self.has_dirichlet else 0
         self._dinv = None
+        self._bdiag = None
+        if robin:
+            self._init_robin(robin)
 
     # -- helpers ---------------------------------------------------------------------
+    def _init_robin(self, robin):
+        """semk_bdiag of the Robin boundaries: the distinct nodes of all of them, ascending,
+        and their assembled sum of alpha dSxW (per boundary a fixed-order face sum, then the
+        boundaries in dict order)."""
+        dense = self.new_vector(0.0)
+        node_sets = [np.zeros(0, dtype=np.uint32)]
+        for bf, a_dsxw in self._robin_terms(robin):
+            dense[bf.nodes_dev] += bf.face_sum(a_dsxw)
+            node_sets.append(bf.nodes)
+        nodes = np.unique(np.concatenate(node_sets))
+        self._bd_node = device.as_i32_bits(nodes, self.dev)
+        self._bd_val = dense[torch.from_numpy(nodes.astype(np.int64)).to(self.dev)].contiguous()
+        self._bd_partials = torch.zeros(int(self._lib.semk_vec_partials_len(nodes.size)),
+                                        dtype=torch.float64, device=self.dev)
+        bd = _lib.semk_bdiag()
+        bd.n = int(nodes.size)
+        bd.node = self._bd_node.data_ptr()
+        bd.val = self._bd_val.data_ptr()
+        bd.partials = self._bd_partials.data_ptr()
+        self._bdiag = bd
+
+    def _no_robin(self, what):
+        if self._bdiag is not None:
+            raise NotImplementedError("%s does not include the Robin boundary term; use apply / "
+                                      "solve_pcg of this operator" % what)
+
     def _mark_box_patches(self, l2g, t):
         """kernel_variant 2 (csrc/semk_box.cu): find the patches that are regular tile boxes
         -- node (m, t) of slot le = lx*by + ly has the id base + (lx*p + m)*ld + ly*p + t --
@@ -440,11 +551,17 @@ class PoissonOperator(_PoissonBase):
         """y = Ahat u with Ahat = M A M + (I - M) (A if no Dirichlet mask).
         ``flags`` overrides the masking (bit-or of MASK_IN, MASK_OUT,
         DIRICHLET_IDENTITY; 0 = the pure Neumann operator A).  ``dot_out``:
-        optional 1-element device tensor receiving u.y."""
+        optional 1-element device tensor receiving u.y.  A Robin operator adds its boundary
+        diagonal on the rows and columns the flags leave unmasked."""
         self._vec(u, "u")
         y = self.new_vector() if out is None else self._vec(out, "out")
         if flags is None:
             flags = self._masked_flags
+        if self._bdiag is not None:
+            _lib.check(self._lib.semk_poisson_apply_bdiag_f64(
+                C.byref(self._op), C.byref(self._bdiag), device.ptr(u), device.ptr(y), int(flags),
+                device.ptr(dot_out), device.stream_ptr()))
+            return y
         _lib.check(self._lib.semk_poisson_apply_f64(
             C.byref(self._op), device.ptr(u), device.ptr(y), int(flags), device.ptr(dot_out),
             device.stream_ptr()))
@@ -452,6 +569,7 @@ class PoissonOperator(_PoissonBase):
 
     def apply_atomic(self, u, out=None, flags=None):
         """Same operator through the independent atomic-scatter kernel."""
+        self._no_robin("apply_atomic")
         if self.l2g_dev is None:
             raise RuntimeError("operator was built with keep_l2g=False")
         self._vec(u, "u")
@@ -495,6 +613,7 @@ class PoissonOperator(_PoissonBase):
         mesh whose plan was built with ``boundary_columns_first``: the patches that touch the
         first / last node column and the prefixes of the interface tables they complete.
         None when the plan has no such prefix."""
+        self._no_robin("boundary_split (the halo-overlapped apply)")
         if not getattr(self, "_boundary_first", False):
             return None
         shape = getattr(self.dof_mngr.mesh, "_structured_shape", None)
@@ -509,6 +628,7 @@ class PoissonOperator(_PoissonBase):
 
     def apply_range(self, u, y, pb, pe, cb, ce, rb, re, flags=None):
         """Patches [pb, pe) and interface entries [cb, ce) / [rb, re) of the apply."""
+        self._no_robin("apply_range")
         if flags is None:
             flags = self._masked_flags
         _lib.check(self._lib.semk_poisson_apply_range_f64(
@@ -522,6 +642,7 @@ class PoissonOperator(_PoissonBase):
         ``stages`` > 1 the three phases are pipelined over that many runs of
         patches (upload of the next run and download of the previous one
         overlap the compute; semk_poisson_apply_host_staged_f64)."""
+        self._no_robin("apply_host")
         if scratch is None:
             scratch = (self.new_vector(), self.new_vector())
         if stages and stages > 1:
@@ -542,6 +663,7 @@ class PoissonOperator(_PoissonBase):
         device scratch sets, so that the upload of apply k+1 overlaps the download of apply
         k (semk_poisson_apply_host_batch_f64).  ``scratch``: four device vectors
         (d_u0, d_y0, d_u1, d_y1) or None.  Synchronised on return."""
+        self._no_robin("apply_host_many")
         if len(u_hosts) != len(y_hosts):
             raise ValueError("u_hosts and y_hosts must have the same length")
         n = len(u_hosts)
@@ -571,16 +693,25 @@ class PoissonOperator(_PoissonBase):
         return y
 
     def diagonal(self, masked=True):
-        """diag(Ahat) (masked: 1 on Dirichlet rows) or diag(A)."""
+        """diag(Ahat) (masked: 1 on Dirichlet rows) or diag(A), Robin diagonal included."""
         loc = torch.empty((self.n_slot_elems, self.n1 * self.n1), dtype=torch.float64,
                           device=self.dev)
         _lib.check(self._lib.semk_poisson_local_diag_f64(
             C.byref(self._op), device.ptr(self.tab.dev()[0]), device.ptr(loc), device.stream_ptr()))
-        return self.assemble(loc, mask=masked and self.has_dirichlet, fill_dirichlet=1.0)
+        mask = masked and self.has_dirichlet
+        d = self.assemble(loc, mask=mask, fill_dirichlet=1.0)
+        if self._bdiag is not None and self._bdiag.n > 0:
+            nodes = self._bd_node.long() & 0xFFFFFFFF
+            val = self._bd_val
+            if mask:
+                val = torch.where(self.dirichlet_dev[nodes].bool(), torch.zeros_like(val), val)
+            d[nodes] += val
+        return d
 
     def rhs(self, f=1.0):
         """Load vector b = Q^T (JxW . f); ``f`` a scalar or nodal values
-        (examples/poisson.py:200 uses f = 1).  No boundary treatment."""
+        (examples/poisson.py:200 uses f = 1).  The volume load only: flux and Robin data enter
+        through ``boundary_load`` (``solve(flux=...)``)."""
         fv = None
         scale = 1.0
         if isinstance(f, torch.Tensor):
@@ -618,17 +749,24 @@ class PoissonOperator(_PoissonBase):
         work = torch.empty(3 * (self.n_nodes + 32), dtype=torch.float64, device=self.dev)
         sc = torch.zeros(8, dtype=torch.float64, device=self.dev)
         info = _lib.semk_pcg_info()
-        rc = self._lib.semk_pcg_solve_f64(
-            C.byref(self._op), device.ptr(b), device.ptr(x), device.ptr(dinv), device.ptr(work),
-            device.ptr(sc), device.ptr(self.vec_partials), float(rtol), int(maxiter),
-            int(check_every), C.byref(info), device.stream_ptr())
+        if self._bdiag is not None:
+            rc = self._lib.semk_pcg_solve_bdiag_f64(
+                C.byref(self._op), C.byref(self._bdiag), device.ptr(b), device.ptr(x),
+                device.ptr(dinv), device.ptr(work), device.ptr(sc), device.ptr(self.vec_partials),
+                float(rtol), int(maxiter), int(check_every), C.byref(info), device.stream_ptr())
+        else:
+            rc = self._lib.semk_pcg_solve_f64(
+                C.byref(self._op), device.ptr(b), device.ptr(x), device.ptr(dinv),
+                device.ptr(work), device.ptr(sc), device.ptr(self.vec_partials), float(rtol),
+                int(maxiter), int(check_every), C.byref(info), device.stream_ptr())
         _lib.check(rc)
         return x, PCGInfo(info.iterations, info.status, info.rel_residual, info.bnorm)
 
-    def solve(self, f=1.0, dirichlet_values=None, **pcg_kwargs):
-        """Poisson solve in one call: assemble the load, lift the Dirichlet
-        data, run PCG.  Returns (u, PCGInfo)."""
-        b = self.lift(self.rhs(f), dirichlet_values)
+    def solve(self, f=1.0, dirichlet_values=None, flux=None, **pcg_kwargs):
+        """Poisson solve in one call: assemble the load, add the boundary loads of ``flux =
+        {name: g}`` (``boundary_load``), lift the Dirichlet data, run PCG.  Returns (u,
+        PCGInfo)."""
+        b = self.lift(self._load(f, flux), dirichlet_values)
         return self.solve_pcg(b, **pcg_kwargs)
 
     # -- small-mesh test helper ----------------------------------------------------------
