@@ -12,7 +12,7 @@ the matrix-free device operator and the device-resident Jacobi-PCG.
 
     python examples/poisson.py [--n 64] [--order 8] [--msh file.msh] [--kind S|C]
                                [--solver matrix-free|condensed|condensed-two-level]
-                               [--bc reference|neumann|robin]
+                               [--bc reference|neumann|robin] [--convergence]
 
 ``--solver condensed`` follows the reference example literally: static
 condensation of the element interiors (DOFManagerSC, sem/discrete.py:404-528),
@@ -22,7 +22,10 @@ solve on the element-exterior DOFs, interior back-substitution -- on the device;
 ``--bc neumann`` / ``--bc robin`` solve a manufactured problem instead: u smooth and known,
 f = -lap(u) as nodal values, u on "ebc", and on "nbc" the flux condition du/dn = g
 (``neumann``) or the Robin condition du/dn + 2 u = g (``robin``) with g taken from u; the
-max nodal error against u is printed.
+max nodal, L2 and H1 errors against u are printed (``DOFManager.error_norms``), and the flux
+of the solution through "nbc" (``DOFManager.boundary_flux``) beside the integral of the
+exact flux.  ``--convergence`` solves that problem on the same mesh for p = 2 ... 10 and
+prints one row per order: the errors fall exponentially in p.
 
 With ``--msh`` the mesh is read from a Gmsh 2.2 binary file with physical
 names "ebc", "nbc" (lines) and a surface (the reference's examples/meshes/
@@ -52,28 +55,26 @@ def f_exact(x, y):
     return 0.81 * (np.cos(0.9 * x + 0.3) + np.cos(0.9 * y + 0.3)) + 0.49 * np.sin(0.7 * (x + y))
 
 
+def _du(s, t):
+    import torch
+    return -0.9 * torch.sin(0.9 * s + 0.3) + 0.35 * torch.cos(0.7 * (s + t))
+
+
+def grad_exact(x, y):
+    """Gradient of ``u_exact`` on CUDA tensors."""
+    return _du(x, y), _du(y, x)
+
+
 def flux_nbc(x, y):
     """du/dn on "nbc" (right side: du/dx; top side: du/dy) on CUDA tensors."""
     import torch
-
-    def du(s, t):
-        return -0.9 * torch.sin(0.9 * s + 0.3) + 0.35 * torch.cos(0.7 * (s + t))
-    return torch.where(x >= y, du(x, y), du(y, x))
-
-
-def gll_coordinates(mngr):
-    """Physical coordinates of every GLL node (the solution's nodes), [2, n_nodes]."""
-    from spectralelementmethod_b200 import device
-    mesh = mngr.mesh
-    l2g = mesh.node_map_array().reshape(mesh.n_cells, -1).astype(np.int64)
-    xp = device.element_geometry(mngr._basis, mesh.nodes, l2g, jacobian=False)["x_phys"]
-    X = np.zeros((2, mesh.n_nodes))
-    X[:, l2g.ravel()] = xp.reshape(mesh.n_cells, 2, -1).transpose(1, 0, 2).reshape(2, -1)
-    return X
+    return torch.where(x >= y, _du(x, y), _du(y, x))
 
 
 def run(n=16, order=8, msh=None, kind="S", write_msh=None, rtol=1e-12, quiet=False,
-        solver="matrix-free", bc="reference"):
+        solver="matrix-free", bc="reference", report=None):
+    """Solve; returns (mngr, on_ebc, essential values, u, info).  With ``bc`` neumann / robin,
+    ``report`` (a dict, if given) receives the error norms and the "nbc" fluxes."""
     import torch
     t0 = time.perf_counter()
     if msh is None and write_msh is not None:
@@ -96,7 +97,7 @@ def run(n=16, order=8, msh=None, kind="S", write_msh=None, rtol=1e-12, quiet=Fal
             soln[loc] = 0.2 * ((x + 1) + (y + 1))
             on_ebc[loc] = True
     elif bc in ("neumann", "robin"):
-        X = gll_coordinates(mngr)
+        X = mngr.node_coordinates().cpu().numpy()
         on_ebc = mngr.boundary_node_mask("ebc")
         soln = u_exact(X[0], X[1])
         f = torch.from_numpy(f_exact(X[0], X[1])).cuda()
@@ -122,6 +123,11 @@ def run(n=16, order=8, msh=None, kind="S", write_msh=None, rtol=1e-12, quiet=Fal
                        **extra)
     torch.cuda.synchronize()
     t_solve = time.perf_counter() - t0
+    post = {} if report is None else report
+    if bc != "reference":
+        post.update(mngr.error_norms(u, lambda x, y: u_exact(x, y, torch), grad_exact),
+                    flux=mngr.boundary_flux(u, "nbc"),
+                    flux_exact=float(op.boundary_load("nbc", flux_nbc).sum()))
     u = u.cpu().numpy()
     if not quiet:
         print("mesh: %d cells of order %d, %d DOF (%d on the essential boundary)"
@@ -131,7 +137,24 @@ def run(n=16, order=8, msh=None, kind="S", write_msh=None, rtol=1e-12, quiet=Fal
         print("u: min %.6f  max %.6f  mean %.6f" % (u.min(), u.max(), u.mean()))
         if bc != "reference":
             print("%s boundary on \"nbc\": max nodal error %.3e" % (bc, np.abs(u - soln).max()))
+            print("errors: L2 %.3e  H1 semi-norm %.3e" % (post["l2"], post["h1_semi"]))
+            print("flux through \"nbc\": %.15f (integral of the exact flux %.15f)"
+                  % (post["flux"], post["flux_exact"]))
     return mngr, on_ebc, soln, u, info
+
+
+def convergence(n=8, kind="S", solver="matrix-free", bc="neumann", orders=range(2, 11)):
+    """The manufactured problem of ``--bc neumann|robin`` on one structured n x n mesh for
+    every order: one row of errors per order."""
+    print("%3s %9s %6s %11s %11s %11s %11s" % ("p", "DOF", "iters", "max nodal", "L2", "H1 semi",
+                                               "flux error"))
+    for p in orders:
+        rep = {}
+        mngr, _on_ebc, _soln, _u, info = run(n, p, None, kind, rtol=1e-13, quiet=True,
+                                             solver=solver, bc=bc, report=rep)
+        print("%3d %9d %6d %11.3e %11.3e %11.3e %11.3e"
+              % (p, mngr.ndof, info.iterations, rep["max_nodal"], rep["l2"], rep["h1_semi"],
+                 abs(rep["flux"] - rep["flux_exact"])))
 
 
 def main():
@@ -146,7 +169,14 @@ def main():
     ap.add_argument("--bc", default="reference", choices=["reference", "neumann", "robin"],
                     help="reference: the reference example (du/dn = 0 on \"nbc\"); neumann / "
                          "robin: a manufactured problem with flux / Robin data on \"nbc\"")
+    ap.add_argument("--convergence", action="store_true",
+                    help="solve the manufactured problem (--bc neumann unless robin is given) "
+                         "for p = 2 ... 10 on the structured --n x --n mesh and print the "
+                         "errors per order")
     args = ap.parse_args()
+    if args.convergence:
+        convergence(args.n, args.kind, args.solver, "robin" if args.bc == "robin" else "neumann")
+        return
     run(args.n, args.order, args.msh, args.kind, args.write_msh, solver=args.solver, bc=args.bc)
 
 

@@ -270,6 +270,33 @@ int semk_geom_factors_f64(int n1, int64_t n_elem, const double *nodes_x, const d
                           double *x_phys, double *J, double *invJ, double *detJ,
                           int32_t *bad_flag, void *stream);
 
+/* Nodal fields after a solve: K1's geometry recomputed (the same device arithmetic, so
+ * nothing per element is kept between calls), then the physical gradient of a nodal
+ * vector u, grad u = invJ^T (D u, u D^T) -- FiniteElement.gradient (sem/discrete.py:680-684).
+ * One pass over the elements `elems` (device int64 [n_elem], NULL = all, in order), one CTA
+ * per element.  Replaces, with n_nodes-long device vectors and every output optional
+ * (NULL = skip):
+ *   xy [2][n_nodes]: GLL-node coordinates, x_phys written at the entries whose winner byte
+ *     is set (winner as in semk_values_at_nodes_f64: the last element containing a node);
+ *     the loop `X[:, node_ind] = fe.x_phys` over finite_elements(x_phys=True).
+ *   grad_loc [2][n_elem][NN] (component-major, element in list order): grad u per element
+ *     (fe.gradient(u[fe.node_ind])), times JxW when `weighted` (for the JxW-weighted nodal
+ *     average: sum each component and jxw_loc onto nodes with semk_face_sum_f64);
+ *     jxw_loc [n_elem][NN]: JxW (fe.detJxW).
+ *   sums [5] (device): sum over elements of fe.integrate((u - u_ref)^2),
+ *     fe.integrate(|grad u - g_ref|^2), max |u - u_ref| over the nodes,
+ *     fe.integrate(u_ref^2), fe.integrate(|g_ref|^2); u_ref [n_nodes] and g_ref
+ *     [2][n_nodes] nodal, NULL = 0.  GLL collocation quadrature, as the reference's.
+ *     Fixed-order reduction: bitwise reproducible.  partials: semk_vec_partials_len()
+ *     doubles, zeroed once; no other call may use them concurrently.
+ * u may be NULL when only xy is asked for.  bad_flag as in semk_geom_factors_f64. */
+int semk_field_grad_f64(int n1, int64_t n_elem, const double *nodes_x, const double *nodes_y,
+                        const uint32_t *l2g, const double *Einv, const double *D, const double *w,
+                        const int64_t *elems, int64_t n_nodes, const double *u,
+                        const uint8_t *winner, double *xy, double *grad_loc, int weighted,
+                        double *jxw_loc, const double *u_ref, const double *g_ref, double *sums,
+                        double *partials, int32_t *bad_flag, void *stream);
+
 /* G (engine slot layout) from externally supplied factors in the reference's
  * layouts: invJ [n_elem][2][2][NN] (fe.invJ) and JxW [n_elem][NN]
  * (fe.detJxW).  Parity tier T1 (SURVEY.md 8c). */

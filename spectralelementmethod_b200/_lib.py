@@ -167,6 +167,8 @@ SIGNATURES = {
     "semk_resident_ctas_variant": (_L, [_I, _I, _I, _L, _L, _L, _L]),
     "semk_geom_factors_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _P, _P, _L, _I, _P, _P, _P,
                                    _P, _P, _P, _P]),
+    "semk_field_grad_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _I, _P,
+                                 _P, _P, _P, _P, _P, _P]),
     "semk_gfactors_from_invj_f64": (_I, [_I, _L, _P, _P, _P, _P, _L, _I, _P]),
     "semk_poisson_apply_f64": (_I, [C.POINTER(semk_op), _P, _P, _I, _P, _P]),
     "semk_poisson_apply_atomic_f64": (_I, [_I, _L, _L, _P, _P, _P, _L, _I, _P, _P, _P, _P, _I,

@@ -18,6 +18,92 @@
 
 namespace {
 
+// K1's arithmetic for node k = (m, n) of element `row` (its L2G row), shared by geom_kernel
+// and field_grad_kernel so that the two cannot drift apart: gather the equispaced nodes,
+// subtract the element-local origin (node 0), E^{-1} on axis 0 then axis 1 (GLL
+// coefficients of x - origin, left in sA), J = D x, the closed-form 2x2 inverse and
+// JxW = detJ w_m w_n.  Sets *bad_flag on detJ <= 0.  Every thread of the CTA calls it (it
+// synchronises); the results are meaningful where `on`.  On return sB is free and sA is
+// still read by no one.
+struct NodeGeom {
+  double ox, oy, xg, yg;        // origin; x_phys - origin at the node
+  double j00, j01, j10, j11;    // J[i][a] = d x_i / d xi_a
+  double det, i00, i01, i10, i11, jw;
+};
+
+template <int N>
+__device__ __forceinline__ NodeGeom node_geometry(const uint32_t *__restrict__ row,
+                                                  const double *__restrict__ nodes_x,
+                                                  const double *__restrict__ nodes_y,
+                                                  const double *sE, const double *sD,
+                                                  const double *sw, double (*sA)[N * N],
+                                                  double (*sB)[N * N], int k, bool on, int m,
+                                                  int n, int32_t *__restrict__ bad_flag) {
+  NodeGeom r;
+  const uint32_t g0 = row[0];
+  r.ox = nodes_x[g0];
+  r.oy = nodes_y[g0];
+  __syncthreads();  // tables loaded / previous iteration done with sA, sB
+  if (on) {
+    const uint32_t g = row[k];
+    sA[0][k] = __dsub_rn(nodes_x[g], r.ox);
+    sA[1][k] = __dsub_rn(nodes_y[g], r.oy);
+  }
+  __syncthreads();
+  // equispaced values -> GLL coefficients: axis 0, then axis 1
+  double t0 = 0.0, t1 = 0.0;
+  if (on) {
+#pragma unroll
+    for (int q = 0; q < N; ++q) {
+      const double c = sE[m * N + q];
+      t0 = fma(c, sA[0][q * N + n], t0);
+      t1 = fma(c, sA[1][q * N + n], t1);
+    }
+    sB[0][k] = t0;
+    sB[1][k] = t1;
+  }
+  __syncthreads();
+  r.xg = 0.0;
+  r.yg = 0.0;
+  if (on) {
+#pragma unroll
+    for (int s = 0; s < N; ++s) {
+      const double c = sE[n * N + s];
+      r.xg = fma(c, sB[0][m * N + s], r.xg);
+      r.yg = fma(c, sB[1][m * N + s], r.yg);
+    }
+    sA[0][k] = r.xg;  // all reads of sA happened before the previous barrier
+    sA[1][k] = r.yg;
+  }
+  __syncthreads();
+  if (on) {
+    double j00 = 0.0, j01 = 0.0, j10 = 0.0, j11 = 0.0;
+#pragma unroll
+    for (int q = 0; q < N; ++q) {
+      const double d0 = sD[m * N + q];  // d/dxi0 acts on the first index
+      const double d1 = sD[n * N + q];  // d/dxi1 acts on the second index
+      j00 = fma(d0, sA[0][q * N + n], j00);
+      j10 = fma(d0, sA[1][q * N + n], j10);
+      j01 = fma(d1, sA[0][m * N + q], j01);
+      j11 = fma(d1, sA[1][m * N + q], j11);
+    }
+    const double det = __dsub_rn(__dmul_rn(j00, j11), __dmul_rn(j01, j10));
+    if (!(det > 0.0)) atomicExch(bad_flag, 1);
+    const double rdet = __drcp_rn(det);
+    r.j00 = j00;
+    r.j01 = j01;
+    r.j10 = j10;
+    r.j11 = j11;
+    r.det = det;
+    r.i00 = __dmul_rn(j11, rdet);
+    r.i01 = __dmul_rn(-j01, rdet);
+    r.i10 = __dmul_rn(-j10, rdet);
+    r.i11 = __dmul_rn(j00, rdet);
+    r.jw = __dmul_rn(__dmul_rn(det, sw[m]), sw[n]);
+  }
+  return r;
+}
+
 template <int N>
 __global__ void __launch_bounds__(((N * N + 31) / 32) * 32)
     geom_kernel(int64_t n_elem, const double *__restrict__ nodes_x,
@@ -44,58 +130,10 @@ __global__ void __launch_bounds__(((N * N + 31) / 32) * 32)
   for (int64_t slot = blockIdx.x; slot < n_elem; slot += gridDim.x) {
     const int64_t e = elem_of_slot ? elem_of_slot[slot] : slot;
     if (e < 0) continue;  // empty slot of the engine order (uniform over the CTA): G stays 0
-    const uint32_t *row = l2g + e * NN;
-    const uint32_t g0 = row[0];
-    const double ox = nodes_x[g0], oy = nodes_y[g0];
-    __syncthreads();  // tables loaded / previous iteration done with sA, sB
+    const NodeGeom q =
+        node_geometry<N>(l2g + e * NN, nodes_x, nodes_y, sE, sD, sw, sA, sB, k, on, m, n, bad_flag);
     if (on) {
-      const uint32_t g = row[k];
-      sA[0][k] = __dsub_rn(nodes_x[g], ox);
-      sA[1][k] = __dsub_rn(nodes_y[g], oy);
-    }
-    __syncthreads();
-    // equispaced values -> GLL coefficients: axis 0, then axis 1
-    double t0 = 0.0, t1 = 0.0;
-    if (on) {
-#pragma unroll
-      for (int r = 0; r < N; ++r) {
-        const double c = sE[m * N + r];
-        t0 = fma(c, sA[0][r * N + n], t0);
-        t1 = fma(c, sA[1][r * N + n], t1);
-      }
-      sB[0][k] = t0;
-      sB[1][k] = t1;
-    }
-    __syncthreads();
-    double xg = 0.0, yg = 0.0;
-    if (on) {
-#pragma unroll
-      for (int s = 0; s < N; ++s) {
-        const double c = sE[n * N + s];
-        xg = fma(c, sB[0][m * N + s], xg);
-        yg = fma(c, sB[1][m * N + s], yg);
-      }
-      sA[0][k] = xg;  // all reads of sA happened before the previous barrier
-      sA[1][k] = yg;
-    }
-    __syncthreads();
-    if (on) {
-      double j00 = 0.0, j01 = 0.0, j10 = 0.0, j11 = 0.0;
-#pragma unroll
-      for (int r = 0; r < N; ++r) {
-        const double d0 = sD[m * N + r];  // d/dxi0 acts on the first index
-        const double d1 = sD[n * N + r];  // d/dxi1 acts on the second index
-        j00 = fma(d0, sA[0][r * N + n], j00);
-        j10 = fma(d0, sA[1][r * N + n], j10);
-        j01 = fma(d1, sA[0][m * N + r], j01);
-        j11 = fma(d1, sA[1][m * N + r], j11);
-      }
-      const double det = __dsub_rn(__dmul_rn(j00, j11), __dmul_rn(j01, j10));
-      if (!(det > 0.0)) atomicExch(bad_flag, 1);
-      const double rdet = __drcp_rn(det);
-      const double i00 = __dmul_rn(j11, rdet), i01 = __dmul_rn(-j01, rdet);
-      const double i10 = __dmul_rn(-j10, rdet), i11 = __dmul_rn(j00, rdet);
-      const double jw = __dmul_rn(__dmul_rn(det, sw[m]), sw[n]);
+      const double i00 = q.i00, i01 = q.i01, i10 = q.i10, i11 = q.i11, jw = q.jw;
       if (G) {
         // patch-interleaved layout: ((c*N + m)*PE + le)*N + n inside the patch block
         const int64_t patch = slot / pe;
@@ -107,17 +145,17 @@ __global__ void __launch_bounds__(((N * N + 31) / 32) * 32)
         gs[2 * N * grow] = jw * (i10 * i10 + i11 * i11);
       }
       if (JxW) JxW[e * NN + k] = jw;
-      if (detJout) detJout[e * NN + k] = det;
+      if (detJout) detJout[e * NN + k] = q.det;
       if (x_phys) {
-        x_phys[(e * 2 + 0) * NN + k] = xg + ox;
-        x_phys[(e * 2 + 1) * NN + k] = yg + oy;
+        x_phys[(e * 2 + 0) * NN + k] = q.xg + q.ox;
+        x_phys[(e * 2 + 1) * NN + k] = q.yg + q.oy;
       }
       if (Jout) {
         double *jp = Jout + e * 4 * NN;
-        jp[k] = j00;
-        jp[NN + k] = j01;
-        jp[2 * NN + k] = j10;
-        jp[3 * NN + k] = j11;
+        jp[k] = q.j00;
+        jp[NN + k] = q.j01;
+        jp[2 * NN + k] = q.j10;
+        jp[3 * NN + k] = q.j11;
       }
       if (invJout) {
         double *ip = invJout + e * 4 * NN;
@@ -127,6 +165,109 @@ __global__ void __launch_bounds__(((N * N + 31) / 32) * 32)
         ip[3 * NN + k] = i11;
       }
     }
+  }
+}
+
+// Nodal fields after a solve (one CTA per element, one thread per node, like K1): the
+// geometry again by node_geometry (nothing per element is stored between calls), then
+// ur = D u, us = u D^T through shared memory and grad u = invJ^T (ur, us)
+// (FiniteElement.gradient).  Outputs, each optional:
+//   xy       [2][n_nodes]: x_phys at the entries whose winner byte is set;
+//   grad_loc [2][n_elem][NN] (list order): grad u, times JxW when `weighted`;
+//   jxw_loc  [n_elem][NN] (list order): JxW;
+//   sums     [5]: JxW-sums of (u - u_ref)^2, |grad u - g_ref|^2, max |u - u_ref|,
+//            JxW-sums of u_ref^2, |g_ref|^2 (u_ref / g_ref NULL = 0), reduced in a fixed
+//            order over the CTAs (semk_finish_reduction); the max goes through the spare
+//            slot after the arrival counter of `partials` and is exact in any order.
+template <int N>
+__global__ void __launch_bounds__(((N * N + 31) / 32) * 32)
+    field_grad_kernel(int64_t n_elem, const double *__restrict__ nodes_x,
+                      const double *__restrict__ nodes_y, const uint32_t *__restrict__ l2g,
+                      const double *__restrict__ Einv, const double *__restrict__ D,
+                      const double *__restrict__ w, const int64_t *__restrict__ elems,
+                      const double *__restrict__ u, int64_t n_nodes,
+                      const uint8_t *__restrict__ winner, double *__restrict__ xy,
+                      double *__restrict__ grad_loc, int weighted, double *__restrict__ jxw_loc,
+                      const double *__restrict__ u_ref, const double *__restrict__ g_ref,
+                      double *__restrict__ sums, double *__restrict__ partials,
+                      int32_t *__restrict__ bad_flag) {
+  constexpr int NN = N * N;
+  __shared__ double sE[NN], sD[NN], sw[N];
+  __shared__ double sA[2][NN], sB[2][NN], sU[NN];
+  const int k = threadIdx.x;
+  const bool on = k < NN;
+  const int m = on ? k / N : 0, n = on ? k % N : 0;
+  if (on) {
+    sE[k] = Einv[k];
+    sD[k] = D[k];
+  }
+  if (k < N) sw[k] = w[k];
+  double acc[4] = {0.0, 0.0, 0.0, 0.0};  // (u-u_ref)^2, |grad-g_ref|^2, u_ref^2, |g_ref|^2
+  double umax = 0.0;
+
+  for (int64_t slot = blockIdx.x; slot < n_elem; slot += gridDim.x) {
+    const int64_t e = elems ? elems[slot] : slot;
+    const uint32_t *row = l2g + e * NN;
+    const uint32_t g = on ? row[k] : 0u;
+    const double uk = (u && on) ? u[g] : 0.0;
+    const NodeGeom q =
+        node_geometry<N>(row, nodes_x, nodes_y, sE, sD, sw, sA, sB, k, on, m, n, bad_flag);
+    if (on && xy && winner[e * NN + k]) {
+      xy[g] = q.xg + q.ox;
+      xy[n_nodes + g] = q.yg + q.oy;
+    }
+    if (!u) continue;  // coordinates only (uniform over the grid)
+    if (on) sU[k] = uk;  // the previous element's reads of sU precede node_geometry's barriers
+    __syncthreads();
+    if (on) {
+      double ur = 0.0, us = 0.0;
+#pragma unroll
+      for (int r = 0; r < N; ++r) {
+        ur = fma(sD[m * N + r], sU[r * N + n], ur);
+        us = fma(sD[n * N + r], sU[m * N + r], us);
+      }
+      const double gx = q.i00 * ur + q.i10 * us;
+      const double gy = q.i01 * ur + q.i11 * us;
+      if (grad_loc) {
+        const double s = weighted ? q.jw : 1.0;
+        grad_loc[slot * NN + k] = s * gx;
+        grad_loc[(n_elem + slot) * NN + k] = s * gy;
+      }
+      if (jxw_loc) jxw_loc[slot * NN + k] = q.jw;
+      if (sums) {
+        const double ue = u_ref ? u_ref[g] : 0.0;
+        const double gex = g_ref ? g_ref[g] : 0.0, gey = g_ref ? g_ref[n_nodes + g] : 0.0;
+        const double du = uk - ue, dgx = gx - gex, dgy = gy - gey;
+        acc[0] = fma(q.jw, du * du, acc[0]);
+        acc[1] = fma(q.jw, dgx * dgx + dgy * dgy, acc[1]);
+        acc[2] = fma(q.jw, ue * ue, acc[2]);
+        acc[3] = fma(q.jw, gex * gex + gey * gey, acc[3]);
+        umax = fmax(umax, fabs(du));
+      }
+    }
+  }
+  if (!sums) return;
+  // block max, then one atomicMax on the bit pattern (order-preserving for doubles >= 0)
+  __shared__ double smax[32];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) umax = fmax(umax, __shfl_down_sync(0xffffffffu, umax, o));
+  if ((threadIdx.x & 31u) == 0) smax[threadIdx.x >> 5] = umax;
+  __syncthreads();
+  unsigned long long *max_slot =
+      reinterpret_cast<unsigned long long *>(semk_red_counter(partials) + 1);
+  if (threadIdx.x == 0) {
+    double bm = 0.0;
+    for (unsigned i = 0; i < (blockDim.x + 31u) >> 5; ++i) bm = fmax(bm, smax[i]);
+    atomicMax(max_slot, (unsigned long long)__double_as_longlong(bm));
+  }
+  double tot[4];
+  if (semk_finish_reduction<4>(acc, partials, tot) && threadIdx.x == 0) {
+    sums[0] = tot[0];
+    sums[1] = tot[1];
+    sums[2] = __longlong_as_double((long long)__ldcg(max_slot));
+    sums[3] = tot[2];
+    sums[4] = tot[3];
+    *max_slot = 0ull;
   }
 }
 
@@ -246,5 +387,34 @@ extern "C" int semk_scale_gfactors_f64(int n1, int64_t n_elem, const double *wei
   scale_gfactors_kernel<<<grid, block, 0, semk_stream(stream)>>>(n1, n_elem, weight, elem_of_slot, G,
                                                                 g_patch_stride, elems_per_patch);
   SEMK_LAUNCH_CHECK("scale_gfactors_kernel");
+  return SEMK_OK;
+}
+
+extern "C" int semk_field_grad_f64(int n1, int64_t n_elem, const double *nodes_x,
+                                   const double *nodes_y, const uint32_t *l2g, const double *Einv,
+                                   const double *D, const double *w, const int64_t *elems,
+                                   int64_t n_nodes, const double *u, const uint8_t *winner,
+                                   double *xy, double *grad_loc, int weighted, double *jxw_loc,
+                                   const double *u_ref, const double *g_ref, double *sums,
+                                   double *partials, int32_t *bad_flag, void *stream) {
+  SEMK_REQUIRE(n_elem >= 0 && n_nodes > 0, "semk_field_grad_f64: bad sizes");
+  SEMK_REQUIRE(nodes_x && nodes_y && l2g && Einv && D && w && bad_flag,
+               "semk_field_grad_f64: null input pointer");
+  SEMK_REQUIRE(!xy || winner, "semk_field_grad_f64: xy needs winner");
+  SEMK_REQUIRE(u || !(grad_loc || jxw_loc || sums), "semk_field_grad_f64: outputs need u");
+  SEMK_REQUIRE(!sums || partials, "semk_field_grad_f64: sums need partials");
+  SEMK_REQUIRE(!xy || (xy != u && xy != u_ref && xy != g_ref),
+               "semk_field_grad_f64: xy aliases an input");
+  if (n_elem == 0) return SEMK_OK;
+  // the fixed-order reduction bounds the grid (kSemkRedMaxBlocks CTAs of partials)
+  const int64_t cap = sums ? kSemkRedMaxBlocks : (1 << 20);
+  const unsigned grid = (unsigned)(n_elem < cap ? n_elem : cap);
+#define SEMK_CALL(NV)                                                                      \
+  field_grad_kernel<NV><<<grid, ((NV * NV + 31) / 32) * 32, 0, semk_stream(stream)>>>(     \
+      n_elem, nodes_x, nodes_y, l2g, Einv, D, w, elems, u, n_nodes, winner, xy, grad_loc,   \
+      weighted, jxw_loc, u_ref, g_ref, sums, partials, bad_flag)
+  SEMK_DISPATCH_N1(n1, SEMK_CALL)
+#undef SEMK_CALL
+  SEMK_LAUNCH_CHECK("field_grad_kernel");
   return SEMK_OK;
 }

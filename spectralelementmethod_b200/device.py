@@ -12,7 +12,8 @@ import torch
 from . import _lib
 
 __all__ = ["stream_ptr", "as_i32_bits", "basis_tables", "element_geometry", "ptr",
-           "boundary_face_tables", "csr_by_key", "BoundaryFaces"]
+           "boundary_face_tables", "csr_by_key", "BoundaryFaces", "winner_table",
+           "node_entries_csr", "field_grad"]
 
 
 def stream_ptr():
@@ -89,6 +90,49 @@ def geom_factors(tab, nodes_dev, l2g_dev, n_elem, elem_of_slot=None, G=None, g_p
         ptr(JxW), ptr(x_phys), ptr(J), ptr(invJ), ptr(detJ), ptr(bad), stream_ptr()))
     if check and int(bad.item()) != 0:
         raise AssertionError("non-positive Jacobian determinant in the mesh")
+
+
+def field_grad(tab, nodes_dev, l2g_dev, n_elem, n_nodes, elems=None, u=None, winner=None,
+               xy=None, grad_loc=None, weighted=False, jxw_loc=None, u_ref=None, g_ref=None,
+               sums=None, partials=None):
+    """Launch the nodal-field kernel (csrc/semk_geom.cu, semk_field_grad_f64): K1's geometry
+    again, then the gradient of ``u`` and whichever outputs are given.  Raises AssertionError
+    on a non-positive Jacobian, like ``geom_factors``."""
+    lib = _lib.load()
+    D, Einv, w = tab.dev()
+    bad = torch.zeros(1, dtype=torch.int32, device=nodes_dev.device)
+    _lib.check(lib.semk_field_grad_f64(
+        tab.n1, int(n_elem), ptr(nodes_dev[0]), ptr(nodes_dev[1]), ptr(l2g_dev), ptr(Einv),
+        ptr(D), ptr(w), ptr(elems), int(n_nodes), ptr(u), ptr(winner), ptr(xy), ptr(grad_loc),
+        int(bool(weighted)), ptr(jxw_loc), ptr(u_ref), ptr(g_ref), ptr(sums), ptr(partials),
+        ptr(bad), stream_ptr()))
+    if int(bad.item()) != 0:
+        raise AssertionError("non-positive Jacobian determinant in the mesh")
+
+
+def winner_table(l2g, n_nodes):
+    """``uint8`` per entry of the L2G map (any shape, flat order): 1 where the entry is the
+    last one naming its node -- the element whose value the reference's element loop keeps
+    (fancy assignment keeps the last value for repeated indices).  Pure NumPy."""
+    flat = np.asarray(l2g).ravel()
+    last = np.empty(int(n_nodes), dtype=np.int64)
+    last[flat] = np.arange(flat.size, dtype=np.int64)
+    return (last[flat] == np.arange(flat.size, dtype=np.int64)).astype(np.uint8)
+
+
+def node_entries_csr(l2g_t, n_nodes):
+    """Node -> entries CSR of the whole L2G map: ``pos[ptr[j]:ptr[j+1]]`` the flat entries
+    ``e * NN + k`` naming node j, ascending (a stable sort: the order of ``csr_by_key``, and
+    the fixed order in which ``semk_face_sum_f64`` sums element-local values onto nodes).
+    ``l2g_t``: int32-bit-pattern tensor [E, NN] on any device; returns int32-bit-pattern
+    tensors (ptr [n_nodes + 1], pos [E * NN]) on that device."""
+    flat = l2g_t.reshape(-1).to(torch.int64) & 0xFFFFFFFF
+    if flat.numel() >= 2 ** 31:
+        raise NotImplementedError("more than 2^31 L2G entries")
+    pos = torch.sort(flat, stable=True).indices.to(torch.int32)
+    ptr_ = torch.zeros(int(n_nodes) + 1, dtype=torch.int64, device=flat.device)
+    torch.cumsum(torch.bincount(flat, minlength=int(n_nodes)), 0, out=ptr_[1:])
+    return ptr_.to(torch.int32), pos
 
 
 def stiffness_factors(tab, mesh, l2g_dev, n_slots, G, g_stride, elems_per_patch, JxW,
@@ -187,8 +231,10 @@ class BoundaryFaces(object):
 
     * ``x [F, 2, n1]``: physical coordinates of the face nodes, and ``dSxW [F, n1]``: the face's
       GLL weight times ``|dx/dxi_t|`` -- the host mirror's ``SubFiniteElement.x_phys`` /
-      ``dSxW``.  K1 runs on the boundary cells only (as ``DOFManager.boundary_elements`` does)
-      and the face slice and the tangent length follow ``SubMapping._tangents``.
+      ``dSxW``; ``n_dSxW [F, 2, n1]``: the outward normal times ``dSxW``
+      (``SubFiniteElement.n_dSxW``, the normal of ``SubMapping._compute_normal_vec``).  K1
+      runs on the boundary cells only (as ``DOFManager.boundary_elements`` does) and the face
+      slice and the tangent length follow ``SubMapping._tangents``.
     * ``nodes``: the distinct boundary nodes, ascending, and ``keys``: the distinct
       element-local slots ``cell * NN + local`` of the face nodes; ``face_sum`` adds
       face-node values ``[F, n1]`` onto either in a fixed order (``csr_by_key``)."""
@@ -213,6 +259,7 @@ class BoundaryFaces(object):
         f64 = dict(dtype=torch.float64, device=dev)
         self.x = torch.empty((F, 2, n1), **f64)
         self.dSxW = torch.empty((F, n1), **f64)
+        self.n_dSxW = torch.empty((F, 2, n1), **f64)
         if F == 0:
             return
         l2g = as_i32_bits(mesh.node_map_array().reshape(-1, NN)[self.cells], dev)
@@ -227,7 +274,13 @@ class BoundaryFaces(object):
         along = torch.from_numpy(1 - self.faces // 2).to(dev)
         tan = torch.gather(J[torch.arange(F, device=dev), :, along, :], 2, loc)
         dS = torch.sqrt(tan[:, 0] * tan[:, 0] + tan[:, 1] * tan[:, 1])
-        self.dSxW.copy_(dS * _f64(tab.w_host, dev)[None, :])
+        w = _f64(tab.w_host, dev)[None, :]
+        self.dSxW.copy_(dS * w)
+        # counter-clockwise tangent (faces 0 and 3 run against the parametric direction),
+        # turned clockwise: (t_y, -t_x) points out of the cell
+        sgn = torch.from_numpy(np.where((self.faces == 0) | (self.faces == 3), -1.0, 1.0)).to(dev)
+        self.n_dSxW[:, 0].copy_(sgn[:, None] * tan[:, 1] * w)
+        self.n_dSxW[:, 1].copy_(-sgn[:, None] * tan[:, 0] * w)
 
     def face_sum(self, vals, onto="nodes"):
         """Sum face-node values ``vals [F, n1]`` onto the distinct boundary nodes (``onto =

@@ -212,30 +212,215 @@ class DOFManager(object):
             raise ValueError("coeffs must be a float64 CUDA tensor [..., n_nodes]")
         lib = _lib.load()
         tab = device.basis_tables(self._basis)
-        NN = tab.n1 * tab.n1
-        cache = getattr(self, "_field_tables", None)
-        if cache is None or cache[0] != coeffs.device:
-            l2g = self.node_map_array().reshape(-1, NN)
-            flat = l2g.ravel()
-            # the reference's loop overwrites shared nodes: the last element containing a
-            # node wins (fancy assignment keeps the last value for repeated indices)
-            last = np.empty(self._mesh.n_nodes, dtype=np.int64)
-            last[flat] = np.arange(flat.size, dtype=np.int64)
-            winner = (last[flat] == np.arange(flat.size, dtype=np.int64)).astype(np.uint8)
-            sub = [b for _, b in self._basis.iter_subbases()][0]
-            cache = (coeffs.device, device.as_i32_bits(l2g, coeffs.device),
-                     torch.from_numpy(winner).to(coeffs.device),
-                     device._f64(np.ascontiguousarray(sub.interp_eq_mat), coeffs.device),
-                     int(l2g.shape[0]))
-            self._field_tables = cache
-        _, l2g_dev, winner_dev, emat_dev, n_elem = cache
+        t = self._device_field_tables(coeffs.device)
         src = coeffs.contiguous().reshape(-1, coeffs.shape[-1])
         out = torch.empty_like(src)
         for i in range(src.shape[0]):
             _lib.check(lib.semk_values_at_nodes_f64(
-                tab.n1, n_elem, device.ptr(l2g_dev), device.ptr(winner_dev), device.ptr(emat_dev),
-                device.ptr(src[i]), device.ptr(out[i]), device.stream_ptr()))
+                tab.n1, t["n_elem"], device.ptr(t["l2g"]), device.ptr(t["winner"]),
+                device.ptr(t["emat"]), device.ptr(src[i]), device.ptr(out[i]),
+                device.stream_ptr()))
         return out.reshape(coeffs.shape)
+
+    def _device_field_tables(self, dev):
+        """Device tables of the nodal-field kernels, built once and kept: the L2G map, the
+        winner bytes of the last-element-wins rule (``device.winner_table``) and the 1-D
+        equispaced interpolation matrix."""
+        cache = getattr(self, "_field_tables", None)
+        if cache is None or cache["dev"] != dev:
+            import torch
+            from . import device
+            NN = device.basis_tables(self._basis).n1 ** 2
+            l2g = self.node_map_array().reshape(-1, NN)
+            sub = [b for _, b in self._basis.iter_subbases()][0]
+            winner = device.winner_table(l2g, self._mesh.n_nodes)
+            cache = dict(dev=dev, l2g=device.as_i32_bits(l2g, dev),
+                         winner=torch.from_numpy(winner).to(dev),
+                         emat=device._f64(np.ascontiguousarray(sub.interp_eq_mat), dev),
+                         n_elem=int(l2g.shape[0]))
+            self._field_tables = cache
+        return cache
+
+    # -- nodal fields after a solve: coordinates, gradients, norms, fluxes (device) -----------
+    def _post_tables(self, dev):
+        """``_device_field_tables`` plus what the post-processing methods need (on first use):
+        the mesh nodes, the node -> entries CSR of the whole L2G map
+        (``device.node_entries_csr``) and reduction scratch."""
+        import torch
+        from . import _lib, device
+        t = self._device_field_tables(dev)
+        if "csr" not in t:
+            tab, ftab = device.basis_tables(self._map_basis), device.basis_tables(self._basis)
+            if not (tab.n1 == ftab.n1 and np.array_equal(tab.D_host, ftab.D_host)
+                    and np.array_equal(tab.w_host, ftab.w_host)):
+                raise NotImplementedError("nodal fields need the isoparametric case")
+            nodes = device._f64(self._mesh.nodes, dev)
+            if nodes.shape[0] != 2:
+                raise NotImplementedError("Only supporting 2D elements right now")
+            t.update(tab=tab, nodes=nodes,
+                     csr=device.node_entries_csr(t["l2g"], self._mesh.n_nodes),
+                     partials=torch.zeros(int(_lib.load().semk_vec_partials_len(0)),
+                                          dtype=torch.float64, device=dev))
+        return t
+
+    def _nodal_input(self, u, what="u"):
+        import torch
+        if not (isinstance(u, torch.Tensor) and u.is_cuda and u.dtype == torch.float64
+                and tuple(u.shape) == (self._mesh.n_nodes,)):
+            raise ValueError("%s must be a float64 CUDA tensor [n_nodes]" % what)
+        return u.contiguous()
+
+    def _element_gradients(self, u, elems=None, weighted=False):
+        """Physical gradient of the nodal vector ``u`` on the elements ``elems`` (int64 CUDA
+        tensor, None = all): ``(grad [2, n, NN], JxW [n, NN])`` with ``grad[:, i]`` the
+        host mirror's ``fe.gradient(u[fe.node_ind])`` of element ``elems[i]`` (times JxW
+        when ``weighted``).  One pass of csrc/semk_geom.cu's field kernel."""
+        import torch
+        from . import device
+        u = self._nodal_input(u)
+        t = self._post_tables(u.device)
+        n = t["n_elem"] if elems is None else int(elems.numel())
+        NN = t["tab"].n1 ** 2
+        g = torch.empty((2, n, NN), dtype=torch.float64, device=u.device)
+        jxw = torch.empty((n, NN), dtype=torch.float64, device=u.device)
+        device.field_grad(t["tab"], t["nodes"], t["l2g"], n, self._mesh.n_nodes, elems=elems,
+                          u=u, grad_loc=g, weighted=weighted, jxw_loc=jxw)
+        return g, jxw
+
+    def node_coordinates(self):
+        """Physical coordinates of every GLL node -- the points the operators' nodal vectors
+        live on -- as a CUDA tensor ``[2, n_nodes]``: ``fe.x_phys`` of the last element
+        containing the node (the loop ``X[:, fe.node_ind] = fe.x_phys`` over
+        ``finite_elements``), by the geometry kernel's arithmetic (csrc/semk_geom.cu)."""
+        import torch
+        from . import _lib, device
+        _lib.require_device()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        t = self._post_tables(dev)
+        n = self._mesh.n_nodes
+        xy = torch.zeros((2, n), dtype=torch.float64, device=dev)
+        device.field_grad(t["tab"], t["nodes"], t["l2g"], t["n_elem"], n, winner=t["winner"],
+                          xy=xy)
+        return xy
+
+    def gradient(self, u):
+        """Gradient of the nodal vector ``u`` (a float64 CUDA tensor ``[n_nodes]``, as both
+        Poisson operators return) at the nodes, a CUDA tensor ``[2, n_nodes]``: the
+        JxW-weighted average of the element gradients (``fe.gradient``) of the elements
+        sharing a node, ``sum_e JxW grad u_e / sum_e JxW`` -- the lumped L2 projection onto
+        the continuous space.  The sums run over a fixed order (bitwise reproducible)."""
+        import torch
+        from . import _lib, device
+        g, jxw = self._element_gradients(u, weighted=True)
+        t = self._post_tables(g.device)
+        ptr_, pos = t["csr"]
+        n = self._mesh.n_nodes
+        out = torch.empty((3, n), dtype=torch.float64, device=g.device)
+        for i, v in enumerate((g[0], g[1], jxw)):
+            _lib.check(_lib.load().semk_face_sum_f64(n, device.ptr(ptr_), device.ptr(pos),
+                                                     device.ptr(v), device.ptr(out[i]),
+                                                     device.stream_ptr()))
+        return out[:2] / out[2]
+
+    def _reference_values(self, f, rows, X, what):
+        """``exact`` / ``grad_exact`` of ``error_norms`` as a [rows, n_nodes] CUDA tensor:
+        nodal values (a gradient also as a pair of components) or a callable of the node
+        coordinates (``X[0]``, computed on first need); scalars are broadcast."""
+        import torch
+        n = self._mesh.n_nodes
+        dev = torch.device("cuda", torch.cuda.current_device())
+        if callable(f):
+            if X[0] is None:
+                X[0] = self.node_coordinates()
+            f = f(X[0][0], X[0][1])
+        parts = list(f) if rows == 2 and isinstance(f, (tuple, list)) else [f]
+        parts = [torch.as_tensor(c, dtype=torch.float64, device=dev) for c in parts]
+        parts = [c.expand(n) if c.ndim == 0 else c for c in parts]
+        want = "[n_nodes]" if rows == 1 else "[2, n_nodes]"
+        if len(parts) > 1:
+            if len(parts) != 2 or any(tuple(c.shape) != (n,) for c in parts):
+                raise ValueError("%s must have shape %s" % (what, want))
+            parts = [torch.stack(parts)]
+        v = parts[0]
+        if tuple(v.shape) != ((n,) if rows == 1 else (2, n)):
+            raise ValueError("%s must have shape %s" % (what, want))
+        return v.contiguous()
+
+    def error_norms(self, u, exact=None, grad_exact=None):
+        """Norms of the error of the nodal vector ``u`` (float64 CUDA ``[n_nodes]``) against
+        ``exact`` (nodal values or a callable ``f(x, y)`` on CUDA tensors of the node
+        coordinates, the convention of ``robin=`` / ``flux=``) and its gradient
+        ``grad_exact`` (``[2, n_nodes]``, a pair of nodal components, or a callable returning
+        the pair).  A dict:
+
+        * ``l2``: ``sqrt(sum_e fe.integrate((u - exact)^2))``, ``h1_semi``: the same of
+          ``|grad u - grad_exact|^2``, ``max_nodal``: ``max |u - exact|`` over the nodes;
+        * ``l2_ref`` / ``h1_semi_ref``: the norms of ``exact`` / ``grad_exact`` themselves.
+
+        ``exact=None``: the norms of ``u`` itself (the reference and its gradient are zero).
+        ``grad_exact=None`` with an ``exact``: the H1 entries are None.  The integrals use
+        GLL collocation quadrature at the element nodes -- the reference's
+        ``FiniteElement.integrate`` -- not over-integration.  One pass of the field kernel with
+        a fixed-order reduction (csrc/semk_geom.cu): bitwise reproducible."""
+        import math
+        import torch
+        from . import device
+        u = self._nodal_input(u)
+        t = self._post_tables(u.device)
+        X = [None]
+        u_ref = None if exact is None else self._reference_values(exact, 1, X, "exact")
+        g_ref = None if grad_exact is None else self._reference_values(grad_exact, 2, X,
+                                                                        "grad_exact")
+        sums = torch.empty(5, dtype=torch.float64, device=u.device)
+        device.field_grad(t["tab"], t["nodes"], t["l2g"], t["n_elem"], self._mesh.n_nodes, u=u,
+                          u_ref=u_ref, g_ref=g_ref, sums=sums, partials=t["partials"])
+        s = sums.tolist()
+        h1 = exact is None or grad_exact is not None
+        return dict(l2=math.sqrt(s[0]), h1_semi=math.sqrt(s[1]) if h1 else None,
+                    max_nodal=s[2], l2_ref=math.sqrt(s[3]),
+                    h1_semi_ref=math.sqrt(s[4]) if h1 else None)
+
+    def boundary_flux(self, u, name, weight=1.0):
+        """Flux of the nodal vector ``u`` (float64 CUDA ``[n_nodes]``) through the named
+        boundary, ``sum_faces sum_k w_k (grad u . n dS w)_k`` -- the host recipe
+        ``sum bfe.integrate(w * (bfe.gradient(u[fe.node_ind]) . bfe.unit_normal))`` over
+        ``boundary_elements(name)``, with the outward normal of
+        ``SubMapping._compute_normal_vec`` -- as a float.  ``weight`` (the ``w`` of a
+        ``-div(w grad u)`` operator; operators do not keep theirs): a scalar, nodal values or
+        a callable ``w(x, y)`` on CUDA tensors of the face-node coordinates.  The field
+        kernel runs on the boundary cells only; the sum is semk_dot_f64's fixed order.
+        An unknown name raises the ``KeyError`` of ``boundary_elements``."""
+        import torch
+        from . import _lib, device
+        u = self._nodal_input(u)
+        dev = u.device
+        cache = self.__dict__.setdefault("_bfaces_dev", {})
+        if (name, dev) not in cache:
+            cache[(name, dev)] = device.BoundaryFaces(device.basis_tables(self._basis),
+                                                      self._mesh, name, dev)
+        bf = cache[(name, dev)]
+        if bf.n_faces == 0:
+            return 0.0
+        t = self._post_tables(dev)
+        cells, inv = np.unique(bf.cells, return_inverse=True)
+        g, _ = self._element_gradients(u, elems=torch.from_numpy(cells).to(dev))
+        NN = t["tab"].n1 ** 2
+        idx = torch.from_numpy(inv[:, None] * NN + bf.local).to(dev)
+        gn = g[0].reshape(-1)[idx] * bf.n_dSxW[:, 0] + g[1].reshape(-1)[idx] * bf.n_dSxW[:, 1]
+        if callable(weight):
+            w = torch.as_tensor(weight(bf.x[:, 0, :], bf.x[:, 1, :]), dtype=torch.float64,
+                                device=dev).expand(gn.shape)
+        elif isinstance(weight, torch.Tensor) or np.ndim(weight) != 0:
+            w = self._nodal_input(torch.as_tensor(weight, dtype=torch.float64, device=dev),
+                                  "weight")[bf.node_ids_dev]
+        else:
+            w = torch.full(gn.shape, float(weight), dtype=torch.float64, device=dev)
+        w, gn = w.contiguous(), gn.contiguous()
+        out = torch.empty(1, dtype=torch.float64, device=dev)
+        _lib.check(_lib.load().semk_dot_f64(int(gn.numel()), device.ptr(w), device.ptr(gn),
+                                            device.ptr(out), device.ptr(t["partials"]),
+                                            device.stream_ptr()))
+        return float(out)
 
     # -- batched point location / evaluation on the device (additive API) -------------------
     def _locate_tables(self):
