@@ -34,7 +34,25 @@ __all__ = ["StripPartition", "CondensedStripView", "DistributedOperator", "PeerH
            "DistributedCondensedPoisson"]
 
 
-class StripPartition(object):
+class _StripColumns(object):
+    """Contiguous id ranges of the two interface columns and the owned prefix of a strip, from
+    ``NY`` (entries of one column), ``n_local`` and ``right`` (the right neighbour owns the
+    column it shares)."""
+
+    @property
+    def left_slice(self):
+        return slice(0, self.NY)
+
+    @property
+    def right_slice(self):
+        return slice(self.n_local - self.NY, self.n_local)
+
+    @property
+    def n_owned(self):
+        return self.n_local - (self.NY if self.right is not None else 0)
+
+
+class StripPartition(_StripColumns):
     """Description of one rank's strip of a global (nx_local*world) x ny mesh."""
 
     def __init__(self, rank, world, nx_local, ny, p, bounds=(-1.0, 1.0, -1.0, 1.0)):
@@ -48,21 +66,11 @@ class StripPartition(object):
         self.n_local = self.NX_local * self.NY
         self.left = rank - 1 if rank > 0 else None
         self.right = rank + 1 if rank < world - 1 else None
-        self.n_owned = self.n_local - (self.NY if self.right is not None else 0)
         x0, x1, y0, y1 = bounds
         w = (x1 - x0) / self.world
         self.bounds_global = bounds
         self.bounds_local = (x0 + rank * w, x0 + (rank + 1) * w, y0, y1)
         self.n_global = (self.nx_global * self.p + 1) * self.NY
-
-    # contiguous id ranges of the two interface columns
-    @property
-    def left_slice(self):
-        return slice(0, self.NY)
-
-    @property
-    def right_slice(self):
-        return slice(self.n_local - self.NY, self.n_local)
 
     def global_ids(self):
         """Global lattice id of every local node (global id = i*NY + j)."""
@@ -108,7 +116,7 @@ class StripPartition(object):
         return mesh
 
 
-class CondensedStripView(object):
+class CondensedStripView(_StripColumns):
     """A strip partition seen through the exterior-first numbering of
     ``DOFManagerSC`` (sem/discrete.py:314-359) on the rank-local mesh: condensed
     vectors have ``n_ext`` entries, and because the renumbering keeps the
@@ -127,15 +135,6 @@ class CondensedStripView(object):
         # ny + 1 describes vertex (coarse) vectors, whose compact ids are ordered the same way
         self.NY = part.NY if column is None else int(column)
         self.n_local = int(n_ext)
-        self.n_owned = self.n_local - (self.NY if self.right is not None else 0)
-
-    @property
-    def left_slice(self):
-        return slice(0, self.NY)
-
-    @property
-    def right_slice(self):
-        return slice(self.n_local - self.NY, self.n_local)
 
 
 def _all_ok(ok, group, device):
@@ -310,9 +309,9 @@ class DistributedOperator(object):
                  dot=None, overlap=None):
         self.part = part
         self.local_apply = local_apply
-        # overlap(u, out) -> out: local apply + peer exchange in one native call with the
-        # exchange hidden behind the interior patches (semk_poisson_apply_halo_f64); used
-        # whenever no fused dot is requested
+        # overlap(u, out, dirichlet_u8) -> out: local apply + peer exchange in one native call
+        # with the exchange hidden behind the interior patches (PoissonOperator.apply_halo);
+        # used whenever no fused dot is requested
         self.overlap = overlap
         self._dot = dot               # dot(a, b, out): the C-ABI reduction (PCGKernels.dot)
         self.group = group
@@ -370,7 +369,13 @@ class DistributedOperator(object):
         global value."""
         if self.overlap is not None and dot_out is None and self.halo is not None:
             return self.overlap(u, out, self._dir_u8)
-        y = self.local_apply(u, out, dot_out)
+        return self.finish(self.local_apply(u, out, dot_out), u, dot_out)
+
+    def finish(self, y, u, dot_out=None):
+        """Second half of ``apply`` for a local result ``y`` (also one computed elsewhere, such
+        as the staged host apply's): sum the interface columns across neighbours and re-impose
+        the Dirichlet identity rows on them, in place.  ``dot_out``: this rank's share of u.y
+        from the local apply, corrected here for the shared column."""
         if self.halo is not None:
             return self.halo.exchange(y, u, self._dir_u8, dot_out)
         self.exchange_add(y)
@@ -380,17 +385,6 @@ class DistributedOperator(object):
             # identity rows on a shared column were counted by both ranks
             dup = u[self._fix_nonowned]
             dot_out -= (dup * dup).sum()
-        return y
-
-    def finish(self, y, u):
-        """Second half of ``apply`` for a local result ``y`` computed elsewhere (the staged
-        host apply): sum the interface columns across neighbours and re-impose the Dirichlet
-        identity rows on them, in place."""
-        if self.halo is not None:
-            return self.halo.exchange(y, u, self._dir_u8, None)
-        self.exchange_add(y)
-        if self._fix_ids is not None:
-            y[self._fix_ids] = u[self._fix_ids]
         return y
 
     def owned_dot(self, a, b):
@@ -581,90 +575,165 @@ def strip_vertex_aggregates(part, vertex_lex_ids, dirichlet_c, max_tiles=4096):
     return agg, int(tx * ty), int(k)
 
 
-def _native_jacobi_pcg(owner, op_struct, sc_struct, halo, n_owned, b, x, dinv, vec_partials, rtol,
-                       maxiter, check_every):
-    """semk_pcg_dist_solve_f64 on a partition whose exchanges run over peer memory: the
-    whole loop (applies, interface exchanges, both all-reduces of an iteration) is issued by
-    the native driver.  ``owner`` keeps the PeerComm."""
-    import ctypes as C
-    from . import _lib, device
-    lib = _lib.load()
-    if getattr(owner, "_comm", None) is None:
-        owner._comm = PeerComm(halo.part.rank, halo.part.world, 64, owner.group, b.device)
-    n = b.numel()
-    work = torch.empty(3 * (n + 32), dtype=torch.float64, device=b.device)
-    sc = torch.zeros(32, dtype=torch.float64, device=b.device)
-    info = _lib.semk_pcg_info()
-    torch.cuda.synchronize(b.device)        # ranks enter together (the peer kernels give up
-    dist.barrier(group=owner.group)         # after ~2 s of waiting)
-    rc = lib.semk_pcg_dist_solve_f64(
-        C.byref(op_struct) if op_struct is not None else None,
-        C.byref(sc_struct) if sc_struct is not None else None,
-        C.byref(halo.c), C.byref(owner._comm.c), int(n_owned), device.ptr(b), device.ptr(x),
-        device.ptr(dinv), device.ptr(work), device.ptr(sc), device.ptr(vec_partials), float(rtol),
-        int(maxiter), int(check_every), C.byref(info), device.stream_ptr())
-    _lib.check(rc)
-    halo.check()
-    owner._comm.check()
-    return info.iterations, info.rel_residual, info.status == 0
+class _StripPoissonBase(object):
+    """What the strip-partitioned plain and condensed Poisson paths share: the interface
+    exchange, the global apply, diagonal, load and lifting, and Jacobi-PCG over all ranks, all
+    written against the rank-local operator (``op`` or ``sc``).  ``_OP_SLOT`` names the argument
+    of semk_pcg_dist_solve_f64 ("op" or "sc_op") that takes that operator's struct."""
 
+    _OP_SLOT = None
 
-class DistributedPoisson(object):
-    """The whole multi-GPU Poisson path for the strip-partitioned structured
-    configurations (BASELINE.json configs[4]): local mesh + DOF manager +
-    device operator on each rank, interface exchange, global Jacobi-PCG."""
-
-    def __init__(self, part, order, kind="S", group=None, elems_per_patch=None, exchange="auto",
-                 overlap=True):
-        from . import discrete
-        from .basis_functions import LagrangeGaussLobatto, TensorProductQS
-        from .operators import PCGKernels
-        self.part = part
-        self.group = group
-        self.mesh = part.build_local_mesh(kind)
-        b1 = LagrangeGaussLobatto(order)
-        self.mngr = discrete.DOFManager(self.mesh, 1, TensorProductQS(b1, b1), rcm_order=False)
-        self.on_ebc = self.mngr.boundary_node_mask("ebc")
-        self.op = self.mngr.poisson_operator(dirichlet=self.on_ebc, elems_per_patch=elems_per_patch,
-                                             boundary_columns_first=overlap)
-        self.kernels = PCGKernels(self.op)
-        op = self.op
+    def __init__(self, part, group, exchange):
         if exchange not in ("auto", "peer", "nccl"):
             raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
+        self.part = part
+        self.group = group
+        self._comm = None
+        self._dinv = None
+
+    def _open_halo(self, strip, exchange, device):
+        """``halo``: the peer-memory exchange of ``strip`` (a StripPartition or a
+        CondensedStripView), or None for NCCL p2p; ``exchange``: which of the two it is."""
         self.halo = None
         if exchange in ("auto", "peer"):
             # PeerHalo sets itself up collectively: either every rank maps its neighbours
             # or every rank raises; "auto" then falls back to NCCL p2p on all ranks
             try:
-                self.halo = PeerHalo(part, group, op.dev)
+                self.halo = PeerHalo(strip, self.group, device)
             except RuntimeError:
                 if exchange == "peer":
                     raise
-                self.halo = None
         self.exchange = "peer" if self.halo is not None else "nccl"
+
+    def _connect(self, local, strip, overlap=None):
+        """``dop``: the global operator over the rank-local operator ``local`` on ``strip``."""
+        from .operators import PCGKernels
+        self._local = local
+        self.kernels = PCGKernels(local, n=local._n_vec)
+        self.dop = DistributedOperator(
+            strip, lambda u, out, dot: local.apply(u, out=out, dot_out=dot),
+            dirichlet=self.on_ebc[:local._n_vec] if local.has_dirichlet else None,
+            group=self.group, device=local.dev, halo=self.halo, dot=self.kernels.dot,
+            overlap=overlap)
+        self._mask = local.dirichlet_dev.bool() if local.has_dirichlet else None
+
+    def apply(self, u, out=None, dot_out=None):
+        return self.dop.apply(u, out=out, dot_out=dot_out)
+
+    def diagonal(self):
+        d = self._local.diagonal(masked=False)
+        self.dop.exchange_add(d)
+        if self._mask is not None:
+            d[self._mask] = 1.0
+        return d
+
+    def rhs(self, f=1.0):
+        return self.dop.exchange_add(self._local.rhs(f))
+
+    def lift(self, b, g=None):
+        """b_f - A_fe g on free rows, g on Dirichlet rows (global operator).  ``g``: a CUDA
+        tensor of the local operator's vector length, or a whole nodal vector, of which the
+        condensed operator reads the leading n_ext entries."""
+        if self._mask is None:
+            return b.clone()
+        gv = torch.zeros_like(b)
+        if g is not None:
+            if g.numel() == self._local.n_nodes:
+                g = g[:self._local._n_vec]
+            gv[self._mask] = g[self._mask]
+        from ._lib import MASK_OUT
+        t = self._local.apply(gv, flags=MASK_OUT)
+        self.dop.exchange_add(t)
+        out = b - t
+        out[self._mask] = gv[self._mask]
+        return out
+
+    def _start(self, b, x0):
+        """PCG start iterate; the global inverse diagonal on first use (collective)."""
+        x = self._local._start_iterate(b, x0)
+        if self._dinv is None:
+            self._dinv = 1.0 / self.diagonal()
+        return x
+
+    def solve_pcg(self, b, x0=None, rtol=1e-12, maxiter=200000, check_every=25, native=True):
+        """Jacobi-PCG over all ranks.  With the peer-memory exchange the native driver
+        semk_pcg_dist_solve_f64 runs the whole loop (``native=False``: the host-driven loop
+        with NCCL all-reduces, which is also what the NCCL / gloo paths use).  Returns (x,
+        iterations, rel_residual, converged)."""
+        x = self._start(b, x0)
+        if self.halo is not None and native:
+            it, rel, ok = self._native_jacobi_pcg(b, x, rtol, maxiter, check_every)
+        else:
+            it, rel, ok = distributed_pcg(self.dop, b, x, self._dinv, self.kernels, rtol=rtol,
+                                          maxiter=maxiter, check_every=check_every)
+        return x, it, rel, ok
+
+    def _native_jacobi_pcg(self, b, x, rtol, maxiter, check_every):
+        """semk_pcg_dist_solve_f64 on a partition whose exchanges run over peer memory: the
+        whole loop (applies, interface exchanges, both all-reduces of an iteration) is issued by
+        the native driver.  The PeerComm of its all-reduces is opened on first use and kept."""
+        import ctypes as C
+        from . import _lib, device
+        lib = _lib.load()
+        if self._comm is None:
+            self._comm = PeerComm(self.part.rank, self.part.world, 64, self.group, b.device)
+        n = b.numel()
+        work = torch.empty(3 * (n + 32), dtype=torch.float64, device=b.device)
+        sc = torch.zeros(32, dtype=torch.float64, device=b.device)
+        info = _lib.semk_pcg_info()
+        ops = {"op": None, "sc_op": None}
+        ops[self._OP_SLOT] = C.byref(self._local._op)
+        torch.cuda.synchronize(b.device)        # ranks enter together (the peer kernels give up
+        dist.barrier(group=self.group)          # after ~2 s of waiting)
+        rc = lib.semk_pcg_dist_solve_f64(
+            ops["op"], ops["sc_op"], C.byref(self.halo.c), C.byref(self._comm.c),
+            int(self.dop.part.n_owned), device.ptr(b), device.ptr(x), device.ptr(self._dinv),
+            device.ptr(work), device.ptr(sc), device.ptr(self._local.vec_partials), float(rtol),
+            int(maxiter), int(check_every), C.byref(info), device.stream_ptr())
+        _lib.check(rc)
+        self.halo.check()
+        self._comm.check()
+        return info.iterations, info.rel_residual, info.status == 0
+
+    def close(self):
+        """Collective tear-down of the peer-memory regions."""
+        if self._comm is not None:
+            self._comm.close()
+            self._comm = None
+        if self.halo is not None:
+            self.halo.close()
+            self.halo = None
+
+
+class DistributedPoisson(_StripPoissonBase):
+    """The whole multi-GPU Poisson path for the strip-partitioned structured
+    configurations (BASELINE.json configs[4]): local mesh + DOF manager +
+    device operator on each rank, interface exchange, global Jacobi-PCG."""
+
+    _OP_SLOT = "op"
+
+    def __init__(self, part, order, kind="S", group=None, elems_per_patch=None, exchange="auto",
+                 overlap=True):
+        _StripPoissonBase.__init__(self, part, group, exchange)
+        from . import discrete
+        from .basis_functions import LagrangeGaussLobatto, TensorProductQS
+        self.mesh = part.build_local_mesh(kind)
+        b1 = LagrangeGaussLobatto(order)
+        self.mngr = discrete.DOFManager(self.mesh, 1, TensorProductQS(b1, b1), rcm_order=False)
+        self.on_ebc = self.mngr.boundary_node_mask("ebc")
+        self.op = op = self.mngr.poisson_operator(dirichlet=self.on_ebc,
+                                                  elems_per_patch=elems_per_patch,
+                                                  boundary_columns_first=overlap)
+        self._open_halo(part, exchange, op.dev)
         split = op.boundary_split() if (overlap and self.halo is not None) else None
         self.overlapped = split is not None
         fn = None
         if split is not None:
-            import ctypes as C
-            from . import _lib, device as _dev
-            lib, halo = _lib.load(), self.halo
+            halo = self.halo
 
             def fn(u, out, dir_u8):
-                y = op.new_vector() if out is None else out
-                _lib.check(lib.semk_poisson_apply_halo_f64(
-                    C.byref(op._op), _dev.ptr(u), _dev.ptr(y), int(op._masked_flags), split[0],
-                    split[1], split[2], C.byref(halo.c), _dev.ptr(dir_u8), _dev.stream_ptr()))
-                return y
-        self.dop = DistributedOperator(
-            part, lambda u, out, dot: op.apply(u, out=out, dot_out=dot),
-            dirichlet=self.on_ebc if op.has_dirichlet else None, group=group, device=op.dev,
-            halo=self.halo, dot=self.kernels.dot, overlap=fn)
-        self._mask = op.dirichlet_dev.bool() if op.has_dirichlet else None
-        self._dinv = None
-
-    def apply(self, u, out=None, dot_out=None):
-        return self.dop.apply(u, out=out, dot_out=dot_out)
+                return op.apply_halo(u, out, split, halo.c, dir_u8)
+        self._connect(op, part, overlap=fn)
 
     def host_operator(self):
         """The local operator of the staged host apply: the same elements in the plain tile
@@ -698,62 +767,8 @@ class DistributedPoisson(object):
         torch.cuda.current_stream(op.dev).synchronize()
         return y_host
 
-    def diagonal(self):
-        d = self.op.diagonal(masked=False)
-        self.dop.exchange_add(d)
-        if self._mask is not None:
-            d[self._mask] = 1.0
-        return d
 
-    def rhs(self, f=1.0):
-        return self.dop.exchange_add(self.op.rhs(f))
-
-    def lift(self, b, g=None):
-        """b_f - A_fe g on free rows, g on Dirichlet rows (global operator)."""
-        if self._mask is None:
-            return b.clone()
-        gv = torch.zeros_like(b)
-        if g is not None:
-            gv[self._mask] = g[self._mask]
-        from ._lib import MASK_OUT
-        t = self.op.apply(gv, flags=MASK_OUT)
-        self.dop.exchange_add(t)
-        out = b - t
-        out[self._mask] = gv[self._mask]
-        return out
-
-    def solve_pcg(self, b, x0=None, rtol=1e-12, maxiter=200000, check_every=25, native=True):
-        """Jacobi-PCG over all ranks.  With the peer-memory exchange the native driver
-        semk_pcg_dist_solve_f64 runs the whole loop (``native=False``: the host-driven loop
-        with NCCL all-reduces, which is also what the NCCL / gloo paths use)."""
-        if x0 is None:
-            x = torch.zeros_like(b)
-            if self._mask is not None:
-                x[self._mask] = b[self._mask]
-        else:
-            x = x0.clone()
-        if self._dinv is None:
-            self._dinv = 1.0 / self.diagonal()
-        if self.halo is not None and native:
-            it, rel, ok = _native_jacobi_pcg(self, self.op._op, None, self.halo, self.part.n_owned,
-                                             b, x, self._dinv, self.op.vec_partials, rtol,
-                                             maxiter, check_every)
-            return x, it, rel, ok
-        it, rel, ok = distributed_pcg(self.dop, b, x, self._dinv, self.kernels, rtol=rtol,
-                                      maxiter=maxiter, check_every=check_every)
-        return x, it, rel, ok
-
-    def close(self):
-        """Collective tear-down of the peer-memory regions."""
-        if getattr(self, "_comm", None) is not None:
-            self._comm.close()
-            self._comm = None
-        if self.halo is not None:
-            self.halo.close()
-            self.halo = None
-
-
-class DistributedCondensedPoisson(object):
+class DistributedCondensedPoisson(_StripPoissonBase):
     """The statically condensed Poisson path (condensed.CondensedPoissonOperator,
     the reference's DOFManagerSC formulation, sem/discrete.py:404-528) on a strip
     partition: each rank condenses its own elements (the Schur complements are
@@ -762,12 +777,12 @@ class DistributedCondensedPoisson(object):
     (``CondensedStripView``), PCG runs on the exterior DOFs of all ranks and the
     interior back-substitution is rank-local."""
 
+    _OP_SLOT = "sc_op"
+
     def __init__(self, part, order, kind="S", group=None, exchange="auto"):
+        _StripPoissonBase.__init__(self, part, group, exchange)
         from . import discrete, meshgen
         from .basis_functions import LagrangeGaussLobatto, TensorProductQS
-        from .operators import PCGKernels
-        self.part = part
-        self.group = group
         self.mesh = part.build_local_mesh(kind)
         b1 = LagrangeGaussLobatto(order)
         self.mngr = discrete.DOFManagerSC(self.mesh, 1, TensorProductQS(b1, b1), rcm_order=False)
@@ -778,56 +793,13 @@ class DistributedCondensedPoisson(object):
         lex = meshgen.structured_node_maps(part.nx_local, part.ny, part.p).reshape(-1)
         self.lexicographic_ids = np.empty(self.mesh.n_nodes, dtype=np.int64)
         self.lexicographic_ids[self.mngr.node_map_array().reshape(-1)] = lex
-        self.kernels = PCGKernels(sc, n=sc.n_ext)
-        if exchange not in ("auto", "peer", "nccl"):
-            raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
-        self.halo = None
-        if exchange in ("auto", "peer"):
-            try:
-                self.halo = PeerHalo(self.view, group, sc.dev)
-            except RuntimeError:
-                if exchange == "peer":
-                    raise
-                self.halo = None
-        self.exchange = "peer" if self.halo is not None else "nccl"
-        on_ext = self.on_ebc[:sc.n_ext]
-        self.dop = DistributedOperator(
-            self.view, lambda u, out, dot: sc.apply(u, out=out, dot_out=dot),
-            dirichlet=on_ext if sc.has_dirichlet else None, group=group, device=sc.dev,
-            halo=self.halo, dot=self.kernels.dot)
-        self._mask = sc.dirichlet_dev.bool() if sc.has_dirichlet else None
-        self._dinv = None
+        self._open_halo(self.view, exchange, sc.dev)
+        self._connect(sc, self.view)
 
     def global_ids(self):
         """Global (lexicographic, whole-mesh) node id of every local node in
         this rank's exterior-first numbering."""
         return self.part.global_ids()[self.lexicographic_ids]
-
-    def apply(self, u, out=None, dot_out=None):
-        return self.dop.apply(u, out=out, dot_out=dot_out)
-
-    def diagonal(self):
-        d = self.sc.diagonal(masked=False)
-        self.dop.exchange_add(d)
-        if self._mask is not None:
-            d[self._mask] = 1.0
-        return d
-
-    def rhs(self, f=1.0):
-        return self.dop.exchange_add(self.sc.rhs(f))
-
-    def lift(self, b, g=None):
-        if self._mask is None:
-            return b.clone()
-        gv = torch.zeros_like(b)
-        if g is not None:
-            gv[self._mask] = g[:self.sc.n_ext][self._mask]
-        from ._lib import MASK_OUT
-        t = self.sc.apply(gv, flags=MASK_OUT)
-        self.dop.exchange_add(t)
-        out = b - t
-        out[self._mask] = gv[self._mask]
-        return out
 
     def solve_pcg(self, b, x0=None, rtol=1e-12, maxiter=200000, check_every=25,
                   preconditioner="jacobi", inner_rtol=1e-2, inner_maxiter=20000, flexible=True,
@@ -841,38 +813,24 @@ class DistributedCondensedPoisson(object):
         (true residual, inner iterations) of a multilevel solve."""
         if preconditioner not in ("jacobi", "two-level", "three-level"):
             raise ValueError("preconditioner must be 'jacobi', 'two-level' or 'three-level'")
-        if x0 is None:
-            x = torch.zeros_like(b)
-            if self._mask is not None:
-                x[self._mask] = b[self._mask]
-        else:
-            x = x0.clone()
-        if self._dinv is None:
-            self._dinv = 1.0 / self.diagonal()
-        if preconditioner != "jacobi":
-            ml = self._multilevel(3 if preconditioner == "three-level" else 2, max_tiles)
-            # ranks enter together: the peer kernels give up after ~2 s of waiting
-            torch.cuda.synchronize(self.sc.dev)
-            dist.barrier(group=self.group)
-            xs, info = self.sc.solve_pcg(
-                b, x0=x, rtol=rtol, maxiter=maxiter, preconditioner=preconditioner,
-                inner_rtol=inner_rtol, inner_maxiter=inner_maxiter, flexible=flexible,
-                inner_chunk=inner_chunk, max_tiles=max_tiles,
-                dist=(ml["dist"], self._dinv, ml["dinv_c"]))
-            self.halo.check()
-            ml["halo_c"].check()
-            ml["comm"].check()
-            self.last_info = info
-            self.last_inner_iterations = info.inner_iterations
-            return xs, info.iterations, info.rel_residual, info.converged
-        if self.halo is not None and native:
-            it, rel, ok = _native_jacobi_pcg(self, None, self.sc._op, self.halo, self.view.n_owned,
-                                             b, x, self._dinv, self.sc.vec_partials, rtol, maxiter,
-                                             check_every)
-            return x, it, rel, ok
-        it, rel, ok = distributed_pcg(self.dop, b, x, self._dinv, self.kernels, rtol=rtol,
-                                      maxiter=maxiter, check_every=check_every)
-        return x, it, rel, ok
+        if preconditioner == "jacobi":
+            return _StripPoissonBase.solve_pcg(self, b, x0, rtol, maxiter, check_every, native)
+        x = self._start(b, x0)
+        ml = self._multilevel(3 if preconditioner == "three-level" else 2, max_tiles)
+        # ranks enter together: the peer kernels give up after ~2 s of waiting
+        torch.cuda.synchronize(self.sc.dev)
+        dist.barrier(group=self.group)
+        xs, info = self.sc.solve_pcg(
+            b, x0=x, rtol=rtol, maxiter=maxiter, preconditioner=preconditioner,
+            inner_rtol=inner_rtol, inner_maxiter=inner_maxiter, flexible=flexible,
+            inner_chunk=inner_chunk, max_tiles=max_tiles,
+            dist=(ml["dist"], self._dinv, ml["dinv_c"]))
+        self.halo.check()
+        ml["halo_c"].check()
+        ml["comm"].check()
+        self.last_info = info
+        self.last_inner_iterations = info.inner_iterations
+        return xs, info.iterations, info.rel_residual, info.converged
 
     def _multilevel(self, levels, max_tiles=4096):
         """Coarse levels of the multilevel preconditioner on the strip partition (lazy):
@@ -932,12 +890,7 @@ class DistributedCondensedPoisson(object):
             if tl["comm"] is not None:
                 tl["comm"].close()
             self._ml = None
-        if getattr(self, "_comm", None) is not None:
-            self._comm.close()
-            self._comm = None
-        if self.halo is not None:
-            self.halo.close()
-            self.halo = None
+        _StripPoissonBase.close(self)
 
     def solve(self, f=1.0, dirichlet_values=None, **pcg_kwargs):
         """Condensed load, lifting, distributed PCG on the exterior DOFs, rank-local

@@ -636,6 +636,18 @@ class PoissonOperator(_PoissonBase):
             int(ce), int(rb), int(re), device.stream_ptr()))
         return y
 
+    def apply_halo(self, u, out, split, halo, dirichlet_u8):
+        """The apply of one rank of a strip partition with its interface exchange overlapped
+        (semk_poisson_apply_halo_f64): the patches of ``split`` (``boundary_split``) first,
+        then the exchange of ``halo`` (a semk_halo struct; uint8 Dirichlet mask
+        ``dirichlet_u8``) on a side stream while the interior patches run."""
+        self._no_robin("apply_halo")
+        y = self.new_vector() if out is None else out
+        _lib.check(self._lib.semk_poisson_apply_halo_f64(
+            C.byref(self._op), device.ptr(u), device.ptr(y), int(self._masked_flags), split[0],
+            split[1], split[2], C.byref(halo), device.ptr(dirichlet_u8), device.stream_ptr()))
+        return y
+
     def apply_host(self, u_host, y_host, scratch=None, stages=16):
         """End-to-end call on HOST buffers (numpy float64 or pinned torch CPU
         tensors): H2D copy, apply, D2H copy, synchronised on return.  With

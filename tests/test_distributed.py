@@ -339,6 +339,17 @@ def test_condensed_strip_view_description():
     assert views[1].NY == NYn and views[1].base is parts[1]
 
 
+def test_unknown_exchange_is_rejected_before_any_set_up():
+    """Both strip wrappers check ``exchange`` before they build a mesh, a DOF manager or a
+    device operator: no GPU and no process group is needed to get the error."""
+    from spectralelementmethod_b200.distributed import (DistributedCondensedPoisson,
+                                                        DistributedPoisson, StripPartition)
+    part = StripPartition(0, 2, 2, 2, 2)
+    for cls in (DistributedPoisson, DistributedCondensedPoisson):
+        with pytest.raises(ValueError, match="exchange"):
+            cls(part, 2, exchange="bogus")
+
+
 # --------------------------------------------------------------------------
 # two-level preconditioner on two ranks: algorithm-level emulation (oracle operators,
 # the product's host tables and partition views) of the scheme the device path will use

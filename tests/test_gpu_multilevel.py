@@ -259,7 +259,7 @@ def test_halo_exchange_kernel_self_exchange(with_dirichlet):
 
 @pytest.mark.parametrize("nx,ny,p", [(12, 24, 8), (13, 9, 4), (6, 16, 5)])
 def test_overlapped_apply_and_exchange_on_one_gpu(nx, ny, p):
-    """semk_poisson_apply_halo_f64 on ONE GPU: boundary tile columns first, the light exchange
+    """PoissonOperator.apply_halo on ONE GPU: boundary tile columns first, the light exchange
     kernel on the side stream with the rank as its own left and right neighbour (a periodic
     strip), interior patches meanwhile.  Must equal the serial sequence apply -> exchange
     bit for bit, and the range-split apply must equal the one-launch apply."""
@@ -292,10 +292,7 @@ def test_overlapped_apply_and_exchange_on_one_gpu(nx, ny, p):
         m = torch.from_numpy(on.astype(np.uint8)).cuda()
         stream = torch.cuda.current_stream().cuda_stream
         for rep in range(3):
-            y = op.new_vector()
-            _lib.check(lib.semk_poisson_apply_halo_f64(
-                C.byref(op._op), u.data_ptr(), y.data_ptr(), int(op._masked_flags), split[0],
-                split[1], split[2], C.byref(halo), m.data_ptr(), stream))
+            y = op.apply_halo(u, op.new_vector(), split, halo, m)
             torch.cuda.synchronize()
             assert int(status.item()) == 0 and halo.epoch == 2 * rep + 1
             want = y_one.clone()
