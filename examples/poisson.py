@@ -12,7 +12,7 @@ the matrix-free device operator and the device-resident Jacobi-PCG.
 
     python examples/poisson.py [--n 64] [--order 8] [--msh file.msh] [--kind S|C]
                                [--solver matrix-free|condensed|condensed-two-level]
-                               [--bc reference|neumann|robin] [--convergence]
+                               [--bc reference|neumann|robin] [--convergence] [--eigen K]
 
 ``--solver condensed`` follows the reference example literally: static
 condensation of the element interiors (DOFManagerSC, sem/discrete.py:404-528),
@@ -26,6 +26,10 @@ max nodal, L2 and H1 errors against u are printed (``DOFManager.error_norms``), 
 of the solution through "nbc" (``DOFManager.boundary_flux``) beside the integral of the
 exact flux.  ``--convergence`` solves that problem on the same mesh for p = 2 ... 10 and
 prints one row per order: the errors fall exponentially in p.
+
+``--eigen K`` computes the K smallest eigenvalues of -lap(u) = lambda u with the example's
+boundary layout instead -- u = 0 on "ebc", du/dn = 0 on "nbc" (``DOFManager.poisson_eigenpairs``)
+-- and prints them beside the exact ones, pi^2/16 ((2m+1)^2 + (2n+1)^2), m, n >= 0.
 
 With ``--msh`` the mesh is read from a Gmsh 2.2 binary file with physical
 names "ebc", "nbc" (lines) and a surface (the reference's examples/meshes/
@@ -157,6 +161,29 @@ def convergence(n=8, kind="S", solver="matrix-free", bc="neumann", orders=range(
                  abs(rep["flux"] - rep["flux_exact"])))
 
 
+def eigen(k, n=16, order=8, kind="S", msh=None):
+    """The k smallest eigenvalues with u = 0 on "ebc" and natural "nbc", beside the exact ones of
+    the square [-1, 1]^2."""
+    if msh is not None:
+        mesh = grid_importers.load_msh(msh, 2)
+    else:
+        mesh = meshgen.structured_quad_mesh(n, n, order, kind)
+    b1 = LagrangeGaussLobatto(order)
+    mngr = discrete.DOFManagerSC(mesh, 1, TensorProductQS(b1, b1), rcm_order=False)
+    t0 = time.perf_counter()
+    lam, _x, info = mngr.poisson_eigenpairs(k, dirichlet="ebc")
+    t = time.perf_counter() - t0
+    r = np.arange(k + 1)
+    ex = np.sort((np.pi ** 2 / 16) * ((2 * r[:, None] + 1) ** 2 + (2 * r[None, :] + 1) ** 2),
+                 axis=None)[:k]
+    print("mesh: %d cells of order %d, %d DOF; %d LOBPCG iterations (%s preconditioner), %.2f s"
+          % (mesh.n_cells, order, mngr.ndof, info["iterations"], info["preconditioner"], t))
+    print("%3s %22s %22s %10s" % ("i", "lambda", "exact", "rel. err"))
+    for i in range(k):
+        print("%3d %22.15f %22.15f %10.2e" % (i, lam[i], ex[i], abs(lam[i] - ex[i]) / ex[i]))
+    return lam, ex
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=64, help="cells per side of the structured mesh")
@@ -173,7 +200,13 @@ def main():
                     help="solve the manufactured problem (--bc neumann unless robin is given) "
                          "for p = 2 ... 10 on the structured --n x --n mesh and print the "
                          "errors per order")
+    ap.add_argument("--eigen", type=int, default=0, metavar="K",
+                    help="print the K smallest eigenvalues (u = 0 on \"ebc\", natural \"nbc\") "
+                         "beside the exact ones instead of solving")
     args = ap.parse_args()
+    if args.eigen:
+        eigen(args.eigen, args.n, args.order, args.kind, args.msh)
+        return
     if args.convergence:
         convergence(args.n, args.kind, args.solver, "robin" if args.bc == "robin" else "neumann")
         return

@@ -991,6 +991,32 @@ int semk_vec_scale_add_f64(int64_t n, double alpha, const double *a, const doubl
 int semk_block2_apply_f64(int64_t n_nodes, const double *binv, const double *r, double *z,
                           void *stream);
 
+/* Block-vector kernels of the block eigensolver (eigen.py).  A block of m vectors of length n
+ * is stored as rows X + i*ldx, i < m, ldx >= n; 1 <= m, k <= 96.
+ *   semk_block_gram_f64    : G[i*k + j] = sum_t X[i*ldx + t] * w[t] * Y[j*ldy + t]   (w == NULL:
+ *                            w = 1).  X, Y and w are read once; fixed per-CTA ranges, the last
+ *                            CTA adds the partial matrices in CTA order: bitwise reproducible for
+ *                            a given (n, m, k).  partials: semk_block_gram_partials_len(m, k)
+ *                            doubles (-1 for m or k out of range), zero-filled once before the
+ *                            first call; every call leaves it ready for the next one, of any
+ *                            m' k' <= m k.
+ *   semk_block_combine_f64 : Y[j] = beta * Y[j] + sum_i C[i*k + j] X[i], j < k (C [m][k] on the
+ *                            device; Y must not overlap X; beta == 0 does not read Y). */
+int64_t semk_block_gram_partials_len(int m, int k);
+int semk_block_gram_f64(int64_t n, int m, const double *X, int64_t ldx, int k, const double *Y,
+                        int64_t ldy, const double *w, double *G, double *partials, void *stream);
+/* The same Gram matrix with the inner product fixed: DFMA (FP64 FMA) or DMMA (FP64 mma.sync
+ * m8n8k4).  semk_block_gram_f64 is the one of the two that measured faster (DESIGN.md section 7);
+ * each is bitwise reproducible on its own. */
+int semk_block_gram_dfma_f64(int64_t n, int m, const double *X, int64_t ldx, int k,
+                             const double *Y, int64_t ldy, const double *w, double *G,
+                             double *partials, void *stream);
+int semk_block_gram_dmma_f64(int64_t n, int m, const double *X, int64_t ldx, int k,
+                             const double *Y, int64_t ldy, const double *w, double *G,
+                             double *partials, void *stream);
+int semk_block_combine_f64(int64_t n, int m, const double *X, int64_t ldx, int k, const double *C,
+                           double beta, double *Y, int64_t ldy, void *stream);
+
 /* A sub-range of semk_poisson_apply_f64: patches [patch_begin, patch_end) and the interface
  * entries [chunk_begin, chunk_end) / [rec_begin, rec_end).  Both interface tables are sorted
  * by the highest patch involved, so what patches [0, P) complete is a prefix of each

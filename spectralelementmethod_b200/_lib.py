@@ -260,6 +260,11 @@ SIGNATURES = {
     "semk_multi_axpy_f64": (_I, [_L, _I, _P, _L, _P, _D, _P, _P]),
     "semk_vec_scale_add_f64": (_I, [_L, _D, _P, _P, _P, _P]),
     "semk_block2_apply_f64": (_I, [_L, _P, _P, _P, _P]),
+    "semk_block_gram_partials_len": (_L, [_I, _I]),
+    "semk_block_gram_f64": (_I, [_L, _I, _P, _L, _I, _P, _L, _P, _P, _P, _P]),
+    "semk_block_gram_dfma_f64": (_I, [_L, _I, _P, _L, _I, _P, _L, _P, _P, _P, _P]),
+    "semk_block_gram_dmma_f64": (_I, [_L, _I, _P, _L, _I, _P, _L, _P, _P, _P, _P]),
+    "semk_block_combine_f64": (_I, [_L, _I, _P, _L, _I, _P, _D, _P, _L, _P]),
 }
 
 _lib = None

@@ -694,6 +694,21 @@ class CondensedPoissonOperator(_PoissonBase):
         x, info = self.solve_pcg(b, **pcg_kwargs)
         return self.backsolve(x, f), info
 
+    def solve_load(self, r, f, rtol=1e-8, preconditioner="three-level"):
+        """u = A^-1 r for an assembled nodal load vector ``r`` (length n_nodes, zero on the
+        Dirichlet nodes).  ``f = r * inv_mass_int``: r divided by the mass on the element-
+        interior nodes and zero on the exterior ones, the nodal values whose element load JxW f
+        is r on every interior node.  Condensed load of f plus the exterior entries of r
+        (semk_sc_rhs_finish_f64), PCG on the exterior DOFs to ``rtol``, interior
+        back-substitution.  Returns (u[n_nodes], PCGInfo)."""
+        g = self.rhs(f)
+        b = torch.empty_like(g)
+        _lib.check(self._lib.semk_sc_rhs_finish_f64(
+            self.n_ext, device.ptr(g), device.ptr(r), device.ptr(self.dirichlet_dev)
+            if self.has_dirichlet else None, device.ptr(b), device.stream_ptr()))
+        x, info = self.solve_pcg(b, rtol=rtol, preconditioner=preconditioner)
+        return self.backsolve(x, f), info
+
 
 class CondensedLocalSystems(CondensedPoissonOperator):
     """Static condensation of the CALLER'S OWN dense local systems: the literal

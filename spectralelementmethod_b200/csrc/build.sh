@@ -6,7 +6,7 @@ NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -O3"
 OBJS=""
 PIDS=""
-for f in semk_api.cu semk_geom.cu semk_apply.cu semk_box.cu semk_vec.cu semk_peer.cu semk_sc.cu semk_field.cu semk_ml.cu semk_ho.cu semk_locate.cu semk_stokes.cu; do
+for f in semk_api.cu semk_geom.cu semk_apply.cu semk_box.cu semk_vec.cu semk_peer.cu semk_sc.cu semk_field.cu semk_ml.cu semk_ho.cu semk_locate.cu semk_stokes.cu semk_block.cu; do
   [ -f "$f" ] || continue
   o="${f%.cu}.o"
   if [ ! -f "$o" ] || [ "$f" -nt "$o" ] || [ semk_common.cuh -nt "$o" ] || [ semk_elem.cuh -nt "$o" ] || [ semk_patch.cuh -nt "$o" ] || [ ../../include/semk.h -nt "$o" ]; then

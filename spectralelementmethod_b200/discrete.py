@@ -591,6 +591,30 @@ class DOFManager(object):
         return PoissonOperator(self, dirichlet=dirichlet,
                                geometric_factors=geometric_factors, **kwargs)
 
+    def poisson_eigenpairs(self, k, dirichlet=None, robin=None, weight=None, tol=1e-8,
+                           maxiter=500):
+        """The ``k`` smallest eigenpairs of ``K x = lambda M x`` on the GPU: ``K`` the stiffness
+        of -div(w grad u) with these boundary conditions, ``M`` the diagonal GLL mass
+        (block eigensolver LOBPCG, see eigen.py).
+
+        k : 1 <= k <= 32 and smaller than the number of free nodes.
+        dirichlet : bool[n_nodes], a boundary name or a list of names, optional -- u = 0 there.
+        robin : {boundary name: alpha}, optional -- w du/dn + alpha u = 0 there (alpha >= 0);
+            every other boundary is natural (w du/dn = 0).
+        weight : as for ``poisson_operator``.
+        tol : pair i has converged when ||K x_i - lambda_i M x_i||_{M^-1} / max_j |lambda_j|
+            <= tol (x_i M-normalised); the eigenvalue error is about its square.
+
+        The preconditioner follows from the DOF manager: the condensed three-level solve for a
+        ``DOFManagerSC`` (orders 2..10), Jacobi otherwise; for K + M when K is singular (no
+        Dirichlet node, no Robin boundary).  Returns ``(lam, X, info)``: ``lam`` float64[k]
+        ascending, ``X`` a CUDA tensor [k, n_nodes], M-orthonormal and zero on the Dirichlet
+        nodes, ``info`` a dict (iterations, per-pair residuals, converged flags, preconditioner
+        applications, time per phase)."""
+        from .eigen import poisson_eigenpairs
+        return poisson_eigenpairs(self, k, dirichlet=dirichlet, robin=robin, weight=weight,
+                                  tol=tol, maxiter=maxiter)
+
     def axisymmetric_stokes_operator(self, n_rey=0.0, essential=None, **kwargs):
         """Matrix-free Jacobian / residual of the axisymmetric stream function - vorticity
         system of examples/squirmer-axisymmetric.py:163-297 on the GPU (two DOFs per node;

@@ -599,18 +599,12 @@ class PoissonBlockPreconditioner(object):
     def poisson_solve(self, r, f=None):
         """u = Khat^-1 r for a nodal residual r (zero on the Dirichlet nodes); f = r *
         inv_mass_int if the caller has it already."""
-        sc, lib = self.sc, self.op._lib
         if f is None:
             f = r * self.inv_mass_int
-        g = sc.rhs(f)
-        b = torch.empty_like(g)
-        _lib.check(lib.semk_sc_rhs_finish_f64(
-            self.n_ext, device.ptr(g), device.ptr(r), device.ptr(sc.dirichlet_dev)
-            if sc.has_dirichlet else None, device.ptr(b), device.stream_ptr()))
-        x, info = sc.solve_pcg(b, rtol=self.rtol, preconditioner=self.kind)
+        u, info = self.sc.solve_load(r, f, rtol=self.rtol, preconditioner=self.kind)
         self.solves += 1
         self.inner_outer_iterations += info.iterations
-        return sc.backsolve(x, f)
+        return u
 
     def __call__(self, src, dst):
         op, lib, n = self.op, self.op._lib, self.op.n_nodes
