@@ -580,6 +580,41 @@ int semk_sc_backsolve_stored_f64(int n1, int64_t n_elem, const double *W, const 
                                  const uint32_t *l2g, const int32_t *ext_loc, double *u,
                                  void *stream);
 
+/* Block loads: the three entries above for k load columns at once (host-only query of the
+ * largest k: semk_sc_block_max_cols, 32 for n1 in 3..11 and -1 otherwise; a larger k returns
+ * SEMK_ERR_UNSUPPORTED).  Every block is a [k][ld] device array, row j at offset j * ld.
+ * Column j's load is f_scale[j] * JxW * (bit j of nodal_mask ? F[j][l2g] : 1); f_scale is a
+ * host array of k entries, F [k][ldf] is read only in the nodal columns.  Column j of every
+ * output is bitwise the output of the single-load entry on load j: the same operations in
+ * the same order, whatever k and the other columns.
+ *
+ * semk_sc_element_block_f64: one CTA per element factorises A_ii once for all k columns.
+ *   mode SEMK_SC_RHS: g_loc [k][ldg >= n_elem * 4p] = f_e - A_ei A_ii^{-1} f_i (the condensed
+ *   load of compute_local_sc_system, sem/discrete.py:438-476), and, if c_out is not NULL,
+ *   c_out [k][ldc >= n_elem * (p-1)^2] = A_ii^{-1} f_i.  Mode SEMK_SC_BACKSOLVE: U [k][ldu]
+ *   nodal vectors, exterior entries read, interior entries written with
+ *   u_i = A_ii^{-1} (f_i - A_ie u_e) (_solve_interior_dofs, sem/discrete.py:513-524).
+ *   G ... react as semk_sc_element_react_f64.
+ * semk_sc_load_stored_block_f64: semk_sc_load_stored_f64 per column, A_ii^{-1} and W read once.
+ * semk_sc_backsolve_stored_block_f64: semk_sc_backsolve_stored_f64 per column, W read once;
+ *   c [k][ldc] or NULL (zero load). */
+int semk_sc_block_max_cols(int n1);
+int semk_sc_element_block_f64(int n1, int64_t n_elem, const double *G, int64_t g_patch_stride,
+                              int elems_per_patch, const double *D, const int32_t *ext_loc,
+                              const uint32_t *l2g, const double *JxW, const double *react,
+                              int mode, int k, const double *F, int64_t ldf, uint32_t nodal_mask,
+                              const double *f_scale, double *g_loc, int64_t ldg, double *c_out,
+                              int64_t ldc, double *U, int64_t ldu, int32_t *bad_flag,
+                              void *stream);
+int semk_sc_load_stored_block_f64(int n1, int64_t n_elem, const double *W, const double *Ainv,
+                                  const uint32_t *l2g, const int32_t *ext_loc, const double *JxW,
+                                  int k, const double *F, int64_t ldf, uint32_t nodal_mask,
+                                  const double *f_scale, double *g_loc, int64_t ldg, double *c_out,
+                                  int64_t ldc, void *stream);
+int semk_sc_backsolve_stored_block_f64(int n1, int64_t n_elem, const double *W, const double *c,
+                                       int64_t ldc, const uint32_t *l2g, const int32_t *ext_loc,
+                                       int k, double *U, int64_t ldu, void *stream);
+
 /* The same element kernel on the CALLER'S OWN local systems instead of the Poisson
  * recipe -- the literal inputs of DOFManagerSC.assemble_global_sc_system / solve
  * (sem/discrete.py:478-528): A_hier device [n_elem][NN][NN] and f_hier device

@@ -203,6 +203,12 @@ SIGNATURES = {
                                        _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "semk_sc_load_stored_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _D, _P, _P, _P]),
     "semk_sc_backsolve_stored_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P]),
+    "semk_sc_block_max_cols": (_I, [_I]),
+    "semk_sc_element_block_f64": (_I, [_I, _L, _P, _L, _I, _P, _P, _P, _P, _P, _I, _I, _P, _L,
+                                       C.c_uint32, _P, _P, _L, _P, _L, _P, _L, _P, _P]),
+    "semk_sc_load_stored_block_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _I, _P, _L, C.c_uint32,
+                                           _P, _P, _L, _P, _L, _P]),
+    "semk_sc_backsolve_stored_block_f64": (_I, [_I, _L, _P, _P, _L, _P, _P, _I, _P, _L, _P]),
     "semk_sc_element_dense_f64": (_I, [_I, _L, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P, _P]),
     "semk_sc_apply_f64": (_I, [C.POINTER(semk_sc_op), _P, _P, _I, _P, _P]),
     "semk_sc_assemble_f64": (_I, [C.POINTER(semk_sc_op), _P, _P, _I, _D, _P]),

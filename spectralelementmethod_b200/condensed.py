@@ -709,6 +709,242 @@ class CondensedPoissonOperator(_PoissonBase):
         x, info = self.solve_pcg(b, rtol=rtol, preconditioner=preconditioner)
         return self.backsolve(x, f), info
 
+    # -- blocks of loads ---------------------------------------------------------------
+    # Column j of every *_many result is bitwise the single-load call on load j: the block
+    # kernels (semk_sc_element_block_f64 and the stored-operator streams) factorise each
+    # element once per chunk of columns and repeat the single kernels' operations per column,
+    # and every column takes the path the single call would take.
+    def _block_cap(self):
+        return int(self._lib.semk_sc_block_max_cols(self.n1))
+
+    def _block_chunks(self, k):
+        """Column ranges of a block of k loads (block_chunks with this operator's cap, the
+        temporaries g_loc and c of one column and the free device memory)."""
+        per_col = 8 * self.n_elem * (self.n_ext_loc + self.n_int_loc)
+        return block_chunks(k, self._block_cap(), per_col, torch.cuda.mem_get_info(self.dev)[0])
+
+    def _block_loads(self, F):
+        """(columns [(f_scale, nodal CUDA vector or None, cacheable)], F if it is a block)."""
+        if isinstance(F, torch.Tensor):
+            if not (F.is_cuda and F.dtype == torch.float64 and F.dim() == 2
+                    and F.shape[1] == self.n_nodes and F.stride(1) == 1 and F.shape[0] >= 1):
+                raise ValueError("F must be a float64 CUDA [k, n_nodes] block (k >= 1) with "
+                                 "contiguous rows, or a sequence of loads")
+            return [(1.0, F[j], True) for j in range(F.shape[0])], F
+        cols = []
+        for f in F:
+            if isinstance(f, torch.Tensor):
+                cols.append((1.0, self._vec(f, "f", self.n_nodes), True))
+            elif np.ndim(f) == 0:
+                cols.append((float(f), None, True))
+            else:     # a host array: not cacheable, as in rhs / backsolve
+                cols.append((1.0, self._vec(self.from_host(f), "f", self.n_nodes), False))
+        if not cols:
+            raise ValueError("a block of loads needs at least one column")
+        return cols, None
+
+    def _block_groups(self, cols):
+        """Column index lists, each taking one path.  With W kept, the columns whose interior
+        solution the single path caches (CUDA and scalar loads) are split from the others
+        (host arrays), so that each column's load and back-solve use the single path's
+        kernels."""
+        k = len(cols)
+        if getattr(self, "_W", None) is None:
+            return [(False, list(range(k)))]
+        hit = [j for j in range(k) if cols[j][2]]
+        miss = [j for j in range(k) if not cols[j][2]]
+        return [(cached, g) for cached, g in ((True, hit), (False, miss)) if g]
+
+    def _chunk_load(self, cols, idx, block):
+        """(F, ldf, nodal mask, f_scale ctypes array) of the columns ``idx``."""
+        sub = [cols[j] for j in idx]
+        mask = 0
+        for q, (_, t, _) in enumerate(sub):
+            if t is not None:
+                mask |= 1 << q
+        scales = (C.c_double * len(sub))(*[s for s, _, _ in sub])
+        if not mask:
+            return None, 0, 0, scales
+        if block is not None and idx == list(range(idx[0], idx[0] + len(idx))):
+            return block[idx[0]:idx[0] + len(idx)], block.stride(0), mask, scales
+        Fs = torch.empty((len(sub), self.n_nodes), dtype=torch.float64, device=self.dev)
+        for q, (_, t, _) in enumerate(sub):
+            if t is not None:
+                Fs[q].copy_(t)
+        return Fs, self.n_nodes, mask, scales
+
+    def _element_block(self, mode, load, g_loc=None, c=None, U=None):
+        """One launch of sc_element_block_kernel (csrc/semk_sc.cu)."""
+        F, ldf, mask, scales = load
+        self._bad.zero_()
+        _lib.check(self._lib.semk_sc_element_block_f64(
+            self.n1, self.n_elem, device.ptr(self.G), self.g_stride, 1,
+            device.ptr(self.tab.dev()[0]), device.ptr(self._t["ext_loc"]),
+            device.ptr(self.l2g_dev), device.ptr(self.JxW), device.ptr(self._react), int(mode),
+            len(scales), device.ptr(F), int(ldf), mask, scales, device.ptr(g_loc),
+            self.n_elem * self.n_ext_loc, device.ptr(c), self.n_elem * self.n_int_loc,
+            device.ptr(U), 0 if U is None else U.stride(0), device.ptr(self._bad),
+            device.stream_ptr()))
+        if int(self._bad.item()) != 0:
+            raise AssertionError("an element-interior stiffness block is not positive definite")
+
+    def _block_rhs(self, cols, block, keep_c):
+        """Element-local condensed loads, chunk by chunk: yields (column ids, g_loc [kc, E, 4p],
+        c [kc, E, (p-1)^2] = A_ii^-1 f_i or None, load descriptor).  ``keep_c``: compute c where
+        the single path would cache it (W kept, cacheable load)."""
+        f64 = dict(dtype=torch.float64, device=self.dev)
+        stored_load = (getattr(self, "_Ainv", None) is not None and self._W is not None
+                       and type(self) is CondensedPoissonOperator)
+        for cacheable, group in self._block_groups(cols):
+            for j0, j1 in self._block_chunks(len(group)):
+                idx = group[j0:j1]
+                kc = len(idx)
+                load = self._chunk_load(cols, idx, block)
+                F, ldf, mask, scales = load
+                g_loc = torch.empty((kc, self.n_elem, self.n_ext_loc), **f64)
+                c = None
+                if cacheable and (keep_c or stored_load):
+                    c = torch.empty((kc, self.n_elem, self.n_int_loc), **f64)
+                if cacheable and stored_load:
+                    _lib.check(self._lib.semk_sc_load_stored_block_f64(
+                        self.n1, self.n_elem, device.ptr(self._W), device.ptr(self._Ainv),
+                        device.ptr(self.l2g_dev), device.ptr(self._t["ext_loc"]),
+                        device.ptr(self.JxW), kc, device.ptr(F), int(ldf), mask, scales,
+                        device.ptr(g_loc), self.n_elem * self.n_ext_loc, device.ptr(c),
+                        self.n_elem * self.n_int_loc, device.stream_ptr()))
+                else:
+                    self._element_block(_lib.SC_RHS, load, g_loc=g_loc, c=c)
+                yield idx, g_loc, (c if keep_c else None), load
+
+    def _block_backsolve(self, X, idx, load, c, U):
+        """Rows ``idx`` of the nodal block U from the exterior solutions X [kc, n_ext]: the
+        stream over W with the loads' c, else the element pass on the loads."""
+        contiguous = idx == list(range(idx[0], idx[0] + len(idx)))
+        Ub = U[idx[0]:idx[0] + len(idx)] if contiguous else torch.empty(
+            (len(idx), self.n_nodes), dtype=torch.float64, device=self.dev)
+        Ub[:, :self.n_ext].copy_(X)
+        if c is not None:
+            _lib.check(self._lib.semk_sc_backsolve_stored_block_f64(
+                self.n1, self.n_elem, device.ptr(self._W), device.ptr(c),
+                self.n_elem * self.n_int_loc, device.ptr(self.l2g_dev),
+                device.ptr(self._t["ext_loc"]), len(idx), device.ptr(Ub), Ub.stride(0),
+                device.stream_ptr()))
+        else:
+            self._element_block(_lib.SC_BACKSOLVE, load, U=Ub)
+        if not contiguous:
+            for q, j in enumerate(idx):
+                U[j].copy_(Ub[q])
+
+    def _block_out(self, out, k, n, what="out"):
+        if out is None:
+            return torch.empty((k, n), dtype=torch.float64, device=self.dev)
+        if not (isinstance(out, torch.Tensor) and out.is_cuda and out.dtype == torch.float64
+                and tuple(out.shape) == (k, n) and out.stride(1) == 1):
+            raise ValueError("%s must be a float64 CUDA [%d, %d] block with contiguous rows"
+                             % (what, k, n))
+        return out
+
+    def _block_vectors(self, X, k, n, what):
+        """Rows of a [k, n] CUDA block or a sequence of k vectors of length n."""
+        rows = list(X) if not isinstance(X, torch.Tensor) or X.dim() == 2 else None
+        if rows is None or len(rows) != k:
+            raise ValueError("%s must be a [%d, %d] block or %d vectors" % (what, k, n, k))
+        return [self._vec(r, what, n) for r in rows]
+
+    def rhs_many(self, F):
+        """Condensed loads of a block of loads, ``[k, n_ext]``: row j is ``rhs(F[j])``.
+        ``F``: a float64 CUDA ``[k, n_nodes]`` block or a sequence of loads in any form
+        ``rhs`` accepts."""
+        cols, block = self._block_loads(F)
+        out = torch.empty((len(cols), self.n_ext), dtype=torch.float64, device=self.dev)
+        for idx, g_loc, _, _ in self._block_rhs(cols, block, keep_c=False):
+            for q, j in enumerate(idx):
+                self.assemble(g_loc[q], out=out[j])
+        return out
+
+    def backsolve_many(self, X_ext, F, out=None):
+        """Full nodal vectors ``[k, n_nodes]`` from exterior solutions ``X_ext`` ([k, n_ext] or
+        k vectors) and their loads ``F``: row j is ``backsolve(X_ext[j], F[j])`` when that call
+        does not find the load in the single-load cache (the interiors are recomputed)."""
+        cols, block = self._block_loads(F)
+        k = len(cols)
+        X = self._block_vectors(X_ext, k, self.n_ext, "X_ext")
+        U = self._block_out(out, k, self.n_nodes)
+        for j0, j1 in self._block_chunks(k):
+            idx = list(range(j0, j1))
+            Xc = torch.stack(X[j0:j1])
+            self._block_backsolve(Xc, idx, self._chunk_load(cols, idx, block), None, U)
+        return U
+
+    def _solve_block(self, cols, block, out, condensed_rhs, pcg):
+        """Shared loop of solve_many / solve_load_many: per chunk the block load pass, per
+        column ``condensed_rhs(j, g)`` and ``pcg(j, b)``, then the block back-solve."""
+        k = len(cols)
+        U = self._block_out(out, k, self.n_nodes)
+        infos = [None] * k
+        for idx, g_loc, c, load in self._block_rhs(cols, block, keep_c=True):
+            X = torch.empty((len(idx), self.n_ext), dtype=torch.float64, device=self.dev)
+            for q, j in enumerate(idx):
+                x, infos[j] = pcg(j, condensed_rhs(j, self.assemble(g_loc[q])))
+                X[q].copy_(x)
+            del g_loc
+            self._block_backsolve(X, idx, load, c, U)
+        return U, infos
+
+    def solve_many(self, F, dirichlet_values=None, flux=None, **pcg_kwargs):
+        """``solve`` for a block of loads: returns (U [k, n_nodes], [PCGInfo] * k), row j
+        bitwise ``solve(F[j], ...)``.  ``F`` as in ``rhs_many``; ``dirichlet_values`` and
+        ``flux`` are one value for every column or a list of k.  PCG runs column by column."""
+        cols, block = self._block_loads(F)
+        k = len(cols)
+
+        def per_column(v, what):
+            if isinstance(v, (list, tuple)):
+                if len(v) != k:
+                    raise ValueError("%s: a list must have one entry per load (%d)" % (what, k))
+                return list(v)
+            return [v] * k
+
+        dv = per_column(dirichlet_values, "dirichlet_values")
+        fl = per_column(flux, "flux")
+
+        def condensed_rhs(j, b):
+            for name, g in (fl[j] or {}).items():
+                b += self.boundary_load(name, g)
+            return self.lift(b, dv[j])
+
+        return self._solve_block(cols, block, None, condensed_rhs,
+                                 lambda j, b: self.solve_pcg(b, **pcg_kwargs))
+
+    def solve_load_many(self, R, F, rtol=1e-8, preconditioner="three-level", out=None):
+        """``solve_load`` for a block: R and F are [k, n_nodes] blocks or sequences of k nodal
+        CUDA vectors; returns (U [k, n_nodes] or ``out``, [PCGInfo] * k), row j bitwise
+        ``solve_load(R[j], F[j], rtol, preconditioner)``."""
+        cols, block = self._block_loads(F)
+        R = self._block_vectors(R, len(cols), self.n_nodes, "R")
+        mask = device.ptr(self.dirichlet_dev) if self.has_dirichlet else None
+
+        def condensed_rhs(j, g):
+            b = torch.empty_like(g)
+            _lib.check(self._lib.semk_sc_rhs_finish_f64(
+                self.n_ext, device.ptr(g), device.ptr(R[j]), mask, device.ptr(b),
+                device.stream_ptr()))
+            return b
+
+        return self._solve_block(cols, block, out, condensed_rhs,
+                                 lambda j, b: self.solve_pcg(b, rtol=rtol,
+                                                             preconditioner=preconditioner))
+
+
+def block_chunks(k, cap, bytes_per_col, free_bytes):
+    """Column ranges ``[(j0, j1)]`` of a block of ``k`` loads: at most ``cap`` columns each,
+    fewer when ``free_bytes`` would not hold ``bytes_per_col`` per column, at least one."""
+    k, cap = int(k), int(cap)
+    if k < 1 or cap < 1:
+        raise ValueError("a block needs k >= 1 columns and a cap >= 1")
+    width = max(1, min(cap, int(free_bytes) // max(int(bytes_per_col), 1)))
+    return [(j0, min(j0 + width, k)) for j0 in range(0, k, width)]
+
 
 class CondensedLocalSystems(CondensedPoissonOperator):
     """Static condensation of the CALLER'S OWN dense local systems: the literal
@@ -764,6 +1000,12 @@ class CondensedLocalSystems(CondensedPoissonOperator):
         b = self.lift(self.rhs(), dirichlet_values)
         x, info = self.solve_pcg(b, **pcg_kwargs)
         return self.backsolve(x), info
+
+    def _no_blocks(self, *args, **kwargs):
+        raise NotImplementedError("CondensedLocalSystems holds one load (the caller's local "
+                                  "right-hand sides); blocks of loads are not supported")
+
+    rhs_many = backsolve_many = solve_many = solve_load_many = _no_blocks
 
 
 def coarse_tables(l2g_ext, node_ptr, node_pos, dirichlet, gll_nodes):

@@ -82,6 +82,117 @@ struct ScElemArgs {
   double *Ainv_out;            // [n_elem][NI][NI] A_ii^{-1} (mode STORE_INV), or nullptr
 };
 
+// ---- element work shared by sc_element_kernel and sc_element_block_kernel -----------------
+// Local stiffness entry (p,q),(r,s) from the staged factors (closed form in the file header).
+template <int N>
+__device__ __forceinline__ double sc_entry(const double *sG, const double *sD, const double *sR,
+                                           int p, int q, int r, int s) {
+  constexpr int NN = N * N;
+  double v = sD[r * N + p] * sG[NN + r * N + q] * sD[q * N + s] +
+             sD[p * N + r] * sG[NN + p * N + s] * sD[s * N + q];
+  if (q == s) {
+#pragma unroll
+    for (int m = 0; m < N; ++m) v = fma(sD[m * N + p] * sD[m * N + r], sG[m * N + q], v);
+  }
+  if (p == r) {
+#pragma unroll
+    for (int n = 0; n < N; ++n)
+      v = fma(sD[n * N + s] * sD[n * N + q], sG[2 * NN + p * N + n], v);
+    if (q == s) v += sR[p * N + q];
+  }
+  return v;
+}
+
+// Stage element e's geometric factors, D, reaction term and exterior index table.
+template <int N>
+__device__ __forceinline__ void sc_stage_element(int64_t e, const int64_t *slot_of_elem,
+                                                 const double *G, int64_t g_patch_stride, int pe,
+                                                 const double *D, const double *react,
+                                                 const int32_t *ext_loc, double *sG, double *sD,
+                                                 double *sR, int *sExt, int tid) {
+  constexpr int NN = N * N, NE = ScCfg<N>::NE;
+  const int NP = N * pe;
+  const int64_t slot = slot_of_elem ? slot_of_elem[e] : e;
+  const int64_t patch = slot / pe;
+  const int lp = (int)(slot - patch * pe);
+  const double *g = G + patch * g_patch_stride + lp * N;
+  for (int i = tid; i < 3 * NN; i += kScThreads) {
+    const int c = i / NN, k = i - c * NN;
+    const int m = k / N, n = k - m * N;
+    sG[i] = g[(c * N + m) * NP + n];
+  }
+  for (int i = tid; i < NN; i += kScThreads) sD[i] = D[i];
+  for (int i = tid; i < NN; i += kScThreads) sR[i] = react ? react[e * NN + i] : 0.0;
+  for (int i = tid; i < NE; i += kScThreads) sExt[i] = ext_loc[i];
+}
+
+// Interior block (lower triangle) into sA and A_ie into the first NE columns of sZ.
+template <int N>
+__device__ __forceinline__ void sc_build_interior(const double *sG, const double *sD,
+                                                  const double *sR, const int *sExt, double *sA,
+                                                  double *sZ, int ldz, int tid) {
+  constexpr int NE = ScCfg<N>::NE, NI = ScCfg<N>::NI, LDI = ScCfg<N>::LDI, M = N - 2;
+  for (int idx = tid; idx < NI * NI; idx += kScThreads) {
+    const int i = idx / NI, j = idx - i * NI;
+    if (j <= i)
+      sA[i * LDI + j] = sc_entry<N>(sG, sD, sR, 1 + i / M, 1 + i % M, 1 + j / M, 1 + j % M);
+  }
+  for (int idx = tid; idx < NI * NE; idx += kScThreads) {
+    const int i = idx / NE, k = idx - i * NE;
+    const int x = sExt[k];
+    sZ[i * ldz + k] = sc_entry<N>(sG, sD, sR, 1 + i / M, 1 + i % M, x / N, x % N);
+  }
+}
+
+// A_ii = L L^T, right-looking, in place (lower triangle); sInv[i] = 1 / L[i][i].
+template <int N>
+__device__ __forceinline__ void sc_cholesky(double *sA, double *sInv, int *sBad, int tid) {
+  constexpr int NI = ScCfg<N>::NI, LDI = ScCfg<N>::LDI;
+  const int tx = tid % kScTX, ty = tid / kScTX;
+  for (int k = 0; k < NI; ++k) {
+    const double d = sA[k * LDI + k];  // nobody writes (k,k) during step k
+    const double inv = 1.0 / sqrt(d);
+    if (tid == 0) {
+      sInv[k] = inv;
+      if (!(d > 0.0)) *sBad = 1;
+    }
+    for (int i = k + 1 + tid; i < NI; i += kScThreads) sA[i * LDI + k] *= inv;
+    __syncthreads();
+    for (int i = k + 1 + ty; i < NI; i += kScTY) {
+      const double lik = sA[i * LDI + k];
+      for (int j = k + 1 + tx; j <= i; j += kScTX)
+        sA[i * LDI + j] = fma(-lik, sA[j * LDI + k], sA[i * LDI + j]);
+    }
+    __syncthreads();
+  }
+}
+
+// Columns [0, ncols) of sZ <- L^{-1} sZ: one thread per column, forward substitution.
+template <int N>
+__device__ __forceinline__ void sc_forward(const double *sA, const double *sInv, double *sZ,
+                                           int ldz, int ncols, int tid) {
+  constexpr int NI = ScCfg<N>::NI, LDI = ScCfg<N>::LDI;
+  if (tid < ncols) {
+    for (int i = 0; i < NI; ++i) {
+      double acc = sZ[i * ldz + tid];
+      for (int j = 0; j < i; ++j) acc = fma(-sA[i * LDI + j], sZ[j * ldz + tid], acc);
+      sZ[i * ldz + tid] = acc * sInv[i];
+    }
+  }
+}
+
+// Column col of sZ <- L^{-T} sZ (backward substitution in place), by the calling thread.
+template <int N>
+__device__ __forceinline__ void sc_backward_col(const double *sA, const double *sInv, double *sZ,
+                                                int ldz, int col) {
+  constexpr int NI = ScCfg<N>::NI, LDI = ScCfg<N>::LDI;
+  for (int i = NI - 1; i >= 0; --i) {
+    double acc = sZ[i * ldz + col];
+    for (int j = i + 1; j < NI; ++j) acc = fma(-sA[j * LDI + i], sZ[j * ldz + col], acc);
+    sZ[i * ldz + col] = acc * sInv[i];
+  }
+}
+
 template <int N>
 __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
   using C = ScCfg<N>;
@@ -102,41 +213,17 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
   int *sExt = reinterpret_cast<int *>(sX + NI * LDI);  // [NE] lexicographic index of exterior k
   int *sBad = sExt + NE;
   const int tid = threadIdx.x;
-  const int tx = tid % kScTX, ty = tid / kScTX;
-  const int NP = N * a.pe;
   const bool need_f = (a.mode & (SEMK_SC_RHS | SEMK_SC_BACKSOLVE)) != 0;
 
   auto entry = [&](int p, int q, int r, int s) -> double {
-    double v = sD[r * N + p] * sG[NN + r * N + q] * sD[q * N + s] +
-               sD[p * N + r] * sG[NN + p * N + s] * sD[s * N + q];
-    if (q == s) {
-#pragma unroll
-      for (int m = 0; m < N; ++m) v = fma(sD[m * N + p] * sD[m * N + r], sG[m * N + q], v);
-    }
-    if (p == r) {
-#pragma unroll
-      for (int n = 0; n < N; ++n)
-        v = fma(sD[n * N + s] * sD[n * N + q], sG[2 * NN + p * N + n], v);
-      if (q == s) v += sR[p * N + q];
-    }
-    return v;
+    return sc_entry<N>(sG, sD, sR, p, q, r, s);
   };
 
   for (int64_t e = blockIdx.x; e < a.n_elem; e += gridDim.x) {
     __syncthreads();  // the previous element is completely done with shared memory
     if (!a.A_dense) {
-      const int64_t slot = a.slot_of_elem ? a.slot_of_elem[e] : e;
-      const int64_t patch = slot / a.pe;
-      const int lp = (int)(slot - patch * a.pe);
-      const double *g = a.G + patch * a.g_patch_stride + lp * N;
-      for (int i = tid; i < 3 * NN; i += kScThreads) {
-        const int c = i / NN, k = i - c * NN;
-        const int m = k / N, n = k - m * N;
-        sG[i] = g[(c * N + m) * NP + n];
-      }
-      for (int i = tid; i < NN; i += kScThreads) sD[i] = a.D[i];
-      for (int i = tid; i < NN; i += kScThreads) sR[i] = a.react ? a.react[e * NN + i] : 0.0;
-      for (int i = tid; i < NE; i += kScThreads) sExt[i] = a.ext_loc[i];
+      sc_stage_element<N>(e, a.slot_of_elem, a.G, a.g_patch_stride, a.pe, a.D, a.react,
+                          a.ext_loc, sG, sD, sR, sExt, tid);
     }
     if (tid == 0) *sBad = 0;
     __syncthreads();
@@ -167,15 +254,7 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
         }
       }
     } else {
-    for (int idx = tid; idx < NI * NI; idx += kScThreads) {
-      const int i = idx / NI, j = idx - i * NI;
-      if (j <= i) sA[i * LDI + j] = entry(1 + i / M, 1 + i % M, 1 + j / M, 1 + j % M);
-    }
-    for (int idx = tid; idx < NI * NE; idx += kScThreads) {
-      const int i = idx / NE, k = idx - i * NE;
-      const int x = sExt[k];
-      sZ[i * LDZ + k] = entry(1 + i / M, 1 + i % M, x / N, x % N);
-    }
+    sc_build_interior<N>(sG, sD, sR, sExt, sA, sZ, LDZ, tid);
     for (int idx = tid; idx < NE * NE; idx += kScThreads) {
       const int k = idx / NE, l = idx - k * NE;
       if (l <= k) {
@@ -200,31 +279,9 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
       }
     }
     __syncthreads();
-    // ---- A_ii = L L^T, right-looking, in place (lower triangle) --------------------
-    for (int k = 0; k < NI; ++k) {
-      const double d = sA[k * LDI + k];  // nobody writes (k,k) during step k
-      const double inv = 1.0 / sqrt(d);
-      if (tid == 0) {
-        sInv[k] = inv;
-        if (!(d > 0.0)) *sBad = 1;
-      }
-      for (int i = k + 1 + tid; i < NI; i += kScThreads) sA[i * LDI + k] *= inv;
-      __syncthreads();
-      for (int i = k + 1 + ty; i < NI; i += kScTY) {
-        const double lik = sA[i * LDI + k];
-        for (int j = k + 1 + tx; j <= i; j += kScTX)
-          sA[i * LDI + j] = fma(-lik, sA[j * LDI + k], sA[i * LDI + j]);
-      }
-      __syncthreads();
-    }
-    // ---- Z = L^{-1} [A_ie | f_i]: one thread per column, forward substitution -------
-    if (tid < NE + (need_f ? 1 : 0)) {
-      for (int i = 0; i < NI; ++i) {
-        double acc = sZ[i * LDZ + tid];
-        for (int j = 0; j < i; ++j) acc = fma(-sA[i * LDI + j], sZ[j * LDZ + tid], acc);
-        sZ[i * LDZ + tid] = acc * sInv[i];
-      }
-    }
+    sc_cholesky<N>(sA, sInv, sBad, tid);
+    // ---- Z = L^{-1} [A_ie | f_i] ------------------------------------------------------
+    sc_forward<N>(sA, sInv, sZ, LDZ, NE + (need_f ? 1 : 0), tid);
     __syncthreads();
     if (tid == 0 && *sBad) *a.bad_flag = 1;
     // ---- S_e = A_ee - Z^T Z (packed lower triangle, row major) ----------------------
@@ -307,13 +364,7 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
     if (store_w || store_c) {
       __syncthreads();  // every reader of Z is done
       const bool mine = (store_w && tid < NE) || (store_c && tid == NE);
-      if (mine) {
-        for (int i = NI - 1; i >= 0; --i) {
-          double acc = sZ[i * LDZ + tid];
-          for (int j = i + 1; j < NI; ++j) acc = fma(-sA[j * LDI + i], sZ[j * LDZ + tid], acc);
-          sZ[i * LDZ + tid] = acc * sInv[i];
-        }
-      }
+      if (mine) sc_backward_col<N>(sA, sInv, sZ, LDZ, tid);
       __syncthreads();
       if (store_w) {
         double *Wo = a.W_out + e * (int64_t)NE * NI;
@@ -410,6 +461,265 @@ __global__ void __launch_bounds__(256)
       for (int j = 0; j < NI; ++j)
         acc = fma(-Wr[j], sF[grp][(1 + j / M) * N + 1 + j % M], acc);
       g_loc[e * (int64_t)NE + i] = acc;
+    }
+  }
+}
+
+// ---- block loads: up to kScBlockMaxCols load columns per element pass ---------------------
+// Column j's load is f_scale[j] * JxW * (nodal_mask bit j ? F[j][l2g] : 1), the expression of
+// sc_element_kernel, and every column goes through the same operations in the same order as a
+// single-load pass, so each column is bitwise the result of that pass.
+constexpr int kScBlockMaxCols = 32;
+
+struct ScBlockLoad {
+  int k;                            // load columns, 1..kScBlockMaxCols
+  const double *F;                  // [k][ldf] nodal loads (rows of scalar columns unread)
+  int64_t ldf;
+  uint32_t nodal_mask;              // bit j: column j is nodal
+  double f_scale[kScBlockMaxCols];
+};
+
+__device__ __forceinline__ double sc_block_load(const ScBlockLoad &L, int j, const double *jw,
+                                                const uint32_t *row, int x) {
+  const double f = ((L.nodal_mask >> j) & 1u) ? L.F[j * L.ldf + row[x]] : 1.0;
+  return L.f_scale[j] * jw[x] * f;
+}
+
+struct ScBlockArgs {
+  int64_t n_elem;
+  const double *G;
+  int64_t g_patch_stride;
+  int pe;
+  const double *D;
+  const int32_t *ext_loc;
+  const uint32_t *l2g;
+  const double *JxW;
+  const double *react;
+  int mode;                         // SEMK_SC_RHS or SEMK_SC_BACKSOLVE
+  ScBlockLoad L;
+  double *g_loc;                    // RHS: [k][ldg], row j = [n_elem][NE]
+  int64_t ldg;
+  double *c_out;                    // RHS, optional: [k][ldc], row j = [n_elem][NI] = A_ii^{-1} f_i
+  int64_t ldc;
+  double *U;                        // BACKSOLVE: [k][ldu] nodal vectors
+  int64_t ldu;
+  int32_t *bad_flag;
+};
+
+// shared memory of sc_element_block_kernel: Z takes (NE + k) | 1 columns; sV holds f_e (RHS) or
+// u_e (BACKSOLVE) of every column, sT the k back-substitution vectors (BACKSOLVE only)
+template <int N>
+size_t sc_block_smem(int k, int mode) {
+  using C = ScCfg<N>;
+  const size_t ldz = (size_t)((C::NE + k) | 1);
+  const size_t nd = 3 * C::NN + 2 * C::NN + C::NI * C::LDI + C::NI * ldz + C::NI +
+                    (size_t)k * C::NE + (mode == SEMK_SC_BACKSOLVE ? (size_t)k * C::NI : 0);
+  return sizeof(double) * nd + sizeof(int) * (C::NE + 4);
+}
+
+template <int N>
+__global__ void __launch_bounds__(kScThreads, 1) sc_element_block_kernel(ScBlockArgs a) {
+  using C = ScCfg<N>;
+  constexpr int NN = C::NN, NE = C::NE, NI = C::NI, LDI = C::LDI, M = N - 2;
+  const int k = a.L.k, ldz = (NE + k) | 1;
+  const bool back = a.mode == SEMK_SC_BACKSOLVE;
+  extern __shared__ __align__(128) double sc_smem[];
+  double *sG = sc_smem;            // [3][N][N]
+  double *sD = sG + 3 * NN;        // [N][N]
+  double *sR = sD + NN;            // [N][N]
+  double *sA = sR + NN;            // [NI][LDI] -> Cholesky factor
+  double *sZ = sA + NI * LDI;      // [NI][ldz] A_ie | f_i of every column -> L^{-1} of all
+  double *sInv = sZ + NI * ldz;    // [NI]
+  double *sV = sInv + NI;          // [k][NE] f_e (RHS) or u_e (BACKSOLVE)
+  double *sT = sV + k * NE;        // [k][NI] (BACKSOLVE)
+  int *sExt = reinterpret_cast<int *>(sT + (back ? k * NI : 0));
+  int *sBad = sExt + NE;
+  const int tid = threadIdx.x;
+  for (int64_t e = blockIdx.x; e < a.n_elem; e += gridDim.x) {
+    __syncthreads();
+    sc_stage_element<N>(e, nullptr, a.G, a.g_patch_stride, a.pe, a.D, a.react, a.ext_loc, sG, sD,
+                        sR, sExt, tid);
+    if (tid == 0) *sBad = 0;
+    __syncthreads();
+    sc_build_interior<N>(sG, sD, sR, sExt, sA, sZ, ldz, tid);
+    const double *jw = a.JxW + e * NN;
+    const uint32_t *row = a.l2g + e * NN;
+    for (int idx = tid; idx < k * NI; idx += kScThreads) {
+      const int j = idx / NI, i = idx - j * NI;
+      sZ[i * ldz + NE + j] = sc_block_load(a.L, j, jw, row, (1 + i / M) * N + 1 + i % M);
+    }
+    for (int idx = tid; idx < k * NE; idx += kScThreads) {
+      const int j = idx / NE, q = idx - j * NE;
+      sV[idx] = back ? a.U[j * a.ldu + row[sExt[q]]] : sc_block_load(a.L, j, jw, row, sExt[q]);
+    }
+    __syncthreads();
+    sc_cholesky<N>(sA, sInv, sBad, tid);
+    sc_forward<N>(sA, sInv, sZ, ldz, NE + k, tid);
+    __syncthreads();
+    if (tid == 0 && *sBad) *a.bad_flag = 1;
+    if (!back) {
+      // g_e = f_e - Z^T (L^{-1} f_i)
+      for (int idx = tid; idx < k * NE; idx += kScThreads) {
+        const int j = idx / NE, q = idx - j * NE;
+        double acc = sV[idx];
+        for (int i = 0; i < NI; ++i) acc = fma(-sZ[i * ldz + q], sZ[i * ldz + NE + j], acc);
+        a.g_loc[j * a.ldg + e * NE + q] = acc;
+      }
+      if (a.c_out) {  // c = L^{-T} (L^{-1} f_i), one thread per column
+        __syncthreads();
+        if (tid < k) sc_backward_col<N>(sA, sInv, sZ, ldz, NE + tid);
+        __syncthreads();
+        for (int idx = tid; idx < k * NI; idx += kScThreads) {
+          const int j = idx / NI, i = idx - j * NI;
+          a.c_out[j * a.ldc + e * NI + i] = sZ[i * ldz + NE + j];
+        }
+      }
+    } else {
+      // u_i = L^{-T} (L^{-1} f_i - Z u_e): the product one thread per entry, the backward
+      // sweep one warp per column
+      for (int idx = tid; idx < k * NI; idx += kScThreads) {
+        const int j = idx / NI, i = idx - j * NI;
+        const double *ue = sV + j * NE;
+        double acc = sZ[i * ldz + NE + j];
+        for (int q = 0; q < NE; ++q) acc = fma(-sZ[i * ldz + q], ue[q], acc);
+        sT[idx] = acc;
+      }
+      __syncthreads();
+      const int warp = tid >> 5, lane = tid & 31;
+      for (int j = warp; j < k; j += kScThreads / 32) {
+        double *t = sT + j * NI;
+        for (int i = NI - 1; i >= 0; --i) {
+          const double xi = t[i] * sInv[i];
+          __syncwarp();
+          if (lane == 0) t[i] = xi;
+          for (int jj = lane; jj < i; jj += 32) t[jj] = fma(-sA[i * LDI + jj], xi, t[jj]);
+          __syncwarp();
+        }
+      }
+      __syncthreads();
+      for (int idx = tid; idx < k * NI; idx += kScThreads) {
+        const int j = idx / NI, i = idx - j * NI;
+        a.U[j * a.ldu + row[(1 + i / M) * N + 1 + i % M]] = sT[idx];
+      }
+    }
+  }
+}
+
+// sc_backsolve_stored_kernel for k <= KB columns: W is read once for all of them; column j of
+// u_i is c[j] - W u_e[j], the same fma chain as the single kernel.  KB (1, 2, 4, ... 32) is the
+// register tile: the launch takes the smallest that holds k, so that a few columns do not pay
+// for 32 predicated accumulators.
+template <int N, int KB>
+__global__ void __launch_bounds__(256, 1)
+    sc_backsolve_stored_block_kernel(int64_t n_elem, const double *__restrict__ W,
+                                     const double *__restrict__ c, int64_t ldc,
+                                     const uint32_t *__restrict__ l2g,
+                                     const int32_t *__restrict__ ext_loc, int k,
+                                     double *__restrict__ U, int64_t ldu) {
+  using C = ScCfg<N>;
+  constexpr int NN = C::NN, NE = C::NE, NI = C::NI, M = N - 2;
+  constexpr int GT = ((NI + 31) / 32) * 32;
+  constexpr int GPB = 256 / GT;
+  extern __shared__ __align__(128) double sc_smem[];   // [GPB][k][NE] exterior values
+  const int tid = threadIdx.x;
+  const int grp = tid / GT, i = tid - grp * GT;
+  double *sUe = sc_smem + (grp < GPB ? grp : 0) * k * NE;
+  const int64_t n_steps = (n_elem + GPB - 1) / GPB;
+  for (int64_t step = blockIdx.x; step < n_steps; step += gridDim.x) {
+    const int64_t e = step * GPB + grp;
+    const bool on = grp < GPB && e < n_elem;
+    __syncthreads();
+    if (on) {
+      const uint32_t *row = l2g + e * NN;
+      for (int idx = i; idx < k * NE; idx += GT) {
+        const int j = idx / NE, q = idx - j * NE;
+        sUe[idx] = U[j * ldu + row[ext_loc[q]]];
+      }
+    }
+    __syncthreads();
+    if (on && i < NI) {
+      double acc[KB];
+#pragma unroll
+      for (int j = 0; j < KB; ++j)
+        acc[j] = (j < k && c) ? c[j * ldc + e * (int64_t)NI + i] : 0.0;
+      const double *Wt = W + e * (int64_t)NE * NI + i;
+      for (int q = 0; q < NE; ++q) {
+        const double w = __ldcs(Wt + (int64_t)q * NI);
+#pragma unroll
+        for (int j = 0; j < KB; ++j)
+          if (j < k) acc[j] = fma(-w, sUe[j * NE + q], acc[j]);
+      }
+      const int64_t g = l2g[e * NN + (1 + i / M) * N + 1 + i % M];
+#pragma unroll
+      for (int j = 0; j < KB; ++j)
+        if (j < k) U[j * ldu + g] = acc[j];
+    }
+  }
+}
+
+// sc_load_stored_kernel for k <= KB columns: A_ii^{-1} and W are read once for all of them.
+template <int N, int KB>
+__global__ void __launch_bounds__(256)
+    sc_load_stored_block_kernel(int64_t n_elem, const double *__restrict__ W,
+                                const double *__restrict__ Ainv, const uint32_t *__restrict__ l2g,
+                                const int32_t *__restrict__ ext_loc,
+                                const double *__restrict__ JxW, ScBlockLoad L,
+                                double *__restrict__ g_loc, int64_t ldg,
+                                double *__restrict__ c_out, int64_t ldc) {
+  using C = ScCfg<N>;
+  constexpr int NN = C::NN, NE = C::NE, NI = C::NI, M = N - 2;
+  constexpr int GT = ((NI + 31) / 32) * 32;
+  constexpr int GPB = 256 / GT;
+  extern __shared__ __align__(128) double sc_smem[];   // [GPB][k][NN] element loads
+  const int k = L.k;
+  const int tid = threadIdx.x;
+  const int grp = tid / GT, i = tid - grp * GT;
+  double *sF = sc_smem + (grp < GPB ? grp : 0) * k * NN;
+  const int64_t n_steps = (n_elem + GPB - 1) / GPB;
+  for (int64_t step = blockIdx.x; step < n_steps; step += gridDim.x) {
+    const int64_t e = step * GPB + grp;
+    const bool on = grp < GPB && e < n_elem;
+    __syncthreads();
+    if (on) {
+      const uint32_t *row = l2g + e * NN;
+      const double *jw = JxW + e * NN;
+      for (int idx = i; idx < k * NN; idx += GT) {
+        const int j = idx / NN, x = idx - j * NN;
+        sF[idx] = sc_block_load(L, j, jw, row, x);
+      }
+    }
+    __syncthreads();
+    double acc[KB];
+    if (on && i < NI) {
+      const double *Ac = Ainv + e * (int64_t)NI * NI + i;
+#pragma unroll
+      for (int j = 0; j < KB; ++j) acc[j] = 0.0;
+      for (int jj = 0; jj < NI; ++jj) {
+        const double v = __ldcs(Ac + (int64_t)jj * NI);
+        const int x = (1 + jj / M) * N + 1 + jj % M;
+#pragma unroll
+        for (int j = 0; j < KB; ++j)
+          if (j < k) acc[j] = fma(v, sF[j * NN + x], acc[j]);
+      }
+#pragma unroll
+      for (int j = 0; j < KB; ++j)
+        if (j < k) c_out[j * ldc + e * (int64_t)NI + i] = acc[j];
+    }
+    if (on && i < NE) {
+      const double *Wr = W + e * (int64_t)NE * NI + (int64_t)i * NI;
+      const int xe = ext_loc[i];
+#pragma unroll
+      for (int j = 0; j < KB; ++j) acc[j] = j < k ? sF[j * NN + xe] : 0.0;
+      for (int jj = 0; jj < NI; ++jj) {
+        const double w = Wr[jj];
+        const int x = (1 + jj / M) * N + 1 + jj % M;
+#pragma unroll
+        for (int j = 0; j < KB; ++j)
+          if (j < k) acc[j] = fma(-w, sF[j * NN + x], acc[j]);
+      }
+#pragma unroll
+      for (int j = 0; j < KB; ++j)
+        if (j < k) g_loc[j * ldg + e * (int64_t)NE + i] = acc[j];
     }
   }
 }
@@ -645,6 +955,69 @@ int check_sc_op(const semk_sc_op *op, const char *who) {
   return SEMK_OK;
 }
 
+// launch of a stored block kernel with the smallest register tile KB >= k
+template <int N, int KB>
+int launch_load_stored_block(int64_t n_elem, const double *W, const double *Ainv,
+                             const uint32_t *l2g, const int32_t *ext_loc, const double *JxW,
+                             const ScBlockLoad &L, double *g_loc, int64_t ldg, double *c_out,
+                             int64_t ldc, cudaStream_t st) {
+  constexpr int GT = ((ScCfg<N>::NI + 31) / 32) * 32, GPB = 256 / GT;
+  const size_t smem = sizeof(double) * (size_t)GPB * L.k * ScCfg<N>::NN;
+  SEMK_CUDA_CHECK(cudaFuncSetAttribute(sc_load_stored_block_kernel<N, KB>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)(sizeof(double) * GPB * KB * ScCfg<N>::NN)));
+  const int64_t steps = (n_elem + GPB - 1) / GPB;
+  const unsigned grid = (unsigned)(steps < 148 * 16 ? steps : 148 * 16);
+  sc_load_stored_block_kernel<N, KB><<<grid, 256, smem, st>>>(n_elem, W, Ainv, l2g, ext_loc, JxW,
+                                                              L, g_loc, ldg, c_out, ldc);
+  return SEMK_OK;
+}
+
+template <int N, int KB>
+int launch_backsolve_stored_block(int64_t n_elem, const double *W, const double *c, int64_t ldc,
+                                  const uint32_t *l2g, const int32_t *ext_loc, int k, double *U,
+                                  int64_t ldu, cudaStream_t st) {
+  constexpr int GT = ((ScCfg<N>::NI + 31) / 32) * 32, GPB = 256 / GT;
+  const size_t smem = sizeof(double) * (size_t)GPB * k * ScCfg<N>::NE;
+  const int64_t steps = (n_elem + GPB - 1) / GPB;
+  const unsigned grid = (unsigned)(steps < 148 * 16 ? steps : 148 * 16);
+  sc_backsolve_stored_block_kernel<N, KB><<<grid, 256, smem, st>>>(n_elem, W, c, ldc, l2g,
+                                                                   ext_loc, k, U, ldu);
+  return SEMK_OK;
+}
+
+template <int N>
+int launch_load_stored_block_tiled(int64_t n_elem, const double *W, const double *Ainv,
+                                   const uint32_t *l2g, const int32_t *ext_loc, const double *JxW,
+                                   const ScBlockLoad &L, double *g_loc, int64_t ldg,
+                                   double *c_out, int64_t ldc, cudaStream_t st) {
+#define SEMK_TILE(KB) \
+  return launch_load_stored_block<N, KB>(n_elem, W, Ainv, l2g, ext_loc, JxW, L, g_loc, ldg, \
+                                         c_out, ldc, st)
+  if (L.k <= 1) SEMK_TILE(1);
+  if (L.k <= 2) SEMK_TILE(2);
+  if (L.k <= 4) SEMK_TILE(4);
+  if (L.k <= 8) SEMK_TILE(8);
+  if (L.k <= 16) SEMK_TILE(16);
+  SEMK_TILE(32);
+#undef SEMK_TILE
+}
+
+template <int N>
+int launch_backsolve_stored_block_tiled(int64_t n_elem, const double *W, const double *c,
+                                        int64_t ldc, const uint32_t *l2g, const int32_t *ext_loc,
+                                        int k, double *U, int64_t ldu, cudaStream_t st) {
+#define SEMK_TILE(KB) \
+  return launch_backsolve_stored_block<N, KB>(n_elem, W, c, ldc, l2g, ext_loc, k, U, ldu, st)
+  if (k <= 1) SEMK_TILE(1);
+  if (k <= 2) SEMK_TILE(2);
+  if (k <= 4) SEMK_TILE(4);
+  if (k <= 8) SEMK_TILE(8);
+  if (k <= 16) SEMK_TILE(16);
+  SEMK_TILE(32);
+#undef SEMK_TILE
+}
+
 }  // namespace
 
 #define SEMK_DISPATCH_SC(n1, CALL)                                                   \
@@ -840,6 +1213,148 @@ extern "C" int semk_sc_load_stored_f64(int n1, int64_t n_elem, const double *W, 
   SEMK_DISPATCH_SC(n1, SEMK_CALL)
 #undef SEMK_CALL
   SEMK_LAUNCH_CHECK("sc_load_stored_kernel");
+  return SEMK_OK;
+}
+
+extern "C" int semk_sc_block_max_cols(int n1) {
+  return (n1 >= 3 && n1 <= 11) ? kScBlockMaxCols : -1;
+}
+
+// common checks of the block entries; fills the load descriptor
+static int sc_block_load_args(const char *who, int n1, int k, const double *F, int64_t ldf,
+                              uint32_t nodal_mask, const double *f_scale, ScBlockLoad *L) {
+  if (n1 < 3 || n1 > 11) {
+    semk_set_error(std::string(who) + ": static condensation supports orders 2..10");
+    return SEMK_ERR_UNSUPPORTED;
+  }
+  if (k > kScBlockMaxCols) {
+    semk_set_error(std::string(who) + ": more load columns than semk_sc_block_max_cols");
+    return SEMK_ERR_UNSUPPORTED;
+  }
+  SEMK_REQUIRE(k >= 1, (std::string(who) + ": k must be >= 1").c_str());
+  SEMK_REQUIRE(f_scale, (std::string(who) + ": f_scale must not be NULL").c_str());
+  const uint32_t cols = k == 32 ? 0xFFFFFFFFu : ((1u << k) - 1u);
+  SEMK_REQUIRE((nodal_mask & ~cols) == 0 && (!nodal_mask || (F && ldf > 0)),
+               (std::string(who) + ": nodal columns need F and ldf > 0").c_str());
+  L->k = k;
+  L->F = F;
+  L->ldf = ldf;
+  L->nodal_mask = nodal_mask;
+  for (int j = 0; j < kScBlockMaxCols; ++j) L->f_scale[j] = j < k ? f_scale[j] : 0.0;
+  return SEMK_OK;
+}
+
+extern "C" int semk_sc_element_block_f64(int n1, int64_t n_elem, const double *G,
+                                         int64_t g_patch_stride, int elems_per_patch,
+                                         const double *D, const int32_t *ext_loc,
+                                         const uint32_t *l2g, const double *JxW,
+                                         const double *react, int mode, int k, const double *F,
+                                         int64_t ldf, uint32_t nodal_mask, const double *f_scale,
+                                         double *g_loc, int64_t ldg, double *c_out, int64_t ldc,
+                                         double *U, int64_t ldu, int32_t *bad_flag,
+                                         void *stream) {
+  ScBlockArgs a;
+  int rc = sc_block_load_args("semk_sc_element_block_f64", n1, k, F, ldf, nodal_mask, f_scale,
+                              &a.L);
+  if (rc != SEMK_OK) return rc;
+  SEMK_REQUIRE(n_elem > 0 && G && D && ext_loc && l2g && JxW && bad_flag && elems_per_patch > 0 &&
+                   g_patch_stride > 0,
+               "semk_sc_element_block_f64: bad argument");
+  SEMK_REQUIRE(mode == SEMK_SC_RHS || mode == SEMK_SC_BACKSOLVE,
+               "semk_sc_element_block_f64: mode must be SEMK_SC_RHS or SEMK_SC_BACKSOLVE");
+  const int ne = 4 * (n1 - 1), ni = (n1 - 2) * (n1 - 2);
+  if (mode == SEMK_SC_RHS) {
+    SEMK_REQUIRE(g_loc && ldg >= n_elem * ne && (!c_out || ldc >= n_elem * ni),
+                 "semk_sc_element_block_f64: RHS needs g_loc [k][ldg >= n_elem * 4p] (and c_out "
+                 "[k][ldc >= n_elem * (p-1)^2])");
+  } else {
+    SEMK_REQUIRE(U && ldu > 0 && !c_out,
+                 "semk_sc_element_block_f64: BACKSOLVE needs U [k][ldu] and no c_out");
+  }
+  a.n_elem = n_elem;
+  a.G = G;
+  a.g_patch_stride = g_patch_stride;
+  a.pe = elems_per_patch;
+  a.D = D;
+  a.ext_loc = ext_loc;
+  a.l2g = l2g;
+  a.JxW = JxW;
+  a.react = react;
+  a.mode = mode;
+  a.g_loc = g_loc;
+  a.ldg = ldg;
+  a.c_out = c_out;
+  a.ldc = ldc;
+  a.U = U;
+  a.ldu = ldu;
+  a.bad_flag = bad_flag;
+  cudaStream_t st = semk_stream(stream);
+  const unsigned grid = (unsigned)(n_elem < 148 * 16 ? n_elem : 148 * 16);
+#define SEMK_CALL(NV)                                                                      \
+  do {                                                                                     \
+    const size_t smem = sc_block_smem<NV>(k, mode);                                        \
+    SEMK_CUDA_CHECK(cudaFuncSetAttribute(sc_element_block_kernel<NV>,                      \
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize,      \
+                                         (int)sc_block_smem<NV>(kScBlockMaxCols,           \
+                                                                SEMK_SC_BACKSOLVE)));      \
+    sc_element_block_kernel<NV><<<grid, kScThreads, smem, st>>>(a);                        \
+  } while (0)
+  SEMK_DISPATCH_SC(n1, SEMK_CALL)
+#undef SEMK_CALL
+  SEMK_LAUNCH_CHECK("sc_element_block_kernel");
+  return SEMK_OK;
+}
+
+extern "C" int semk_sc_load_stored_block_f64(int n1, int64_t n_elem, const double *W,
+                                             const double *Ainv, const uint32_t *l2g,
+                                             const int32_t *ext_loc, const double *JxW, int k,
+                                             const double *F, int64_t ldf, uint32_t nodal_mask,
+                                             const double *f_scale, double *g_loc, int64_t ldg,
+                                             double *c_out, int64_t ldc, void *stream) {
+  ScBlockLoad L;
+  int rc = sc_block_load_args("semk_sc_load_stored_block_f64", n1, k, F, ldf, nodal_mask,
+                              f_scale, &L);
+  if (rc != SEMK_OK) return rc;
+  const int ne = 4 * (n1 - 1), ni = (n1 - 2) * (n1 - 2);
+  SEMK_REQUIRE(n_elem > 0 && W && Ainv && l2g && ext_loc && JxW && g_loc && c_out &&
+                   ldg >= n_elem * ne && ldc >= n_elem * ni,
+               "semk_sc_load_stored_block_f64: bad argument");
+  cudaStream_t st = semk_stream(stream);
+#define SEMK_CALL(NV)                                                                      \
+  rc = launch_load_stored_block_tiled<NV>(n_elem, W, Ainv, l2g, ext_loc, JxW, L, g_loc, ldg, \
+                                          c_out, ldc, st)
+  SEMK_DISPATCH_SC(n1, SEMK_CALL)
+#undef SEMK_CALL
+  if (rc != SEMK_OK) return rc;
+  SEMK_LAUNCH_CHECK("sc_load_stored_block_kernel");
+  return SEMK_OK;
+}
+
+extern "C" int semk_sc_backsolve_stored_block_f64(int n1, int64_t n_elem, const double *W,
+                                                  const double *c, int64_t ldc,
+                                                  const uint32_t *l2g, const int32_t *ext_loc,
+                                                  int k, double *U, int64_t ldu, void *stream) {
+  const char *who = "semk_sc_backsolve_stored_block_f64";
+  if (n1 < 3 || n1 > 11) {
+    semk_set_error(std::string(who) + ": static condensation supports orders 2..10");
+    return SEMK_ERR_UNSUPPORTED;
+  }
+  if (k > kScBlockMaxCols) {
+    semk_set_error(std::string(who) + ": more columns than semk_sc_block_max_cols");
+    return SEMK_ERR_UNSUPPORTED;
+  }
+  const int ni = (n1 - 2) * (n1 - 2);
+  SEMK_REQUIRE(k >= 1 && n_elem > 0 && W && l2g && ext_loc && U && ldu > 0 &&
+                   (!c || ldc >= n_elem * ni),
+               "semk_sc_backsolve_stored_block_f64: bad argument");
+  cudaStream_t st = semk_stream(stream);
+#define SEMK_CALL(NV) \
+  rc = launch_backsolve_stored_block_tiled<NV>(n_elem, W, c, ldc, l2g, ext_loc, k, U, ldu, st)
+  int rc = SEMK_OK;
+  SEMK_DISPATCH_SC(n1, SEMK_CALL)
+#undef SEMK_CALL
+  if (rc != SEMK_OK) return rc;
+  SEMK_LAUNCH_CHECK("sc_backsolve_stored_block_kernel");
   return SEMK_OK;
 }
 

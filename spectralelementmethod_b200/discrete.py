@@ -606,8 +606,10 @@ class DOFManager(object):
             <= tol (x_i M-normalised); the eigenvalue error is about its square.
 
         The preconditioner follows from the DOF manager: the condensed three-level solve for a
-        ``DOFManagerSC`` (orders 2..10), Jacobi otherwise; for K + M when K is singular (no
-        Dirichlet node, no Robin boundary).  Returns ``(lam, X, info)``: ``lam`` float64[k]
+        ``DOFManagerSC`` (orders 2..10), applied to all active residuals of an iteration at once
+        (``CondensedPoissonOperator.solve_load_many``: one element factorisation per chunk of up
+        to 32 columns, every column bitwise the single solve), Jacobi otherwise; for K + M when
+        K is singular (no Dirichlet node, no Robin boundary).  Returns ``(lam, X, info)``: ``lam`` float64[k]
         ascending, ``X`` a CUDA tensor [k, n_nodes], M-orthonormal and zero on the Dirichlet
         nodes, ``info`` a dict (iterations, per-pair residuals, converged flags, preconditioner
         applications, time per phase)."""

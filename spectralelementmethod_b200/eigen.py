@@ -201,25 +201,27 @@ def poisson_eigenpairs(dm, k, dirichlet=None, robin=None, weight=None, tol=1e-8,
         kind = "jacobi"
     stats = {"applications": 0, "inner_iterations": 0}
 
-    def precondition(R, J, W):
-        """W[q] = T R[J[q]]."""
+    def precondition(R, J, W, F):
+        """W[q] = T R[J[q]]; F: len(J) free rows for the loads of the condensed solves."""
         stats["applications"] += len(J)
         if sc is None:
             for q, j in enumerate(J):
                 torch.mul(R[int(j)], dinv, out=W[q])
             return
-        for q, j in enumerate(J):
-            r = R[int(j)]
-            u, pinfo = sc.solve_load(r, r * inv_mass_int, rtol=CONDENSED_RTOL,
-                                     preconditioner="three-level")
-            W[q].copy_(u)
-            stats["inner_iterations"] += pinfo.iterations
+        rows = [R[int(j)] for j in J]
+        for q, r in enumerate(rows):
+            torch.mul(r, inv_mass_int, out=F[q])
+        _, pinfos = sc.solve_load_many(rows, F, rtol=CONDENSED_RTOL, preconditioner="three-level",
+                                       out=W)
+        stats["inner_iterations"] += sum(pinfo.iterations for pinfo in pinfos)
 
     # -- block storage -------------------------------------------------------------------
     # the block buffers plus the preconditioner's temporaries; the returned X (k vectors) is
     # copied out after three of the four buffers are freed
     n_vec = _BLOCKS_PER_PAIR * k + (_SCRATCH_VECTORS if sc is not None else 0)
     need = 8 * n * n_vec
+    if sc is not None:       # the element-local loads of one chunk of the block solve
+        need += 8 * sc.n_elem * (sc.n_ext_loc + sc.n_int_loc) * min(k, sc._block_cap())
     avail = torch.cuda.mem_get_info(dev)[0]
     if need > avail:
         raise MemoryError("poisson_eigenpairs: %d nodal vectors for k = %d need %.1f GB of device "
@@ -304,7 +306,7 @@ def poisson_eigenpairs(dm, k, dirichlet=None, robin=None, weight=None, tol=1e-8,
         # W = T R on the active columns, M-orthogonal to X, M-orthonormal (CholQR2), K W
         clock("preconditioner")
         Wraw = nxt[:ka]
-        precondition(R, J, Wraw)
+        precondition(R, J, Wraw, nxt[2 * k:2 * k + ka])
         clock("block")
         Wraw.mul_(free)
         C1 = blk.gram(X, Wraw, M)
