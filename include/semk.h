@@ -226,6 +226,12 @@ typedef struct semk_op {
                                base + (lx*p + m)*box_ld + ly*p + t (base = PATCH_HDR word 4) and
                                carries no Dirichlet node; word 3 = mask of its non-empty slots.
                                Patches with word 3 == 0 use the tables.  0 = not a lattice */
+  int64_t separable;        /* 1: the G01 slab of every patch block is zero (axis-aligned elements),
+                               and kernel_variants 0 and 2 run the separable element operator
+                               y = D^T (G00 . D u) + (G11 . u D^T) D, which stages and reads only
+                               the G00 and G11 slabs.  G keeps its three-slab layout (the zero
+                               G01 slab is simply not read).  kernel_variant 1 ignores the
+                               field.  0 = the three-factor operator                          */
 } semk_op;
 
 /* number of doubles the `partials` scratch of an operator must hold
@@ -244,6 +250,14 @@ int64_t semk_resident_ctas_variant(int kernel_variant, int n1, int elems_per_pat
 int64_t semk_patch_smem_bytes(int n1, int elems_per_patch, int64_t g_patch_stride,
                               int64_t pn_patch_stride, int64_t eloc_patch_stride,
                               int64_t inv_patch_stride);
+/* the two queries above for an operator with the given semk_op.separable (1: the separable
+ * kernel, which stages two of the three G slabs); separable = 0 is the plain query */
+int64_t semk_resident_ctas_sep(int kernel_variant, int separable, int n1, int elems_per_patch,
+                               int64_t g_patch_stride, int64_t pn_patch_stride,
+                               int64_t eloc_patch_stride, int64_t inv_patch_stride);
+int64_t semk_patch_smem_bytes_sep(int separable, int n1, int elems_per_patch,
+                                  int64_t g_patch_stride, int64_t pn_patch_stride,
+                                  int64_t eloc_patch_stride, int64_t inv_patch_stride);
 
 /* ------------------------------------------------------------------------
  * K1: geometric factors.  Replaces, per element, Mapping._compute_x_phys /

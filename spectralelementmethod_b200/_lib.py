@@ -66,6 +66,7 @@ class semk_op(C.Structure):
         ("partials", C.c_void_p), ("D_host", C.c_void_p), ("dirichlet", C.c_void_p),
         ("kernel_variant", C.c_int64),
         ("box_ld", C.c_int64),
+        ("separable", C.c_int64),
     ]
 
 
@@ -165,6 +166,8 @@ SIGNATURES = {
     "semk_patch_smem_bytes": (_L, [_I, _I, _L, _L, _L, _L]),
     "semk_resident_ctas": (_L, [_I, _I, _L, _L, _L, _L]),
     "semk_resident_ctas_variant": (_L, [_I, _I, _I, _L, _L, _L, _L]),
+    "semk_resident_ctas_sep": (_L, [_I, _I, _I, _I, _L, _L, _L, _L]),
+    "semk_patch_smem_bytes_sep": (_L, [_I, _I, _I, _L, _L, _L, _L]),
     "semk_geom_factors_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _P, _P, _L, _I, _P, _P, _P,
                                    _P, _P, _P, _P]),
     "semk_field_grad_f64": (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _I, _P,

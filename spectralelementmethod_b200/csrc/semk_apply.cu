@@ -287,20 +287,20 @@ inline bool pe_supported(int pe) { return pe == 4 || pe == 8 || pe == 16 || pe =
 // small elements amortise the per-patch barriers and tables better over a larger patch and
 // have a smaller share of interface nodes.
 constexpr int kBigPatchMaxN1 = 7;
-template <int NV, int MODE, bool OK = (NV <= kBigPatchMaxN1)>
+template <int NV, int MODE, bool SEP = false, bool OK = (NV <= kBigPatchMaxN1)>
 struct BigPatch {
   static int run(const semk_op &op, const DMatEO &dm, const double *u, const double *loc,
                  double *y, int flags, double fill, double *partials, cudaStream_t st,
                  int *grid_out, int64_t pb, int64_t pe) {
-    return PatchLaunch<32, MODE>::template run<NV>(op, dm, u, loc, y, flags, fill, partials, st,
-                                                   grid_out, pb, pe);
+    return PatchLaunch<32, MODE, false, SEP>::template run<NV>(op, dm, u, loc, y, flags, fill,
+                                                               partials, st, grid_out, pb, pe);
   }
   static int occupancy(size_t smem, int *per_sm, int *sms) {
-    return PatchLaunch<32, MODE>::template occupancy<NV>(smem, per_sm, sms);
+    return PatchLaunch<32, MODE, false, SEP>::template occupancy<NV>(smem, per_sm, sms);
   }
 };
-template <int NV, int MODE>
-struct BigPatch<NV, MODE, false> {
+template <int NV, int MODE, bool SEP>
+struct BigPatch<NV, MODE, SEP, false> {
   static int run(const semk_op &, const DMatEO &, const double *, const double *, double *, int,
                  double, double *, cudaStream_t, int *, int64_t, int64_t) {
     semk_set_error("32-element patches are compiled for n1 <= 7 only");
@@ -312,6 +312,32 @@ struct BigPatch<NV, MODE, false> {
   }
 };
 
+template <int MODE, bool SEP>
+int launch_patch_table(const semk_op &op, const DMatEO &dm, const double *u, const double *loc,
+                       double *y, int flags, double fill, double *partials, cudaStream_t st,
+                       int *grid_out, int64_t pb, int64_t pe) {
+#define SEMK_CALL(NV)                                                                     \
+  do {                                                                                    \
+    int rc;                                                                               \
+    if (op.elems_per_patch == 32)                                                         \
+      rc = BigPatch<NV, MODE, SEP>::run(op, dm, u, loc, y, flags, fill, partials, st, grid_out, \
+                                        pb, pe);                                          \
+    else if (op.elems_per_patch == 16)                                                    \
+      rc = PatchLaunch<16, MODE, false, SEP>::template run<NV>(op, dm, u, loc, y, flags, fill, \
+                                                               partials, st, grid_out, pb, pe); \
+    else if (op.elems_per_patch == 8)                                                     \
+      rc = PatchLaunch<8, MODE, false, SEP>::template run<NV>(op, dm, u, loc, y, flags, fill, \
+                                                              partials, st, grid_out, pb, pe); \
+    else                                                                                  \
+      rc = PatchLaunch<4, MODE, false, SEP>::template run<NV>(op, dm, u, loc, y, flags, fill, \
+                                                              partials, st, grid_out, pb, pe); \
+    if (rc != SEMK_OK) return rc;                                                         \
+  } while (0)
+  SEMK_DISPATCH_N1(op.n1, SEMK_CALL)
+#undef SEMK_CALL
+  return SEMK_OK;
+}
+
 template <int MODE>
 int launch_patch(const semk_op &op, const DMatEO &dm, const double *u, const double *loc,
                  double *y, int flags, double fill, double *partials, cudaStream_t st,
@@ -321,25 +347,13 @@ int launch_patch(const semk_op &op, const DMatEO &dm, const double *u, const dou
     return semk_ho_launch(op, u, y, flags, partials, st, grid_out, pb, pe);
   if (MODE == MODE_APPLY && op.kernel_variant == 2)
     return semk_box_launch(op, &dm, u, y, flags, partials, st, grid_out, pb, pe);
-#define SEMK_CALL(NV)                                                                     \
-  do {                                                                                    \
-    int rc;                                                                               \
-    if (op.elems_per_patch == 32)                                                         \
-      rc = BigPatch<NV, MODE>::run(op, dm, u, loc, y, flags, fill, partials, st, grid_out, pb, pe); \
-    else if (op.elems_per_patch == 16)                                                    \
-      rc = PatchLaunch<16, MODE>::template run<NV>(op, dm, u, loc, y, flags, fill, partials, st, \
-                                                   grid_out, pb, pe); \
-    else if (op.elems_per_patch == 8)                                                     \
-      rc = PatchLaunch<8, MODE>::template run<NV>(op, dm, u, loc, y, flags, fill, partials, st,   \
-                                                  grid_out, pb, pe);  \
-    else                                                                                  \
-      rc = PatchLaunch<4, MODE>::template run<NV>(op, dm, u, loc, y, flags, fill, partials, st,   \
-                                                  grid_out, pb, pe);  \
-    if (rc != SEMK_OK) return rc;                                                         \
-  } while (0)
-  SEMK_DISPATCH_N1(op.n1, SEMK_CALL)
-#undef SEMK_CALL
-  return SEMK_OK;
+  if constexpr (MODE == MODE_APPLY) {
+    if (op.separable)
+      return launch_patch_table<MODE, true>(op, dm, u, loc, y, flags, fill, partials, st,
+                                            grid_out, pb, pe);
+  }
+  return launch_patch_table<MODE, false>(op, dm, u, loc, y, flags, fill, partials, st, grid_out,
+                                         pb, pe);
 }
 
 int check_op(const semk_op *op, const char *who) {
@@ -384,28 +398,24 @@ extern "C" int64_t semk_partials_len(int64_t n_patch, int64_t n_shared) {
   return n_patch + n_shared / (2 * kChunkWarps) + kSharedBlocks + 16;
 }
 
-extern "C" int64_t semk_resident_ctas(int n1, int elems_per_patch, int64_t g_patch_stride,
-                                      int64_t pn_patch_stride, int64_t eloc_patch_stride,
-                                      int64_t inv_patch_stride) {
-  if (!pe_supported(elems_per_patch)) return -1;
-  const size_t smem = patch_smem_layout(n1, elems_per_patch, MODE_APPLY, g_patch_stride,
-                                        pn_patch_stride, eloc_patch_stride, inv_patch_stride)
-                          .total;
-  if (smem > 227 * 1024) return -1;
+namespace {
+
+template <bool SEP>
+int64_t resident_ctas_table(int n1, int elems_per_patch, size_t smem) {
   int per_sm = 0, sms = 0;
   auto run = [&]() -> int {
-#define SEMK_CALL(NV)                                                                  \
-  do {                                                                                 \
-    int rc;                                                                            \
-    if (elems_per_patch == 32)                                                         \
-      rc = BigPatch<NV, MODE_APPLY>::occupancy(smem, &per_sm, &sms);                   \
-    else if (elems_per_patch == 16)                                                    \
-      rc = PatchLaunch<16, MODE_APPLY>::template occupancy<NV>(smem, &per_sm, &sms);   \
-    else if (elems_per_patch == 8)                                                     \
-      rc = PatchLaunch<8, MODE_APPLY>::template occupancy<NV>(smem, &per_sm, &sms);    \
-    else                                                                               \
-      rc = PatchLaunch<4, MODE_APPLY>::template occupancy<NV>(smem, &per_sm, &sms);    \
-    if (rc != SEMK_OK) return rc;                                                      \
+#define SEMK_CALL(NV)                                                                           \
+  do {                                                                                          \
+    int rc;                                                                                     \
+    if (elems_per_patch == 32)                                                                  \
+      rc = BigPatch<NV, MODE_APPLY, SEP>::occupancy(smem, &per_sm, &sms);                       \
+    else if (elems_per_patch == 16)                                                             \
+      rc = PatchLaunch<16, MODE_APPLY, false, SEP>::template occupancy<NV>(smem, &per_sm, &sms); \
+    else if (elems_per_patch == 8)                                                              \
+      rc = PatchLaunch<8, MODE_APPLY, false, SEP>::template occupancy<NV>(smem, &per_sm, &sms);  \
+    else                                                                                        \
+      rc = PatchLaunch<4, MODE_APPLY, false, SEP>::template occupancy<NV>(smem, &per_sm, &sms);  \
+    if (rc != SEMK_OK) return rc;                                                               \
   } while (0)
     SEMK_DISPATCH_N1(n1, SEMK_CALL)
 #undef SEMK_CALL
@@ -415,31 +425,59 @@ extern "C" int64_t semk_resident_ctas(int n1, int elems_per_patch, int64_t g_pat
   return (int64_t)per_sm * sms;
 }
 
-extern "C" int64_t semk_resident_ctas_variant(int kernel_variant, int n1, int elems_per_patch,
-                                              int64_t g_patch_stride, int64_t pn_patch_stride,
-                                              int64_t eloc_patch_stride,
-                                              int64_t inv_patch_stride) {
-  if (kernel_variant == 0)
-    return semk_resident_ctas(n1, elems_per_patch, g_patch_stride, pn_patch_stride,
-                              eloc_patch_stride, inv_patch_stride);
-  if ((kernel_variant != 1 && kernel_variant != 2) || !pe_supported(elems_per_patch) ||
-      (kernel_variant == 1 && elems_per_patch == 32))
-    return -1;
-  const size_t smem = patch_smem_layout(n1, elems_per_patch, MODE_APPLY, g_patch_stride,
-                                        pn_patch_stride, eloc_patch_stride, inv_patch_stride)
-                          .total;
-  if (smem > 227 * 1024) return -1;
-  if (kernel_variant == 2) return semk_box_resident(n1, elems_per_patch, smem);
-  return semk_ho_resident(n1, elems_per_patch, smem);
+}  // namespace
+
+extern "C" int64_t semk_patch_smem_bytes_sep(int separable, int n1, int elems_per_patch,
+                                             int64_t g_patch_stride, int64_t pn_patch_stride,
+                                             int64_t eloc_patch_stride,
+                                             int64_t inv_patch_stride) {
+  return (int64_t)patch_smem_layout(n1, elems_per_patch, MODE_APPLY, g_patch_stride,
+                                    pn_patch_stride, eloc_patch_stride, inv_patch_stride,
+                                    separable != 0)
+      .total;
 }
 
 extern "C" int64_t semk_patch_smem_bytes(int n1, int elems_per_patch, int64_t g_patch_stride,
                                          int64_t pn_patch_stride, int64_t eloc_patch_stride,
                                          int64_t inv_patch_stride) {
-  return (int64_t)patch_smem_layout(n1, elems_per_patch, MODE_APPLY, g_patch_stride,
-                                    pn_patch_stride, eloc_patch_stride, inv_patch_stride)
-      .total;
+  return semk_patch_smem_bytes_sep(0, n1, elems_per_patch, g_patch_stride, pn_patch_stride,
+                                   eloc_patch_stride, inv_patch_stride);
 }
+
+// kernel_variant 1 has no separable instantiation: it reports its own (three-factor) footprint
+extern "C" int64_t semk_resident_ctas_sep(int kernel_variant, int separable, int n1,
+                                          int elems_per_patch, int64_t g_patch_stride,
+                                          int64_t pn_patch_stride, int64_t eloc_patch_stride,
+                                          int64_t inv_patch_stride) {
+  if ((kernel_variant != 0 && kernel_variant != 1 && kernel_variant != 2) ||
+      !pe_supported(elems_per_patch) || (kernel_variant == 1 && elems_per_patch == 32))
+    return -1;
+  const bool sep = separable != 0 && kernel_variant != 1;
+  const int64_t smem = semk_patch_smem_bytes_sep(sep, n1, elems_per_patch, g_patch_stride,
+                                                 pn_patch_stride, eloc_patch_stride,
+                                                 inv_patch_stride);
+  if (smem > 227 * 1024) return -1;
+  if (kernel_variant == 1) return semk_ho_resident(n1, elems_per_patch, (size_t)smem);
+  if (kernel_variant == 2) return semk_box_resident(n1, elems_per_patch, sep, (size_t)smem);
+  return sep ? resident_ctas_table<true>(n1, elems_per_patch, (size_t)smem)
+             : resident_ctas_table<false>(n1, elems_per_patch, (size_t)smem);
+}
+
+extern "C" int64_t semk_resident_ctas(int n1, int elems_per_patch, int64_t g_patch_stride,
+                                      int64_t pn_patch_stride, int64_t eloc_patch_stride,
+                                      int64_t inv_patch_stride) {
+  return semk_resident_ctas_sep(0, 0, n1, elems_per_patch, g_patch_stride, pn_patch_stride,
+                                eloc_patch_stride, inv_patch_stride);
+}
+
+extern "C" int64_t semk_resident_ctas_variant(int kernel_variant, int n1, int elems_per_patch,
+                                              int64_t g_patch_stride, int64_t pn_patch_stride,
+                                              int64_t eloc_patch_stride,
+                                              int64_t inv_patch_stride) {
+  return semk_resident_ctas_sep(kernel_variant, 0, n1, elems_per_patch, g_patch_stride,
+                                pn_patch_stride, eloc_patch_stride, inv_patch_stride);
+}
+
 
 extern "C" int semk_poisson_apply_f64(const semk_op *op, const double *u, double *y, int flags,
                                       double *dot_out, void *stream) {

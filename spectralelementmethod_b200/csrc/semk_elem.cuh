@@ -160,7 +160,8 @@ enum { MODE_APPLY = 0, MODE_ASSEMBLE = 1 };
 
 // Shared-memory carve-up of the persistent patch kernel (offsets multiples of
 // 16 B): one G buffer, two stages of {node block, index block}, one copy of
-// the working arrays.
+// the working arrays.  `sep`: the separable kernel stages only the G00 and G11 slabs
+// (2 NN PE doubles) instead of the whole patch block.
 struct PatchSmem {
   size_t hdr, gs, stage0, stage_bytes, pn_off, el_off;  // per stage: node block | index block
   size_t inv, ua, bs, red, total;
@@ -169,14 +170,16 @@ __host__ __device__ inline PatchSmem patch_smem_layout(int N, int PE, int mode,
                                                        int64_t g_patch_stride,
                                                        int64_t pn_patch_stride,
                                                        int64_t eloc_patch_stride,
-                                                       int64_t inv_patch_stride) {
+                                                       int64_t inv_patch_stride,
+                                                       bool sep = false) {
   PatchSmem L;
   const size_t scratch = (size_t)N * scratch_row_stride(N, PE);
   size_t o = 32;  // four mbarriers: tables[2], G, inverse table
   L.hdr = o;      // two 32-byte patch headers (ring)
   o += 64;
   L.gs = o;
-  o += (mode == MODE_APPLY) ? sizeof(double) * (size_t)g_patch_stride : 0;
+  const size_t g_doubles = sep ? 2 * (size_t)N * N * PE : (size_t)g_patch_stride;
+  o += (mode == MODE_APPLY) ? sizeof(double) * g_doubles : 0;
   L.stage0 = o;
   L.pn_off = 0;
   size_t st = 4 * (size_t)pn_patch_stride;
@@ -207,7 +210,7 @@ int semk_ho_launch(const semk_op &op, const double *u, double *y, int flags, dou
                    cudaStream_t st, int *grid_out, int64_t pb, int64_t pe);
 int64_t semk_ho_resident(int n1, int elems_per_patch, size_t smem);
 // semk_box.cu: the BOX instantiations of the patch kernel (regular structured numberings);
-// dm_eo points at the caller's DMatEO
+// dm_eo points at the caller's DMatEO; op.separable picks the separable instantiation
 int semk_box_launch(const semk_op &op, const void *dm_eo, const double *u, double *y, int flags,
                     double *partials, cudaStream_t st, int *grid_out, int64_t pb, int64_t pe);
-int64_t semk_box_resident(int n1, int elems_per_patch, size_t smem);
+int64_t semk_box_resident(int n1, int elems_per_patch, bool sep, size_t smem);

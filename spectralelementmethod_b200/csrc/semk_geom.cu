@@ -62,7 +62,15 @@ __device__ __forceinline__ NodeGeom node_geometry(const uint32_t *__restrict__ r
     sB[0][k] = t0;
     sB[1][k] = t1;
   }
-  __syncthreads();
+  // Axis-aligned element: x depends on m only and y on n only (or, rotated by 90 degrees,
+  // x on n and y on m).  Then J01 = J10 = 0 (J00 = J11 = 0) in exact arithmetic -- E^{-1}
+  // reproduces constants and D annihilates them -- and the roundoff J = D x would leave
+  // there is dropped, so that G01 comes out as an exact zero (the separable apply).  The
+  // dropped products lie far below an ulp of det, invJ's other entries, G00 and G11.
+  const bool x_m = !on || (sA[0][k] == sA[0][m * N] && sA[1][k] == sA[1][n]);
+  const bool x_n = !on || (sA[0][k] == sA[0][n] && sA[1][k] == sA[1][m * N]);
+  const bool axis_mn = __syncthreads_and(x_m) != 0;
+  const bool axis_nm = !axis_mn && __syncthreads_and(x_n) != 0;  // (uniform branch)
   r.xg = 0.0;
   r.yg = 0.0;
   if (on) {
@@ -87,6 +95,8 @@ __device__ __forceinline__ NodeGeom node_geometry(const uint32_t *__restrict__ r
       j01 = fma(d1, sA[0][m * N + q], j01);
       j11 = fma(d1, sA[1][m * N + q], j11);
     }
+    if (axis_mn) j01 = j10 = 0.0;
+    if (axis_nm) j00 = j11 = 0.0;
     const double det = __dsub_rn(__dmul_rn(j00, j11), __dmul_rn(j01, j10));
     if (!(det > 0.0)) atomicExch(bad_flag, 1);
     const double rdet = __drcp_rn(det);

@@ -80,6 +80,68 @@ __device__ __forceinline__ void local_poisson(const DM &dm, int le, int t, bool 
   }
 }
 
+// The separable element operator of an axis-aligned element (G01 == 0):
+//   y = D^T (G00 . D u)  +  (G11 . u D^T) D  =  y0 + y1.
+// The column-owning thread tidp = le*N + t forms y0 of its column in registers; thread
+// `tid` also owns row t' = tid / PE of slot le' = tid % PE and forms y1 of that row in
+// registers.  Only u crosses from the column to the row layout (scratch A) and only y1
+// crosses back (scratch B): two shared-memory round trips instead of four, two barriers
+// instead of four.  Every product and sum is the one local_poisson forms when its G01
+// entries are +-0, so the two routines give the same bits on the same G: there w0 =
+// fl(G00 ur + G01 us) = fl(G00 ur), here the product is rounded on its own (__dmul_rn, so
+// that the compiler cannot fuse it into the even-odd sums of mat_Dt as an FMA).
+//   g0: this thread's column base in the G00 slab, factor m at g0[m * g_row];
+//   g1: the G11 slab; row thread tid reads node (t', n) of slot le' at g1[tid * N + n]
+//       (with N odd, consecutive threads hit distinct banks).
+//   row_active: slot le' of row thread tid holds an element (false for tid >= N * PE).
+// On return ycol = y0 + y1 = fl(y0 + y1) as in local_poisson; scratch B still holds y1 at
+// node positions m*RS + tidp, which the caller may overwrite in place (own entries).
+// Contains two __syncthreads(); every thread of the CTA must call it.
+template <int N, int PE, int RS, class DM, class Hook = NoHook, class Hook0 = NoHook>
+__device__ __forceinline__ void local_poisson_sep(const DM &dm, int le, int t, int tid,
+                                                  bool active, bool row_active,
+                                                  const double (&ucol)[N], double (&ycol)[N],
+                                                  double *__restrict__ A, double *__restrict__ B,
+                                                  const double *__restrict__ g0, int g_row,
+                                                  const double *__restrict__ g1,
+                                                  uint64_t *g_ready, uint32_t g_parity = 0,
+                                                  Hook g_consumed = Hook(),
+                                                  Hook0 after_first_barrier = Hook0()) {
+  const int tidp = le * N + t;
+  if (active) {
+#pragma unroll
+    for (int m = 0; m < N; ++m) A[m * RS + tidp] = ucol[m];
+  }
+  __syncthreads();
+  after_first_barrier();  // every thread has left the previous patch's write-out
+  if (g_ready) semk_mbar_wait(g_ready, g_parity);
+  if (row_active) {
+    const int ler = tid % PE, tr = tid / PE;
+    double ur[N], w[N];
+#pragma unroll
+    for (int s = 0; s < N; ++s) ur[s] = A[tr * RS + ler * N + s];  // row t' of u
+    mat_D<N>(dm, ur, w);  // us[t'][n] = sum_s D[n][s] u[t'][s]
+#pragma unroll
+    for (int n = 0; n < N; ++n) w[n] = __dmul_rn(g1[tid * N + n], w[n]);  // w1[t'][n]
+    mat_Dt<N>(dm, w, ur);  // y1[t'][q] = sum_n w1[t'][n] D[n][q]
+#pragma unroll
+    for (int q = 0; q < N; ++q) B[tr * RS + ler * N + q] = ur[q];
+  }
+  if (active) {
+    double w[N];
+    mat_D<N>(dm, ucol, w);  // ur[m][t] = sum_r D[m][r] u[r][t]
+#pragma unroll
+    for (int m = 0; m < N; ++m) w[m] = __dmul_rn(g0[m * g_row], w[m]);  // w0[m][t]
+    mat_Dt<N>(dm, w, ycol);  // y0[p][t] = sum_m D[m][p] w0[m][t]
+  }
+  __syncthreads();
+  g_consumed();  // every thread has read its G entries: the G buffer may be refilled
+  if (active) {
+#pragma unroll
+    for (int m = 0; m < N; ++m) ycol[m] += B[m * RS + tidp];
+  }
+}
+
 template <int N, int PE>
 struct PatchCfg {
   static constexpr int kThreads = ((N * PE + 31) / 32) * 32;
@@ -88,12 +150,13 @@ struct PatchCfg {
 
 // Resident CTAs per SM the kernel is compiled for (register budget): what the
 // shared-memory footprint of the standard tiles (2x8, 1x8, 1x4 elements) allows.
-__host__ __device__ constexpr int patch_min_blocks(int N, int PE) {
+// `g_slabs`: G slabs staged per patch (3, or 2 for the separable kernel).
+__host__ __device__ constexpr int patch_min_blocks(int N, int PE, int g_slabs = 3) {
   const int bx = PE == 32 ? 4 : (PE == 16 ? 2 : 1), by = PE == 4 ? 4 : 8, p = N - 1;
   const long long mpn = (long long)(bx * p + 1) * (by * p + 1);
   const long long mpn4 = (mpn + 3) & ~3LL;
   const long long nn = (long long)N * N;
-  const long long g = 8 * ((3 * nn * PE + 1) & ~1LL);
+  const long long g = 8 * ((g_slabs * nn * PE + 1) & ~1LL);
   const long long tab = 2 * ((4 * mpn4 + 2 * ((nn * PE + 7) & ~7LL) + 15) & ~15LL) + 64;
   const long long scr = 8LL * N * scratch_row_stride(N, PE);
   const long long ua = scr;
@@ -135,8 +198,14 @@ constexpr int kGatherBatch = 8;
 // the tile-interior nodes (the index arithmetic costs more issue slots than the two table
 // look-ups per node it saves: 0.775 ms); not copying the (then unused) index block of a box
 // patch into shared memory (0.694 vs 0.659 ms -- kept copying it).
-template <int N, int PE, int MODE, bool BOX = false>
-__global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N, PE))
+//
+// SEP (apply only; semk_op.separable): the G01 slab of every patch is zero.  The TMA stages
+// only the G00 and G11 slabs and the element operator is local_poisson_sep: three barriers
+// per patch instead of five, seven shared-memory passes of N doubles per thread instead of
+// twelve, two thirds of the G bytes.  Same results, bit for bit, as the three-factor kernel
+// on the same G (DESIGN.md section 3).
+template <int N, int PE, int MODE, bool BOX = false, bool SEP = false>
+__global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N, PE, SEP ? 2 : 3))
     patch_kernel(semk_op op, DMatEO dm, const double *__restrict__ u,
                  const double *__restrict__ loc, double *__restrict__ y, int flags,
                  double fill_dirichlet, double *__restrict__ dot_partials, int64_t patch_begin,
@@ -145,9 +214,10 @@ __global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N,
   constexpr int NP = N * PE;
   constexpr int kThreads = PatchCfg<N, PE>::kThreads;
   constexpr int RS = PatchCfg<N, PE>::kRS;
+  static_assert(!SEP || MODE == MODE_APPLY, "the separable operator is an apply");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const PatchSmem L = patch_smem_layout(N, PE, MODE, op.g_patch_stride, op.pn_patch_stride,
-                                        op.eloc_patch_stride, op.inv_patch_stride);
+                                        op.eloc_patch_stride, op.inv_patch_stride, SEP);
   uint64_t *mbar = reinterpret_cast<uint64_t *>(smem_raw);  // [0..1]: tables, [2]: G, [3]: inv
   double *Gs = reinterpret_cast<double *>(smem_raw + L.gs);
   const uint16_t *inv_s = reinterpret_cast<const uint16_t *>(smem_raw + L.inv);
@@ -180,15 +250,24 @@ __global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N,
   };
   // The inverse table is single-buffered: patch i's table is fetched right after the
   // first barrier of patch i (when every thread has left patch i-1's write-out, its last
-  // reader) and is first needed five barriers later, in patch i's own write-out.
+  // reader) and is first needed five barriers later (three with SEP), in patch i's own
+  // write-out.
   auto issue_inv = [&](uint32_t block) {  // one thread
     semk_mbar_expect_tx(&mbar[3], inv_bytes);
     semk_bulk_g2s(smem_raw + L.inv, op.inv + (int64_t)block * op.inv_patch_stride, inv_bytes,
                   &mbar[3]);
   };
   auto issue_g = [&](int64_t patch) {  // one thread
-    semk_mbar_expect_tx(&mbar[2], g_bytes);
-    semk_bulk_g2s(Gs, op.G + patch * op.g_patch_stride, g_bytes, &mbar[2]);
+    const double *src = op.G + patch * op.g_patch_stride;
+    if (SEP) {  // slabs 0 (G00) and 2 (G11); the zero G01 slab stays in global memory
+      constexpr uint32_t slab = (uint32_t)(NN * PE * sizeof(double));
+      semk_mbar_expect_tx(&mbar[2], 2 * slab);
+      semk_bulk_g2s(Gs, src, slab, &mbar[2]);
+      semk_bulk_g2s(Gs + NN * PE, src + 2 * NN * PE, slab, &mbar[2]);
+    } else {
+      semk_mbar_expect_tx(&mbar[2], g_bytes);
+      semk_bulk_g2s(Gs, src, g_bytes, &mbar[2]);
+    }
   };
 
   // this CTA's patch sequence: round-robin over the grid, so that at any time the
@@ -308,8 +387,15 @@ __global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N,
           issue_tables(hn[5], hn[6], s ^ 1, after < p_end ? after : -1, s);
         }
       };
-      local_poisson<N, RS>(dm, le, t, active, ucol, ycol, As, Bs, Gs + tid, NP, &mbar[2],
-                           (uint32_t)(it & 1), refill_g, refill_tables);
+      if (SEP) {
+        const bool row_active = tid < NP && slot0 + tid % PE < op.n_elem;
+        local_poisson_sep<N, PE, RS>(dm, le, t, tid, active, row_active, ucol, ycol, As, Bs,
+                                     Gs + tid, NP, Gs + NN * PE, &mbar[2], (uint32_t)(it & 1),
+                                     refill_g, refill_tables);
+      } else {
+        local_poisson<N, RS>(dm, le, t, active, ucol, ycol, As, Bs, Gs + tid, NP, &mbar[2],
+                             (uint32_t)(it & 1), refill_g, refill_tables);
+      }
       // u . y taken element by element: sum_e (Q_e u) . y_e = u . (sum_e Q_e^T y_e), so the
       // write-out never looks at u again.  Dirichlet rows are left out here (under MASK_IN
       // their entries of u are zero anyway) and come back as identity rows below.
@@ -341,7 +427,8 @@ __global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N,
     }
 
     // ---- assemble by GATHERING (no atomics, no colour phases): every thread leaves its
-    // column of element results in scratch B (its own entries, the ones it just read),
+    // column of element results in scratch B (its own entries, the ones it just read; the
+    // separable operator's y1 is overwritten in place),
     // then each patch node sums its <= inv_width contributions in a fixed order (ascending
     // element slot) straight from B and is stored: private nodes -> y, shared nodes ->
     // interface slots ------------------------------------------------------------------
@@ -423,14 +510,14 @@ __global__ void __launch_bounds__(PatchCfg<N, PE>::kThreads, patch_min_blocks(N,
   }
 }
 
-template <int PE, int MODE, bool BOX = false>
+template <int PE, int MODE, bool BOX = false, bool SEP = false>
 struct PatchLaunch {
   // CTAs per SM of this instantiation for the given dynamic shared memory
   template <int N>
   static int occupancy(size_t smem, int *per_sm, int *sms) {
     static size_t configured = 0;  // per instantiation; one device per process
     static int cached_per_sm = 0, cached_sms = 0;
-    auto kern = patch_kernel<N, PE, MODE, BOX>;
+    auto kern = patch_kernel<N, PE, MODE, BOX, SEP>;
     if (smem > configured || cached_per_sm == 0) {
       SEMK_CUDA_CHECK(
           cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -451,7 +538,7 @@ struct PatchLaunch {
                  double *y, int flags, double fill, double *partials, cudaStream_t st,
                  int *grid_out, int64_t pb, int64_t pe) {
     const size_t smem = patch_smem_layout(N, PE, MODE, op.g_patch_stride, op.pn_patch_stride,
-                                          op.eloc_patch_stride, op.inv_patch_stride)
+                                          op.eloc_patch_stride, op.inv_patch_stride, SEP)
                             .total;
     if (smem > 227 * 1024) {
       semk_set_error("patch kernel: shared memory request exceeds 227 KB");
@@ -473,7 +560,7 @@ struct PatchLaunch {
     const unsigned grid = (unsigned)(np < want ? np : want);
     if (grid_out) *grid_out = (int)grid;
     if (grid == 0) return SEMK_OK;
-    patch_kernel<N, PE, MODE, BOX><<<grid, PatchCfg<N, PE>::kThreads, smem, st>>>(
+    patch_kernel<N, PE, MODE, BOX, SEP><<<grid, PatchCfg<N, PE>::kThreads, smem, st>>>(
         op, dm, u, loc, y, flags, fill, partials, pb, pe);
     SEMK_LAUNCH_CHECK("patch_kernel");
     return SEMK_OK;

@@ -375,16 +375,6 @@ class PoissonOperator(_PoissonBase):
                 "elems_per_patch or a more local elem_order" % (pe, _lib.last_error()))
         self.plan_scalars = sc
         self.resident_ctas = actual
-        # CTA b of the persistent kernel runs patches b, b + grid, ...; a grid that is a
-        # multiple of the patches per tile column would pin every CTA to one tile row (a
-        # measured 10 % slowdown): step off the resonance by one CTA
-        self.max_ctas = 0
-        shape = getattr(mesh, "_structured_shape", None)
-        if shape is not None and not user_order:
-            by = (tile if tile is not None else _TILES[pe])[1]
-            per_column = -(-shape[1] // by)
-            if per_column > 1 and actual > 1 and (actual % per_column == 0 or per_column % actual == 0):
-                self.max_ctas = actual - 1
         smem = patch_smem_bytes(n1, pe, sc[_lib.PS_MAX_PATCH_NODES], sc[_lib.PS_PN_STRIDE],
                                 sc[_lib.PS_INV_STRIDE])
         self.smem_bytes = smem
@@ -428,6 +418,34 @@ class PoissonOperator(_PoissonBase):
                 self.resident_ctas = int(self._lib.semk_resident_ctas_variant(
                     0, n1, pe, g_patch_stride_of(n1, pe), int(sc[_lib.PS_PN_STRIDE]),
                     int(sc[_lib.PS_EL_STRIDE]), int(sc[_lib.PS_INV_STRIDE])))
+        # separable element operator (semk_op.separable): every element is axis-aligned, so
+        # K1 wrote the G01 slab as exact zeros (weights included) -- one device reduction.
+        # The pair mapping (kernel_variant 1) has no separable form and keeps three factors.
+        nnp = NN * pe
+        self.separable = (self.kernel_variant != 1 and self.n_patch > 0
+                          and not bool(self.G[:, nnp:2 * nnp].any()))
+        if self.separable:
+            self.kernel_name = self.kernel_name[:-1] + ",SEP>"
+            self.resident_ctas = int(self._lib.semk_resident_ctas_sep(
+                self.kernel_variant, 1, n1, pe, g_patch_stride_of(n1, pe),
+                int(sc[_lib.PS_PN_STRIDE]), int(sc[_lib.PS_EL_STRIDE]),
+                int(sc[_lib.PS_INV_STRIDE])))
+            if self.resident_ctas <= 0:
+                raise NotImplementedError("separable patch kernel: %s" % _lib.last_error())
+            self.smem_bytes = int(self._lib.semk_patch_smem_bytes_sep(
+                1, n1, pe, g_patch_stride_of(n1, pe), int(sc[_lib.PS_PN_STRIDE]),
+                eloc_patch_stride_of(n1, pe), int(sc[_lib.PS_INV_STRIDE])))
+        # CTA b of the persistent kernel runs patches b, b + grid, ...; a grid that is a
+        # multiple of the patches per tile column would pin every CTA to one tile row (a
+        # measured 10 % slowdown): step off the resonance by one CTA
+        actual = self.resident_ctas
+        self.max_ctas = 0
+        shape = getattr(mesh, "_structured_shape", None)
+        if shape is not None and not user_order:
+            by = (tile if tile is not None else _TILES[pe])[1]
+            per_column = -(-shape[1] // by)
+            if per_column > 1 and actual > 1 and (actual % per_column == 0 or per_column % actual == 0):
+                self.max_ctas = actual - 1
         if not keep_l2g:
             self.l2g_dev = None
 
@@ -465,6 +483,7 @@ class PoissonOperator(_PoissonBase):
         op.dirichlet = self.dirichlet_dev.data_ptr() if self.has_dirichlet else None
         op.kernel_variant = self.kernel_variant
         op.box_ld = self.box_ld
+        op.separable = int(self.separable)
         self._op = op
         self._masked_flags = (MASK_IN | MASK_OUT | DIRICHLET_IDENTITY) if self.has_dirichlet else 0
         self._dinv = None
@@ -542,9 +561,10 @@ class PoissonOperator(_PoissonBase):
 
     @property
     def algorithmic_bytes_per_apply(self):
-        """SURVEY.md 8(d): read u, write y, 3 geometric factors + one uint32
-        L2G entry per element-local node."""
-        return 16 * self.n_nodes + 28 * self.n_elem * self.n1 * self.n1
+        """SURVEY.md 8(d): read u, write y, 3 geometric factors (2 for a separable operator,
+        whose apply does not read G01) + one uint32 L2G entry per element-local node."""
+        per_node = 20 if self.separable else 28
+        return 16 * self.n_nodes + per_node * self.n_elem * self.n1 * self.n1
 
     # -- operator --------------------------------------------------------------------
     def apply(self, u, out=None, flags=None, dot_out=None):
