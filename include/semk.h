@@ -547,7 +547,9 @@ typedef struct semk_sc_op {
 #define SEMK_SC_STORE 8       /* also keep W = A_ii^{-1} A_ie (W_out), so that later back-
                                  substitutions are one streaming pass                       */
 
-/* One pass of the element kernel (one CTA per element).
+/* The element passes (one CTA per element): the factorisation outputs (SCHUR, STORE,
+ * STORE_INV) in one pass, then each load output (RHS, then BACKSOLVE) as the k = 1 case of
+ * semk_sc_element_block_f64 below.
  * slot_of_elem: device int64 [n_elem], engine slot holding element e's factors in G
  *   (inverse of SEMK_PA_ELEM_OF_SLOT), or NULL = identity; G / g_patch_stride /
  *   elems_per_patch as in semk_op (elems_per_patch = 1: plain [n_elem][3][NN] blocks).
@@ -559,7 +561,7 @@ typedef struct semk_sc_op {
  * RHS: g_loc [n_elem][n_ext_loc].  BACKSOLVE: u device [n_nodes], exterior entries
  *   read, interior entries written.
  * STORE: W_out device [n_elem][n_ext_loc][n_int] = (A_ii^{-1} A_ie)^T (12.5 KB per element at
- *   p = 8; 180 GB of HBM make it affordable).  c_out (optional, needs a load): device
+ *   p = 8; 180 GB of HBM make it affordable).  c_out (optional, RHS or BACKSOLVE mode): device
  *   [n_elem][n_int] = A_ii^{-1} f_i.  With both, _solve_interior_dofs (sem/discrete.py:513-524)
  *   becomes semk_sc_backsolve_stored_f64.
  * bad_flag: device int32, set to 1 when an interior block is not positive definite. */
@@ -583,13 +585,14 @@ int semk_sc_element_react_f64(int n1, int64_t n_elem, const int64_t *slot_of_ele
 /* Condensed load from the stored interior operators (W: SEMK_SC_STORE, Ainv: SEMK_SC_STORE_INV):
  * c = A_ii^{-1} f_i and g_loc = f_e - W^T f_i with f = f_scale * JxW * f_nodal[l2g] -- the RHS
  * mode of the element kernel (compute_local_sc_system, sem/discrete.py:438-476) without
- * refactorising the interior block. */
+ * refactorising the interior block; the k = 1 case of semk_sc_load_stored_block_f64. */
 int semk_sc_load_stored_f64(int n1, int64_t n_elem, const double *W, const double *Ainv,
                             const uint32_t *l2g, const int32_t *ext_loc, const double *JxW,
                             const double *f_nodal, double f_scale, double *g_loc, double *c_out,
                             void *stream);
 /* u_i = c - W u_e for every element (c NULL: zero load): exterior entries of u read,
- * interior entries written; W, c from semk_sc_element_f64. */
+ * interior entries written; W, c from semk_sc_element_f64.  The k = 1 case of
+ * semk_sc_backsolve_stored_block_f64. */
 int semk_sc_backsolve_stored_f64(int n1, int64_t n_elem, const double *W, const double *c,
                                  const uint32_t *l2g, const int32_t *ext_loc, double *u,
                                  void *stream);
@@ -604,10 +607,10 @@ int semk_sc_backsolve_stored_f64(int n1, int64_t n_elem, const double *W, const 
  *
  * semk_sc_element_block_f64: one CTA per element factorises A_ii once for all k columns.
  *   mode SEMK_SC_RHS: g_loc [k][ldg >= n_elem * 4p] = f_e - A_ei A_ii^{-1} f_i (the condensed
- *   load of compute_local_sc_system, sem/discrete.py:438-476), and, if c_out is not NULL,
- *   c_out [k][ldc >= n_elem * (p-1)^2] = A_ii^{-1} f_i.  Mode SEMK_SC_BACKSOLVE: U [k][ldu]
- *   nodal vectors, exterior entries read, interior entries written with
- *   u_i = A_ii^{-1} (f_i - A_ie u_e) (_solve_interior_dofs, sem/discrete.py:513-524).
+ *   load of compute_local_sc_system, sem/discrete.py:438-476).  Mode SEMK_SC_BACKSOLVE:
+ *   U [k][ldu] nodal vectors, exterior entries read, interior entries written with
+ *   u_i = A_ii^{-1} (f_i - A_ie u_e) (_solve_interior_dofs, sem/discrete.py:513-524).  In
+ *   either mode, if c_out is not NULL: c_out [k][ldc >= n_elem * (p-1)^2] = A_ii^{-1} f_i.
  *   G ... react as semk_sc_element_react_f64.
  * semk_sc_load_stored_block_f64: semk_sc_load_stored_f64 per column, A_ii^{-1} and W read once.
  * semk_sc_backsolve_stored_block_f64: semk_sc_backsolve_stored_f64 per column, W read once;

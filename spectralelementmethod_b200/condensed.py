@@ -175,8 +175,9 @@ class CondensedPoissonOperator(_PoissonBase):
         (n_nodes) or a callable alpha(x, y) on CUDA tensors."""
         self._store_interior = store_interior
         # store_interior_inverse: also keep A_ii^-1 of every element (19 KB at p = 8): the
-        # condensed load of ANY right-hand side then is a streaming pass (semk_sc_load_stored_f64)
-        # instead of a refactorisation per element -- for solvers that call rhs() many times
+        # condensed load of ANY right-hand side then is a streaming pass
+        # (semk_sc_load_stored_block_f64) instead of a refactorisation per element -- for
+        # solvers that call rhs() many times
         self._store_inverse = bool(store_interior_inverse)
         self._init_common(dof_mngr, dirichlet)
         self._init_geometry(geometric_factors, weight)
@@ -332,24 +333,16 @@ class CondensedPoissonOperator(_PoissonBase):
         self._dinv = None
 
     # -- element kernel ----------------------------------------------------------------
-    def _element_pass(self, mode, S=None, sdiag_loc=None, g_loc=None, u=None, f=1.0, W=None,
-                      c=None, Ainv=None):
-        """One launch of sc_element_kernel (csrc/semk_sc.cu)."""
-        f_nodal, f_scale = None, 1.0
-        if isinstance(f, torch.Tensor):
-            f_nodal = self._vec(f, "f", self.n_nodes)
-        elif np.ndim(f) == 0:
-            f_scale = float(f)
-        else:
-            f_nodal = self._vec(self.from_host(f), "f", self.n_nodes)
+    def _element_pass(self, mode, S=None, sdiag_loc=None, W=None, Ainv=None):
+        """One factorisation pass of sc_element_kernel (csrc/semk_sc.cu): modes SCHUR, STORE,
+        STORE_INV.  The loads run in _element_block."""
         self._bad.zero_()
         _lib.check(self._lib.semk_sc_element_react_f64(
             self.n1, self.n_elem, None, device.ptr(self.G), self.g_stride, 1,
-            device.ptr(self.tab.dev()[0]), device.ptr(self._t["ext_loc"]),
-            device.ptr(self.l2g_dev), device.ptr(self.JxW), device.ptr(f_nodal), f_scale,
-            int(mode), device.ptr(S), self.s_stride, device.ptr(sdiag_loc), device.ptr(g_loc),
-            device.ptr(u), device.ptr(W), device.ptr(c), device.ptr(getattr(self, "_react", None)),
-            device.ptr(Ainv), device.ptr(self._bad), device.stream_ptr()))
+            device.ptr(self.tab.dev()[0]), device.ptr(self._t["ext_loc"]), None, None, None, 1.0,
+            int(mode), device.ptr(S), self.s_stride, device.ptr(sdiag_loc), None, None,
+            device.ptr(W), None, device.ptr(self._react), device.ptr(Ainv), device.ptr(self._bad),
+            device.stream_ptr()))
         if int(self._bad.item()) != 0:
             raise AssertionError("an element-interior stiffness block is not positive definite")
 
@@ -400,30 +393,14 @@ class CondensedPoissonOperator(_PoissonBase):
 
     def rhs(self, f=1.0):
         """Condensed load vector: assembled ``f_e - A_ei A_ii^-1 f_i`` with the
-        element load ``JxW . f`` (examples/poisson.py:200; scalar or nodal f)."""
-        g_loc = torch.empty((self.n_elem, self.n_ext_loc), dtype=torch.float64, device=self.dev)
-        c, key = None, _load_key(f)
-        if (getattr(self, "_Ainv", None) is not None and self._W is not None and key is not None
-                and type(self) is CondensedPoissonOperator):
-            # stored interior operators: the load is a stream over W and A_ii^-1
-            f_nodal, f_scale = ((self._vec(f, "f", self.n_nodes), 1.0)
-                                if isinstance(f, torch.Tensor) else (None, float(f)))
-            c = torch.empty((self.n_elem, self.n_int_loc), dtype=torch.float64, device=self.dev)
-            _lib.check(self._lib.semk_sc_load_stored_f64(
-                self.n1, self.n_elem, device.ptr(self._W), device.ptr(self._Ainv),
-                device.ptr(self.l2g_dev), device.ptr(self._t["ext_loc"]), device.ptr(self.JxW),
-                device.ptr(f_nodal), f_scale, device.ptr(g_loc), device.ptr(c),
-                device.stream_ptr()))
-            self._c, self._c_key = c, key
-            return self.assemble(g_loc)
-        if getattr(self, "_W", None) is not None and key is not None:
-            # the interior solution of this load rides along: back-substitution of the same
-            # load later is a stream over W (backsolve)
-            c = torch.empty((self.n_elem, self.n_int_loc), dtype=torch.float64, device=self.dev)
-        self._element_pass(_lib.SC_RHS, g_loc=g_loc, f=f, c=c)
+        element load ``JxW . f`` (examples/poisson.py:200; scalar or nodal f).  With W kept,
+        the interior solution of a CUDA or scalar load rides along: back-substitution of the
+        same load later is a stream over W (backsolve)."""
+        cols, _ = self._block_loads([f])
+        (_, g_loc, c, _), = self._block_rhs(cols, None, keep_c=True)
         if c is not None:
-            self._c, self._c_key = c, key
-        return self.assemble(g_loc)
+            self._c, self._c_key = c[0], _load_key(f)
+        return self.assemble(g_loc[0])
 
     def _build_coarse(self):
         """Vertex coarse space of the two-level preconditioner (lazy): host tables
@@ -674,15 +651,12 @@ class CondensedPoissonOperator(_PoissonBase):
         self._vec(x_ext, "x_ext")
         u = (torch.empty(self.n_nodes, dtype=torch.float64, device=self.dev) if out is None
              else self._vec(out, "out", self.n_nodes))
-        u[:self.n_ext].copy_(x_ext)
-        if (getattr(self, "_W", None) is not None and self._c is not None
-                and self._c_key == _load_key(f)):
-            _lib.check(self._lib.semk_sc_backsolve_stored_f64(
-                self.n1, self.n_elem, device.ptr(self._W), device.ptr(self._c),
-                device.ptr(self.l2g_dev), device.ptr(self._t["ext_loc"]), device.ptr(u),
-                device.stream_ptr()))
-            return u
-        self._element_pass(_lib.SC_BACKSOLVE, u=u, f=f)
+        if self._W is not None and self._c is not None and self._c_key == _load_key(f):
+            self._block_backsolve(x_ext[None], [0], None, self._c, u[None])
+        else:
+            cols, _ = self._block_loads([f])
+            self._block_backsolve(x_ext[None], [0], self._chunk_load(cols, [0], None), None,
+                                  u[None])
         return u
 
     def solve(self, f=1.0, dirichlet_values=None, flux=None, **pcg_kwargs):
@@ -719,7 +693,10 @@ class CondensedPoissonOperator(_PoissonBase):
 
     def _block_chunks(self, k):
         """Column ranges of a block of k loads (block_chunks with this operator's cap, the
-        temporaries g_loc and c of one column and the free device memory)."""
+        temporaries g_loc and c of one column and the free device memory); one column without
+        asking the device (the single-load calls)."""
+        if k == 1:
+            return [(0, 1)]
         per_col = 8 * self.n_elem * (self.n_ext_loc + self.n_int_loc)
         return block_chunks(k, self._block_cap(), per_col, torch.cuda.mem_get_info(self.dev)[0])
 
@@ -765,6 +742,8 @@ class CondensedPoissonOperator(_PoissonBase):
         scales = (C.c_double * len(sub))(*[s for s, _, _ in sub])
         if not mask:
             return None, 0, 0, scales
+        if len(sub) == 1:
+            return sub[0][1], self.n_nodes, mask, scales
         if block is not None and idx == list(range(idx[0], idx[0] + len(idx))):
             return block[idx[0]:idx[0] + len(idx)], block.stride(0), mask, scales
         Fs = torch.empty((len(sub), self.n_nodes), dtype=torch.float64, device=self.dev)
@@ -793,8 +772,7 @@ class CondensedPoissonOperator(_PoissonBase):
         c [kc, E, (p-1)^2] = A_ii^-1 f_i or None, load descriptor).  ``keep_c``: compute c where
         the single path would cache it (W kept, cacheable load)."""
         f64 = dict(dtype=torch.float64, device=self.dev)
-        stored_load = (getattr(self, "_Ainv", None) is not None and self._W is not None
-                       and type(self) is CondensedPoissonOperator)
+        stored_load = self._Ainv is not None      # kept with W only
         for cacheable, group in self._block_groups(cols):
             for j0, j1 in self._block_chunks(len(group)):
                 idx = group[j0:j1]
@@ -978,8 +956,8 @@ class CondensedLocalSystems(CondensedPoissonOperator):
         self._l2g_hier = device.as_i32_bits(np.ascontiguousarray(l2g[:, hier]), self.dev)
         self._schur_pass()
 
-    def _element_pass(self, mode, S=None, sdiag_loc=None, g_loc=None, u=None, f=None, W=None,
-                      c=None, Ainv=None):
+    def _element_pass(self, mode, S=None, sdiag_loc=None, g_loc=None, u=None, W=None, Ainv=None):
+        """One launch of the element kernel on the local systems (W and Ainv are never kept)."""
         self._bad.zero_()
         _lib.check(self._lib.semk_sc_element_dense_f64(
             self.n1, self.n_elem, device.ptr(self._A), device.ptr(self._f),
@@ -991,10 +969,17 @@ class CondensedLocalSystems(CondensedPoissonOperator):
 
     def rhs(self, f=None):
         """Condensed load of the caller's local right-hand sides."""
-        return CondensedPoissonOperator.rhs(self, None)
+        g_loc = torch.empty((self.n_elem, self.n_ext_loc), dtype=torch.float64, device=self.dev)
+        self._element_pass(_lib.SC_RHS, g_loc=g_loc)
+        return self.assemble(g_loc)
 
     def backsolve(self, x_ext, f=None, out=None):
-        return CondensedPoissonOperator.backsolve(self, x_ext, None, out)
+        self._vec(x_ext, "x_ext")
+        u = (torch.empty(self.n_nodes, dtype=torch.float64, device=self.dev) if out is None
+             else self._vec(out, "out", self.n_nodes))
+        u[:self.n_ext].copy_(x_ext)
+        self._element_pass(_lib.SC_BACKSOLVE, u=u)
+        return u
 
     def solve(self, dirichlet_values=None, **pcg_kwargs):
         b = self.lift(self.rhs(), dirichlet_values)

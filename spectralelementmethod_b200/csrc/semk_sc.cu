@@ -10,11 +10,11 @@
 //   sc_element_kernel<N>  one CTA per element.  Rebuilds the 4-index local
 //       stiffness of examples/poisson.py:166-193 entry by entry from the
 //       geometric factors (closed form below), Cholesky-factorises the interior
-//       block in shared memory (A_ii = L L^T), Z = L^{-1} [A_ie | f_i], and
-//       writes  S_e = A_ee - Z^T Z (packed lower triangle),
-//               g_e = f_e - Z^T (L^{-1} f_i),
-//               u_i = L^{-T} (L^{-1} f_i - Z u_e)      (back-substitution).
-//       Set-up / once-per-solve work; the factorisation is recomputed instead
+//       block in shared memory (A_ii = L L^T), Z = L^{-1} A_ie, and writes
+//       S_e = A_ee - Z^T Z (packed lower triangle).  Set-up work.
+//   sc_element_block_kernel<N>  the same factorisation for up to 32 loads
+//       (f_i columns of Z): g_e = f_e - Z^T (L^{-1} f_i) or the back-substitution
+//       u_i = L^{-T} (L^{-1} f_i - Z u_e); once-per-solve work, recomputed instead
 //       of stored (19 KB per element at p = 8 against 4 KB for S_e).
 //   sc_matvec_kernel<N>   the condensed apply, HBM-bound: persistent CTAs stream the
 //       packed S_e blocks through a double-buffered TMA pipeline (evict-first),
@@ -60,26 +60,23 @@ struct ScElemArgs {
   int pe;
   const double *D;
   const int32_t *ext_loc;
-  const uint32_t *l2g;
-  const double *JxW;
-  const double *f_nodal;
-  double f_scale;
   int mode;
   double *S_out;
   int64_t s_stride;
   double *sdiag_loc;
-  double *g_loc;
-  double *u;
+  double *W_out;               // [n_elem][NE][NI] A_ii^{-1} A_ie, transposed (mode STORE), or nullptr
+  const double *react;         // [n_elem][NN] nodal reaction term added to the local diagonal, or nullptr
+  double *Ainv_out;            // [n_elem][NI][NI] A_ii^{-1} (mode STORE_INV), or nullptr
   int32_t *bad_flag;
   // dense mode (semk_sc_element_dense_f64): the caller's own local systems, hierarchical
-  // local order (exterior DOFs first), instead of the Poisson recipe on G
-  double *W_out;               // [n_elem][NE][NI] A_ii^{-1} A_ie, transposed (mode STORE), or nullptr
-  double *c_out;               // [n_elem][NI] A_ii^{-1} f_i (with the load), or nullptr
+  // local order (exterior DOFs first), instead of the Poisson recipe on G; the only mode
+  // whose loads (RHS, BACKSOLVE) this kernel takes -- the recipe's loads run in
+  // sc_element_block_kernel
+  double *g_loc;
+  double *u;
   const double *A_dense;       // [n_elem][NN][NN] or nullptr
   const double *f_dense;       // [n_elem][NN]
   const uint32_t *l2g_hier;    // [n_elem][NN] global ids in hierarchical local order
-  const double *react;         // [n_elem][NN] nodal reaction term added to the local diagonal, or nullptr
-  double *Ainv_out;            // [n_elem][NI][NI] A_ii^{-1} (mode STORE_INV), or nullptr
 };
 
 // ---- element work shared by sc_element_kernel and sc_element_block_kernel -----------------
@@ -197,7 +194,6 @@ template <int N>
 __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
   using C = ScCfg<N>;
   constexpr int NN = C::NN, NE = C::NE, NI = C::NI, NS = C::NS, LDI = C::LDI, LDZ = C::LDZ;
-  constexpr int M = N - 2;
   extern __shared__ __align__(128) double sc_smem[];
   double *sG = sc_smem;            // [3][N][N] geometric factors G00, G01, G11
   double *sD = sG + 3 * NN;        // [N][N]
@@ -213,7 +209,7 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
   int *sExt = reinterpret_cast<int *>(sX + NI * LDI);  // [NE] lexicographic index of exterior k
   int *sBad = sExt + NE;
   const int tid = threadIdx.x;
-  const bool need_f = (a.mode & (SEMK_SC_RHS | SEMK_SC_BACKSOLVE)) != 0;
+  const bool need_f = (a.mode & (SEMK_SC_RHS | SEMK_SC_BACKSOLVE)) != 0;  // dense mode only
 
   auto entry = [&](int p, int q, int r, int s) -> double {
     return sc_entry<N>(sG, sD, sR, p, q, r, s);
@@ -263,21 +259,6 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
       }
     }
     }
-    if (need_f && !a.A_dense) {
-      const double *jw = a.JxW + e * NN;
-      const uint32_t *row = a.l2g + e * NN;
-      for (int i = tid; i < NI; i += kScThreads) {
-        const int k = (1 + i / M) * N + 1 + i % M;
-        const double f = a.f_nodal ? a.f_nodal[row[k]] : 1.0;
-        sZ[i * LDZ + NE] = a.f_scale * jw[k] * f;
-      }
-      for (int k = tid; k < NE; k += kScThreads) {
-        const int x = sExt[k];
-        const double f = a.f_nodal ? a.f_nodal[row[x]] : 1.0;
-        sFe[k] = a.f_scale * jw[x] * f;
-        if (a.mode & SEMK_SC_BACKSOLVE) sUe[k] = a.u[row[x]];
-      }
-    }
     __syncthreads();
     sc_cholesky<N>(sA, sInv, sBad, tid);
     // ---- Z = L^{-1} [A_ie | f_i] ------------------------------------------------------
@@ -324,16 +305,11 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
         }
       }
       __syncthreads();
-      if (a.A_dense) {
-        const uint32_t *row = a.l2g_hier + e * (int64_t)NN;
-        for (int i = tid; i < NI; i += kScThreads) a.u[row[NE + i]] = sT[i];
-      } else {
-        const uint32_t *row = a.l2g + e * NN;
-        for (int i = tid; i < NI; i += kScThreads) a.u[row[(1 + i / M) * N + 1 + i % M]] = sT[i];
-      }
+      const uint32_t *row = a.l2g_hier + e * (int64_t)NN;
+      for (int i = tid; i < NI; i += kScThreads) a.u[row[NE + i]] = sT[i];
     }
     // ---- keep A_ii^{-1} = L^{-T} L^{-1} (symmetric, dense): with W it turns the condensed
-    // load of ANY later right-hand side into a streaming pass (sc_load_stored_kernel) --------
+    // load of ANY later right-hand side into a streaming pass (sc_load_stored_block_kernel) --
     if ((a.mode & SEMK_SC_STORE_INV) && a.Ainv_out) {
       __syncthreads();
       if (tid < NI) {   // column tid of L^{-1}: forward substitution of the unit vector
@@ -355,120 +331,27 @@ __global__ void __launch_bounds__(kScThreads) sc_element_kernel(ScElemArgs a) {
         Ao[idx] = acc;
       }
     }
-    // ---- keep the interior solution operator: W = A_ii^{-1} A_ie = L^{-T} Z and
-    // c = A_ii^{-1} f_i = L^{-T} (L^{-1} f_i), one thread per column, backward substitution
-    // in place; the back-substitution u_i = c - W u_e then is one streaming pass
-    // (sc_backsolve_stored_kernel) instead of a refactorisation per element ---------------
-    const bool store_w = (a.mode & SEMK_SC_STORE) && a.W_out;
-    const bool store_c = need_f && a.c_out;
-    if (store_w || store_c) {
+    // ---- keep the interior solution operator W = A_ii^{-1} A_ie = L^{-T} Z, one thread per
+    // column, backward substitution in place; the back-substitution u_i = c - W u_e then is
+    // one streaming pass (sc_backsolve_stored_block_kernel) instead of a refactorisation per
+    // element --------------------------------------------------------------------------------
+    if ((a.mode & SEMK_SC_STORE) && a.W_out) {
       __syncthreads();  // every reader of Z is done
-      const bool mine = (store_w && tid < NE) || (store_c && tid == NE);
-      if (mine) sc_backward_col<N>(sA, sInv, sZ, LDZ, tid);
+      if (tid < NE) sc_backward_col<N>(sA, sInv, sZ, LDZ, tid);
       __syncthreads();
-      if (store_w) {
-        double *Wo = a.W_out + e * (int64_t)NE * NI;
-        for (int idx = tid; idx < NE * NI; idx += kScThreads) {
-          const int k = idx / NI, i = idx - k * NI;
-          Wo[idx] = sZ[i * LDZ + k];
-        }
-      }
-      if (store_c) {
-        double *co = a.c_out + e * (int64_t)NI;
-        for (int i = tid; i < NI; i += kScThreads) co[i] = sZ[i * LDZ + NE];
+      double *Wo = a.W_out + e * (int64_t)NE * NI;
+      for (int idx = tid; idx < NE * NI; idx += kScThreads) {
+        const int k = idx / NI, i = idx - k * NI;
+        Wo[idx] = sZ[i * LDZ + k];
       }
     }
   }
 }
 
-// Back-substitution from the stored interior operator: u_i = c - W u_e for every element,
-// one thread per interior row; W is stored transposed ([NE][NI]), so the NI threads of an
-// element read consecutive doubles.  A pure stream over W (12.5 KB per element at p = 8).
-template <int N>
-__global__ void __launch_bounds__(256)
-    sc_backsolve_stored_kernel(int64_t n_elem, const double *__restrict__ W,
-                               const double *__restrict__ c, const uint32_t *__restrict__ l2g,
-                               const int32_t *__restrict__ ext_loc, double *__restrict__ u) {
-  using C = ScCfg<N>;
-  constexpr int NN = C::NN, NE = C::NE, NI = C::NI, M = N - 2;
-  constexpr int GT = ((NI + 31) / 32) * 32;     // threads per element
-  constexpr int GPB = 256 / GT;                 // elements per CTA step
-  __shared__ double sUe[GPB][NE];
-  const int tid = threadIdx.x;
-  const int grp = tid / GT, i = tid - grp * GT;
-  const int64_t n_steps = (n_elem + GPB - 1) / GPB;
-  for (int64_t step = blockIdx.x; step < n_steps; step += gridDim.x) {
-    const int64_t e = step * GPB + grp;
-    const bool on = grp < GPB && e < n_elem;
-    __syncthreads();
-    if (on) {
-      const uint32_t *row = l2g + e * NN;
-      for (int k = i; k < NE; k += GT) sUe[grp][k] = u[row[ext_loc[k]]];
-    }
-    __syncthreads();
-    if (on && i < NI) {
-      const double *Wt = W + e * (int64_t)NE * NI + i;
-      double acc = c ? c[e * (int64_t)NI + i] : 0.0;
-#pragma unroll 8
-      for (int k = 0; k < NE; ++k) acc = fma(-__ldcs(Wt + (int64_t)k * NI), sUe[grp][k], acc);
-      u[l2g[e * NN + (1 + i / M) * N + 1 + i % M]] = acc;
-    }
-  }
-}
-
-// Condensed load from the stored interior operators: for every element
-//   c = A_ii^{-1} f_i,   g = f_e - W^T f_i   (A_ei A_ii^{-1} = W^T by symmetry),
-// f = f_scale * JxW * f_nodal[l2g] as in sc_element_kernel.  A pure stream over A_ii^{-1}
-// (19 KB) and W (12.5 KB per element at p = 8) instead of a refactorisation per element.
-template <int N>
-__global__ void __launch_bounds__(256)
-    sc_load_stored_kernel(int64_t n_elem, const double *__restrict__ W,
-                          const double *__restrict__ Ainv, const uint32_t *__restrict__ l2g,
-                          const int32_t *__restrict__ ext_loc, const double *__restrict__ JxW,
-                          const double *__restrict__ f_nodal, double f_scale,
-                          double *__restrict__ g_loc, double *__restrict__ c_out) {
-  using C = ScCfg<N>;
-  constexpr int NN = C::NN, NE = C::NE, NI = C::NI, M = N - 2;
-  constexpr int GT = ((NI + 31) / 32) * 32;
-  constexpr int GPB = 256 / GT;
-  __shared__ double sF[GPB][NN];
-  const int tid = threadIdx.x;
-  const int grp = tid / GT, i = tid - grp * GT;
-  const int64_t n_steps = (n_elem + GPB - 1) / GPB;
-  for (int64_t step = blockIdx.x; step < n_steps; step += gridDim.x) {
-    const int64_t e = step * GPB + grp;
-    const bool on = grp < GPB && e < n_elem;
-    __syncthreads();
-    if (on) {
-      const uint32_t *row = l2g + e * NN;
-      const double *jw = JxW + e * NN;
-      for (int k = i; k < NN; k += GT)
-        sF[grp][k] = f_scale * jw[k] * (f_nodal ? f_nodal[row[k]] : 1.0);
-    }
-    __syncthreads();
-    if (on && i < NI) {
-      // A_ii^{-1} is symmetric: row i read as column i, consecutive across the threads
-      const double *Ac = Ainv + e * (int64_t)NI * NI + i;
-      double acc = 0.0;
-#pragma unroll 7
-      for (int j = 0; j < NI; ++j)
-        acc = fma(__ldcs(Ac + (int64_t)j * NI), sF[grp][(1 + j / M) * N + 1 + j % M], acc);
-      c_out[e * (int64_t)NI + i] = acc;
-    }
-    if (on && i < NE) {
-      const double *Wr = W + e * (int64_t)NE * NI + (int64_t)i * NI;
-      double acc = sF[grp][ext_loc[i]];
-      for (int j = 0; j < NI; ++j)
-        acc = fma(-Wr[j], sF[grp][(1 + j / M) * N + 1 + j % M], acc);
-      g_loc[e * (int64_t)NE + i] = acc;
-    }
-  }
-}
-
-// ---- block loads: up to kScBlockMaxCols load columns per element pass ---------------------
-// Column j's load is f_scale[j] * JxW * (nodal_mask bit j ? F[j][l2g] : 1), the expression of
-// sc_element_kernel, and every column goes through the same operations in the same order as a
-// single-load pass, so each column is bitwise the result of that pass.
+// ---- loads: up to kScBlockMaxCols load columns per pass --------------------------------------
+// Column j's load is f_scale[j] * JxW * (nodal_mask bit j ? F[j][l2g] : 1), and every column
+// goes through the same operations in the same order whatever k and the other columns, so each
+// column is bitwise the result of a one-column pass (the single-load entries).
 constexpr int kScBlockMaxCols = 32;
 
 struct ScBlockLoad {
@@ -487,6 +370,7 @@ __device__ __forceinline__ double sc_block_load(const ScBlockLoad &L, int j, con
 
 struct ScBlockArgs {
   int64_t n_elem;
+  const int64_t *slot_of_elem;
   const double *G;
   int64_t g_patch_stride;
   int pe;
@@ -499,7 +383,7 @@ struct ScBlockArgs {
   ScBlockLoad L;
   double *g_loc;                    // RHS: [k][ldg], row j = [n_elem][NE]
   int64_t ldg;
-  double *c_out;                    // RHS, optional: [k][ldc], row j = [n_elem][NI] = A_ii^{-1} f_i
+  double *c_out;                    // optional: [k][ldc], row j = [n_elem][NI] = A_ii^{-1} f_i
   int64_t ldc;
   double *U;                        // BACKSOLVE: [k][ldu] nodal vectors
   int64_t ldu;
@@ -537,7 +421,7 @@ __global__ void __launch_bounds__(kScThreads, 1) sc_element_block_kernel(ScBlock
   const int tid = threadIdx.x;
   for (int64_t e = blockIdx.x; e < a.n_elem; e += gridDim.x) {
     __syncthreads();
-    sc_stage_element<N>(e, nullptr, a.G, a.g_patch_stride, a.pe, a.D, a.react, a.ext_loc, sG, sD,
+    sc_stage_element<N>(e, a.slot_of_elem, a.G, a.g_patch_stride, a.pe, a.D, a.react, a.ext_loc, sG, sD,
                         sR, sExt, tid);
     if (tid == 0) *sBad = 0;
     __syncthreads();
@@ -564,15 +448,6 @@ __global__ void __launch_bounds__(kScThreads, 1) sc_element_block_kernel(ScBlock
         double acc = sV[idx];
         for (int i = 0; i < NI; ++i) acc = fma(-sZ[i * ldz + q], sZ[i * ldz + NE + j], acc);
         a.g_loc[j * a.ldg + e * NE + q] = acc;
-      }
-      if (a.c_out) {  // c = L^{-T} (L^{-1} f_i), one thread per column
-        __syncthreads();
-        if (tid < k) sc_backward_col<N>(sA, sInv, sZ, ldz, NE + tid);
-        __syncthreads();
-        for (int idx = tid; idx < k * NI; idx += kScThreads) {
-          const int j = idx / NI, i = idx - j * NI;
-          a.c_out[j * a.ldc + e * NI + i] = sZ[i * ldz + NE + j];
-        }
       }
     } else {
       // u_i = L^{-T} (L^{-1} f_i - Z u_e): the product one thread per entry, the backward
@@ -602,15 +477,31 @@ __global__ void __launch_bounds__(kScThreads, 1) sc_element_block_kernel(ScBlock
         a.U[j * a.ldu + row[(1 + i / M) * N + 1 + i % M]] = sT[idx];
       }
     }
+    if (a.c_out) {  // c = L^{-T} (L^{-1} f_i), one thread per column
+      __syncthreads();
+      if (tid < k) sc_backward_col<N>(sA, sInv, sZ, ldz, NE + tid);
+      __syncthreads();
+      for (int idx = tid; idx < k * NI; idx += kScThreads) {
+        const int j = idx / NI, i = idx - j * NI;
+        a.c_out[j * a.ldc + e * NI + i] = sZ[i * ldz + NE + j];
+      }
+    }
   }
 }
 
-// sc_backsolve_stored_kernel for k <= KB columns: W is read once for all of them; column j of
-// u_i is c[j] - W u_e[j], the same fma chain as the single kernel.  KB (1, 2, 4, ... 32) is the
-// register tile: the launch takes the smallest that holds k, so that a few columns do not pay
-// for 32 predicated accumulators.
+// An unroll count of 0 is ignored: the wider tiles' element loops stay the compiler's choice.
+constexpr int kScCompilerUnroll = 0;
+#pragma nv_diag_suppress 20168
+
+// Back-substitution from the stored interior operator: u_i = c - W u_e for every element and
+// each of k <= KB columns, one thread per interior row; W is stored transposed ([NE][NI]), so
+// the NI threads of an element read consecutive doubles, and it is read once for all columns
+// (a pure stream: 12.5 KB per element at p = 8).  KB (1, 2, 4, ... 32) is the register tile:
+// the launch takes the smallest that holds k, so that a few columns do not pay for 32
+// predicated accumulators.  The one-column tile is a latency-bound stream: it keeps eight
+// CTAs per SM (32 registers) and eight loads of W in flight per thread.
 template <int N, int KB>
-__global__ void __launch_bounds__(256, 1)
+__global__ void __launch_bounds__(256, KB == 1 ? 8 : 1)
     sc_backsolve_stored_block_kernel(int64_t n_elem, const double *__restrict__ W,
                                      const double *__restrict__ c, int64_t ldc,
                                      const uint32_t *__restrict__ l2g,
@@ -643,6 +534,7 @@ __global__ void __launch_bounds__(256, 1)
       for (int j = 0; j < KB; ++j)
         acc[j] = (j < k && c) ? c[j * ldc + e * (int64_t)NI + i] : 0.0;
       const double *Wt = W + e * (int64_t)NE * NI + i;
+#pragma unroll(KB == 1 ? 8 : kScCompilerUnroll)
       for (int q = 0; q < NE; ++q) {
         const double w = __ldcs(Wt + (int64_t)q * NI);
 #pragma unroll
@@ -657,7 +549,11 @@ __global__ void __launch_bounds__(256, 1)
   }
 }
 
-// sc_load_stored_kernel for k <= KB columns: A_ii^{-1} and W are read once for all of them.
+// Condensed load from the stored interior operators: for every element and each of k <= KB
+// columns  c = A_ii^{-1} f_i,  g = f_e - W^T f_i  (A_ei A_ii^{-1} = W^T by symmetry).  A pure
+// stream over A_ii^{-1} (19 KB) and W (12.5 KB per element at p = 8), read once for all columns,
+// instead of a refactorisation per element.  The one-column tile keeps seven loads of
+// A_ii^{-1} in flight per thread.
 template <int N, int KB>
 __global__ void __launch_bounds__(256)
     sc_load_stored_block_kernel(int64_t n_elem, const double *__restrict__ W,
@@ -694,6 +590,7 @@ __global__ void __launch_bounds__(256)
       const double *Ac = Ainv + e * (int64_t)NI * NI + i;
 #pragma unroll
       for (int j = 0; j < KB; ++j) acc[j] = 0.0;
+#pragma unroll(KB == 1 ? 7 : kScCompilerUnroll)
       for (int jj = 0; jj < NI; ++jj) {
         const double v = __ldcs(Ac + (int64_t)jj * NI);
         const int x = (1 + jj / M) * N + 1 + jj % M;
@@ -1037,6 +934,17 @@ int launch_backsolve_stored_block_tiled(int64_t n_elem, const double *W, const d
   }
 
 static int launch_sc_element(int n1, const ScElemArgs &a, void *stream);
+static int launch_sc_element_block(int n1, const ScBlockArgs &a, void *stream);
+
+// one load column f_scale * JxW * (f_nodal ? f_nodal[l2g] : 1): the k = 1 case of ScBlockLoad
+static ScBlockLoad sc_single_load(const double *f_nodal, double f_scale) {
+  ScBlockLoad L{};
+  L.k = 1;
+  L.F = f_nodal;
+  L.nodal_mask = f_nodal ? 1u : 0u;
+  L.f_scale[0] = f_scale;
+  return L;
+}
 
 extern "C" int semk_sc_element_f64(int n1, int64_t n_elem, const int64_t *slot_of_elem,
                                    const double *G, int64_t g_patch_stride, int elems_per_patch,
@@ -1051,6 +959,8 @@ extern "C" int semk_sc_element_f64(int n1, int64_t n_elem, const int64_t *slot_o
                                    stream);
 }
 
+// The factorisation outputs (SCHUR, STORE, STORE_INV) are one pass of sc_element_kernel, the
+// loads (RHS, then BACKSOLVE) one-column passes of sc_element_block_kernel, in that order.
 extern "C" int semk_sc_element_react_f64(int n1, int64_t n_elem, const int64_t *slot_of_elem,
                                          const double *G, int64_t g_patch_stride,
                                          int elems_per_patch, const double *D,
@@ -1074,7 +984,7 @@ extern "C" int semk_sc_element_react_f64(int n1, int64_t n_elem, const int64_t *
     semk_set_error("semk_sc_element_f64: static condensation supports orders 2..10");
     return SEMK_ERR_UNSUPPORTED;
   }
-  const int ne = 4 * (n1 - 1);
+  const int ne = 4 * (n1 - 1), ni = (n1 - 2) * (n1 - 2);
   if (mode & SEMK_SC_SCHUR)
     SEMK_REQUIRE(S_out && s_stride == (int64_t)ne * (ne + 1) / 2,
                  "semk_sc_element_f64: SCHUR needs S_out and the packed stride");
@@ -1082,33 +992,52 @@ extern "C" int semk_sc_element_react_f64(int n1, int64_t n_elem, const int64_t *
     SEMK_REQUIRE(g_loc && JxW && l2g, "semk_sc_element_f64: RHS needs g_loc, JxW, l2g");
   if (mode & SEMK_SC_BACKSOLVE)
     SEMK_REQUIRE(u && JxW && l2g, "semk_sc_element_f64: BACKSOLVE needs u, JxW, l2g");
-  ScElemArgs a;
-  a.n_elem = n_elem;
-  a.slot_of_elem = slot_of_elem;
-  a.G = G;
-  a.g_patch_stride = g_patch_stride;
-  a.pe = elems_per_patch;
-  a.D = D;
-  a.ext_loc = ext_loc;
-  a.l2g = l2g;
-  a.JxW = JxW;
-  a.f_nodal = f_nodal;
-  a.f_scale = f_scale;
-  a.mode = mode;
-  a.S_out = S_out;
-  a.s_stride = s_stride;
-  a.sdiag_loc = sdiag_loc;
-  a.g_loc = g_loc;
-  a.u = u;
-  a.bad_flag = bad_flag;
-  a.W_out = W_out;
-  a.c_out = c_out;
-  a.A_dense = nullptr;
-  a.f_dense = nullptr;
-  a.l2g_hier = nullptr;
-  a.react = react;
-  a.Ainv_out = Ainv_out;
-  return launch_sc_element(n1, a, stream);
+  if (mode & (SEMK_SC_SCHUR | SEMK_SC_STORE | SEMK_SC_STORE_INV)) {
+    ScElemArgs a{};
+    a.n_elem = n_elem;
+    a.slot_of_elem = slot_of_elem;
+    a.G = G;
+    a.g_patch_stride = g_patch_stride;
+    a.pe = elems_per_patch;
+    a.D = D;
+    a.ext_loc = ext_loc;
+    a.mode = mode & (SEMK_SC_SCHUR | SEMK_SC_STORE | SEMK_SC_STORE_INV);
+    a.S_out = S_out;
+    a.s_stride = s_stride;
+    a.sdiag_loc = sdiag_loc;
+    a.W_out = W_out;
+    a.react = react;
+    a.Ainv_out = Ainv_out;
+    a.bad_flag = bad_flag;
+    const int rc = launch_sc_element(n1, a, stream);
+    if (rc != SEMK_OK) return rc;
+  }
+  ScBlockArgs b{};
+  b.n_elem = n_elem;
+  b.slot_of_elem = slot_of_elem;
+  b.G = G;
+  b.g_patch_stride = g_patch_stride;
+  b.pe = elems_per_patch;
+  b.D = D;
+  b.ext_loc = ext_loc;
+  b.l2g = l2g;
+  b.JxW = JxW;
+  b.react = react;
+  b.L = sc_single_load(f_nodal, f_scale);
+  b.g_loc = g_loc;
+  b.ldg = n_elem * ne;
+  b.c_out = c_out;
+  b.ldc = n_elem * ni;
+  b.U = u;                          // one column: the row stride ldu is never used
+  b.bad_flag = bad_flag;
+  for (const int load_mode : {SEMK_SC_RHS, SEMK_SC_BACKSOLVE}) {
+    if (!(mode & load_mode)) continue;
+    b.mode = load_mode;
+    const int rc = launch_sc_element_block(n1, b, stream);
+    if (rc != SEMK_OK) return rc;
+    b.c_out = nullptr;              // written by the first load pass
+  }
+  return SEMK_OK;
 }
 
 extern "C" int semk_sc_element_dense_f64(int n1, int64_t n_elem, const double *A_hier,
@@ -1131,32 +1060,19 @@ extern "C" int semk_sc_element_dense_f64(int n1, int64_t n_elem, const double *A
   if (mode & SEMK_SC_BACKSOLVE)
     SEMK_REQUIRE(u && f_hier && l2g_hier,
                  "semk_sc_element_dense_f64: BACKSOLVE needs u, f_hier, l2g_hier");
-  ScElemArgs a;
+  ScElemArgs a{};
   a.n_elem = n_elem;
-  a.slot_of_elem = nullptr;
-  a.G = nullptr;
-  a.g_patch_stride = 0;
   a.pe = 1;
-  a.D = nullptr;
-  a.ext_loc = nullptr;
-  a.l2g = nullptr;
-  a.JxW = nullptr;
-  a.f_nodal = nullptr;
-  a.f_scale = 1.0;
   a.mode = mode;
   a.S_out = S_out;
   a.s_stride = s_stride;
   a.sdiag_loc = sdiag_loc;
+  a.bad_flag = bad_flag;
   a.g_loc = g_loc;
   a.u = u;
-  a.bad_flag = bad_flag;
-  a.W_out = nullptr;
-  a.c_out = nullptr;
   a.A_dense = A_hier;
   a.f_dense = f_hier;
   a.l2g_hier = l2g_hier;
-  a.react = nullptr;
-  a.Ainv_out = nullptr;
   return launch_sc_element(n1, a, stream);
 }
 
@@ -1177,21 +1093,38 @@ static int launch_sc_element(int n1, const ScElemArgs &a, void *stream) {
   return SEMK_OK;
 }
 
+static int launch_sc_element_block(int n1, const ScBlockArgs &a, void *stream) {
+  const int64_t n_elem = a.n_elem;
+  cudaStream_t st = semk_stream(stream);
+  const unsigned grid = (unsigned)(n_elem < 148 * 16 ? n_elem : 148 * 16);
+#define SEMK_CALL(NV)                                                                      \
+  do {                                                                                     \
+    const size_t smem = sc_block_smem<NV>(a.L.k, a.mode);                                  \
+    SEMK_CUDA_CHECK(cudaFuncSetAttribute(sc_element_block_kernel<NV>,                      \
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize,      \
+                                         (int)sc_block_smem<NV>(kScBlockMaxCols,           \
+                                                                SEMK_SC_BACKSOLVE)));      \
+    sc_element_block_kernel<NV><<<grid, kScThreads, smem, st>>>(a);                        \
+  } while (0)
+  SEMK_DISPATCH_SC(n1, SEMK_CALL)
+#undef SEMK_CALL
+  SEMK_LAUNCH_CHECK("sc_element_block_kernel");
+  return SEMK_OK;
+}
+
 extern "C" int semk_sc_backsolve_stored_f64(int n1, int64_t n_elem, const double *W,
                                            const double *c, const uint32_t *l2g,
                                            const int32_t *ext_loc, double *u, void *stream) {
   SEMK_REQUIRE(n_elem > 0 && W && l2g && ext_loc && u, "semk_sc_backsolve_stored_f64: bad argument");
+  const int64_t ldc = n_elem * (n1 - 2) * (n1 - 2);
   cudaStream_t st = semk_stream(stream);
-#define SEMK_CALL(NV)                                                                      \
-  do {                                                                                     \
-    constexpr int GT = ((ScCfg<NV>::NI + 31) / 32) * 32, GPB = 256 / GT;                   \
-    const int64_t steps = (n_elem + GPB - 1) / GPB;                                        \
-    const unsigned grid = (unsigned)(steps < 148 * 16 ? steps : 148 * 16);                 \
-    sc_backsolve_stored_kernel<NV><<<grid, 256, 0, st>>>(n_elem, W, c, l2g, ext_loc, u);   \
-  } while (0)
+  int rc = SEMK_OK;
+#define SEMK_CALL(NV) \
+  rc = launch_backsolve_stored_block_tiled<NV>(n_elem, W, c, ldc, l2g, ext_loc, 1, u, 0, st)
   SEMK_DISPATCH_SC(n1, SEMK_CALL)
 #undef SEMK_CALL
-  SEMK_LAUNCH_CHECK("sc_backsolve_stored_kernel");
+  if (rc != SEMK_OK) return rc;
+  SEMK_LAUNCH_CHECK("sc_backsolve_stored_block_kernel");
   return SEMK_OK;
 }
 
@@ -1201,18 +1134,17 @@ extern "C" int semk_sc_load_stored_f64(int n1, int64_t n_elem, const double *W, 
                                        double *g_loc, double *c_out, void *stream) {
   SEMK_REQUIRE(n_elem > 0 && W && Ainv && l2g && ext_loc && JxW && g_loc && c_out,
                "semk_sc_load_stored_f64: bad argument");
+  const ScBlockLoad L = sc_single_load(f_nodal, f_scale);
+  const int64_t ldg = n_elem * 4 * (n1 - 1), ldc = n_elem * (n1 - 2) * (n1 - 2);
   cudaStream_t st = semk_stream(stream);
-#define SEMK_CALL(NV)                                                                      \
-  do {                                                                                     \
-    constexpr int GT = ((ScCfg<NV>::NI + 31) / 32) * 32, GPB = 256 / GT;                   \
-    const int64_t steps = (n_elem + GPB - 1) / GPB;                                        \
-    const unsigned grid = (unsigned)(steps < 148 * 16 ? steps : 148 * 16);                 \
-    sc_load_stored_kernel<NV><<<grid, 256, 0, st>>>(n_elem, W, Ainv, l2g, ext_loc, JxW,    \
-                                                    f_nodal, f_scale, g_loc, c_out);       \
-  } while (0)
+  int rc = SEMK_OK;
+#define SEMK_CALL(NV)                                                                          \
+  rc = launch_load_stored_block_tiled<NV>(n_elem, W, Ainv, l2g, ext_loc, JxW, L, g_loc, ldg, \
+                                          c_out, ldc, st)
   SEMK_DISPATCH_SC(n1, SEMK_CALL)
 #undef SEMK_CALL
-  SEMK_LAUNCH_CHECK("sc_load_stored_kernel");
+  if (rc != SEMK_OK) return rc;
+  SEMK_LAUNCH_CHECK("sc_load_stored_block_kernel");
   return SEMK_OK;
 }
 
@@ -1253,7 +1185,7 @@ extern "C" int semk_sc_element_block_f64(int n1, int64_t n_elem, const double *G
                                          double *g_loc, int64_t ldg, double *c_out, int64_t ldc,
                                          double *U, int64_t ldu, int32_t *bad_flag,
                                          void *stream) {
-  ScBlockArgs a;
+  ScBlockArgs a{};
   int rc = sc_block_load_args("semk_sc_element_block_f64", n1, k, F, ldf, nodal_mask, f_scale,
                               &a.L);
   if (rc != SEMK_OK) return rc;
@@ -1263,14 +1195,13 @@ extern "C" int semk_sc_element_block_f64(int n1, int64_t n_elem, const double *G
   SEMK_REQUIRE(mode == SEMK_SC_RHS || mode == SEMK_SC_BACKSOLVE,
                "semk_sc_element_block_f64: mode must be SEMK_SC_RHS or SEMK_SC_BACKSOLVE");
   const int ne = 4 * (n1 - 1), ni = (n1 - 2) * (n1 - 2);
-  if (mode == SEMK_SC_RHS) {
-    SEMK_REQUIRE(g_loc && ldg >= n_elem * ne && (!c_out || ldc >= n_elem * ni),
-                 "semk_sc_element_block_f64: RHS needs g_loc [k][ldg >= n_elem * 4p] (and c_out "
-                 "[k][ldc >= n_elem * (p-1)^2])");
-  } else {
-    SEMK_REQUIRE(U && ldu > 0 && !c_out,
-                 "semk_sc_element_block_f64: BACKSOLVE needs U [k][ldu] and no c_out");
-  }
+  if (mode == SEMK_SC_RHS)
+    SEMK_REQUIRE(g_loc && ldg >= n_elem * ne,
+                 "semk_sc_element_block_f64: RHS needs g_loc [k][ldg >= n_elem * 4p]");
+  else
+    SEMK_REQUIRE(U && ldu > 0, "semk_sc_element_block_f64: BACKSOLVE needs U [k][ldu > 0]");
+  SEMK_REQUIRE(!c_out || ldc >= n_elem * ni,
+               "semk_sc_element_block_f64: c_out needs ldc >= n_elem * (p-1)^2");
   a.n_elem = n_elem;
   a.G = G;
   a.g_patch_stride = g_patch_stride;
@@ -1288,21 +1219,7 @@ extern "C" int semk_sc_element_block_f64(int n1, int64_t n_elem, const double *G
   a.U = U;
   a.ldu = ldu;
   a.bad_flag = bad_flag;
-  cudaStream_t st = semk_stream(stream);
-  const unsigned grid = (unsigned)(n_elem < 148 * 16 ? n_elem : 148 * 16);
-#define SEMK_CALL(NV)                                                                      \
-  do {                                                                                     \
-    const size_t smem = sc_block_smem<NV>(k, mode);                                        \
-    SEMK_CUDA_CHECK(cudaFuncSetAttribute(sc_element_block_kernel<NV>,                      \
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,      \
-                                         (int)sc_block_smem<NV>(kScBlockMaxCols,           \
-                                                                SEMK_SC_BACKSOLVE)));      \
-    sc_element_block_kernel<NV><<<grid, kScThreads, smem, st>>>(a);                        \
-  } while (0)
-  SEMK_DISPATCH_SC(n1, SEMK_CALL)
-#undef SEMK_CALL
-  SEMK_LAUNCH_CHECK("sc_element_block_kernel");
-  return SEMK_OK;
+  return launch_sc_element_block(n1, a, stream);
 }
 
 extern "C" int semk_sc_load_stored_block_f64(int n1, int64_t n_elem, const double *W,

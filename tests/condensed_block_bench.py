@@ -111,14 +111,23 @@ def block_passes(sc, F, stored_load=False):
         def blk_rhs(k):
             sc._element_block(_lib.SC_RHS, load_of(k), g_loc=g_blk, c=c_blk)
 
+        def one_element(mode, f, g_loc=None, u=None, c=None):
+            """The single-load C entry: one load pass of the element kernel."""
+            _lib.check(sc._lib.semk_sc_element_react_f64(
+                sc.n1, E, None, device.ptr(sc.G), sc.g_stride, 1, device.ptr(sc.tab.dev()[0]),
+                device.ptr(sc._t["ext_loc"]), device.ptr(sc.l2g_dev), device.ptr(sc.JxW),
+                device.ptr(f), 1.0, mode, None, sc.s_stride, None, device.ptr(g_loc),
+                device.ptr(u), None, device.ptr(c), device.ptr(sc._react), None,
+                device.ptr(sc._bad), device.stream_ptr()))
+
         def one_rhs(j):
-            sc._element_pass(_lib.SC_RHS, g_loc=g_one, f=F[j], c=c_one)
+            one_element(_lib.SC_RHS, F[j], g_loc=g_one, c=c_one)
 
         def blk_back(k):
             sc._element_block(_lib.SC_BACKSOLVE, load_of(k), U=U)
 
         def one_back(j):
-            sc._element_pass(_lib.SC_BACKSOLVE, u=Uo, f=F[j])
+            one_element(_lib.SC_BACKSOLVE, F[j], u=Uo)
 
         def blk_stored(k):
             _lib.check(sc._lib.semk_sc_backsolve_stored_block_f64(

@@ -57,9 +57,9 @@ def test_block_entries_check_their_arguments():
     lib = _lib.load()
     scale = (C.c_double * 33)(*([1.0] * 33))
 
-    def element(n1=9, mode=2, k=3, F=None, mask=0):
+    def element(n1=9, mode=2, k=3, F=None, mask=0, c_out=None, ldc=0, U=None, ldu=0):
         return lib.semk_sc_element_block_f64(n1, 4, 8, 1, 1, 8, 8, 8, 8, None, mode, k, F, 100,
-                                             mask, scale, 8, 1 << 20, None, 0, None, 0, 8, None)
+                                             mask, scale, 8, 1 << 20, c_out, ldc, U, ldu, 8, None)
 
     assert element(k=33) == _lib.ERR_UNSUPPORTED
     assert element(n1=2) == _lib.ERR_UNSUPPORTED
@@ -68,6 +68,9 @@ def test_block_entries_check_their_arguments():
     assert element(mode=1) == _lib.ERR_INVALID
     assert element(mask=1) == _lib.ERR_INVALID          # a nodal column without F
     assert element(mask=8) == _lib.ERR_INVALID          # bit beyond k
+    assert element(mode=4) == _lib.ERR_INVALID          # BACKSOLVE without U
+    assert element(mode=4, U=8, ldu=10, c_out=8, ldc=4 * 49 - 1) == _lib.ERR_INVALID  # short c
+    assert element(mode=2, c_out=8, ldc=4 * 49 - 1) == _lib.ERR_INVALID
     assert lib.semk_sc_load_stored_block_f64(9, 4, 8, 8, 8, 8, 8, 33, None, 0, 0, scale, 8,
                                              1 << 20, 8, 1 << 20, None) == _lib.ERR_UNSUPPORTED
     assert lib.semk_sc_load_stored_block_f64(9, 4, 8, 8, 8, 8, 8, 2, None, 0, 0, scale, 8,

@@ -224,3 +224,46 @@ def test_block_errors():
                  lambda: cs.solve_load_many([cs.new_vector(0.0)], [1.0])):
         with pytest.raises(NotImplementedError):
             call()
+
+
+@pytest.mark.parametrize("p", [2, 8])
+def test_single_load_entry_combined_modes_equal_single_bit_calls(p):
+    """semk_sc_element_react_f64 runs the factorisation bits and the load bits (one-column
+    block passes) in turn: a combined mode, c_out in either load mode and a permuted
+    slot_of_elem give the outputs of the single-bit calls."""
+    from spectralelementmethod_b200 import _lib, device
+    mngr, sc = operator(p, "stored")
+    f64 = dict(dtype=torch.float64, device=sc.dev)
+    E, NE, NI = sc.n_elem, sc.n_ext_loc, sc.n_int_loc
+    rng = np.random.default_rng(p)
+    f = torch.from_numpy(rng.standard_normal(sc.n_nodes)).cuda()
+    x = torch.from_numpy(rng.standard_normal(sc.n_nodes)).cuda()
+    slot = torch.from_numpy(rng.permutation(E).astype(np.int64)).cuda()
+    G_slot = torch.empty_like(sc.G)
+    G_slot[slot] = sc.G
+
+    def call(mode, outs, G=sc.G, slot_of_elem=None):
+        shapes = dict(S=(E, sc.s_stride), sdiag=(E, NE), W=(E, NE, NI), g=(E, NE), c=(E, NI))
+        res = {k: (x.clone() if k == "u" else torch.full(shapes[k], -1.0, **f64)) for k in outs}
+        P = lambda k: device.ptr(res.get(k))      # noqa: E731
+        bad = torch.zeros(1, dtype=torch.int32, device=sc.dev)
+        _lib.check(sc._lib.semk_sc_element_react_f64(
+            sc.n1, E, device.ptr(slot_of_elem), device.ptr(G), sc.g_stride, 1,
+            device.ptr(sc.tab.dev()[0]), device.ptr(sc._t["ext_loc"]), device.ptr(sc.l2g_dev),
+            device.ptr(sc.JxW), device.ptr(f), 0.75, mode, P("S"), sc.s_stride, P("sdiag"),
+            P("g"), P("u"), P("W"), P("c"), None, None, device.ptr(bad), device.stream_ptr()))
+        assert int(bad.item()) == 0
+        return res
+
+    SCHUR, STORE, RHS, BACK = _lib.SC_SCHUR, _lib.SC_STORE, _lib.SC_RHS, _lib.SC_BACKSOLVE
+    schur = call(SCHUR, "S sdiag".split())
+    store = call(STORE, ["W"])
+    rhs = call(RHS, ["g", "c"])
+    back = call(BACK, ["u"])
+    both = call(SCHUR | STORE | RHS, "S sdiag W g c".split())
+    for k, ref in (("S", schur), ("sdiag", schur), ("W", store), ("g", rhs), ("c", rhs)):
+        assert torch.equal(both[k], ref[k]), k
+    loads = call(RHS | BACK, ["g", "u"])
+    assert torch.equal(loads["g"], rhs["g"]) and torch.equal(loads["u"], back["u"])
+    back_c = call(BACK, ["u", "c"], G=G_slot, slot_of_elem=slot)
+    assert torch.equal(back_c["u"], back["u"]) and torch.equal(back_c["c"], rhs["c"])
